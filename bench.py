@@ -2,7 +2,7 @@
 """bench.py -- headline benchmark of the hot path (encode -> canonical l-mer table -> de Bruijn
 graph build) in forward k-mer windows per second (BASELINE.json `metric`).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload NAME]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload NAME] [--dump-outputs DIR]
 
 One process per GPU (torchrun for N > 1).  A step is one pass of the hot path over one batch of
 synthetic reads.  Rank 0 prints ONE JSON line.
@@ -27,6 +27,7 @@ PKG = os.path.join(ROOT, "pycuda-euler_b200")
 for p in (ROOT, PKG):
     if p not in sys.path:
         sys.path.insert(0, p)
+sys.dont_write_bytecode = True   # the benchmark leaves the tree as it found it (which may be read-only): no __pycache__
 
 WORKLOADS = {
     # BASELINE.json configs[1]: the configuration the metric is quoted on for 1 GPU
@@ -183,12 +184,9 @@ def run_reference(args, wl, rank, world):
     for _ in range(min(args.warmup, 1)):
         cpu_rate(wl, max(G1 // 8, 10_000), procs)
     vals, last = [], None
-    t_budget = time.perf_counter()
-    for i in range(args.steps):
+    for _ in range(args.steps):
         last = cpu_rate(wl, G1, procs)
         vals.append(last["value"])
-        if time.perf_counter() - t_budget > 150 and i + 1 >= 2:   # keep the arm within a few minutes
-            break
     value = sorted(vals)[len(vals) // 2]
     nk_step = wl["cov"] * 3 * G1 // wl["L"] * (wl["L"] - wl["k"] + 1)
     line = {
@@ -233,6 +231,49 @@ def roofline_record(st, ms_part, ms_build, ms_step, l, workload, world):
             "traffic": traffic, "peak_source": peak_src, "algorithmic_bytes_per_launch": a_kernel,
             "path_algorithmic_bytes": a_path, "path_frac": a_path / (ms_step * 1e-3) / 1e9 / peak,
             "kernels_ms": {"bkt_partition_kernel": ms_part, "bkt_build_kernel": ms_build} if st.path == 1 else {"count_kernel": ms_part}}
+
+
+def dump_outputs(ctx, st, l, out_dir, max_rows=1 << 18, seed=0):
+    """--dump-outputs: the graph the last timed step left in ctx, as float64 .npy files under out_dir, so that two builds can
+    be compared output for output.  Ids are in table-slot order, which may differ between runs, so the tables are written in
+    key order: l-mers and vertices sorted by key, edge end points as ranks in that vertex order.  A key is stored as its
+    32-bit words, most significant first (float64 holds each exactly).  A table of more than max_rows rows is cut to a fixed,
+    seeded sample of max_rows rows; lmer_rows / kmer_rows hold their places in the sorted table."""
+    import numpy as np
+    import _native as N
+    wide = l > 32
+
+    def keys(which, which_hi):
+        return ctx.download(which), ctx.download(which_hi) if wide else None
+
+    def order(lo, hi):
+        return np.lexsort((lo, hi)) if wide else np.argsort(lo, kind="stable")
+
+    def words(lo, hi):
+        w = [lo >> np.uint64(32), lo & np.uint64(0xFFFFFFFF)]
+        return np.stack(([hi >> np.uint64(32), hi & np.uint64(0xFFFFFFFF)] if wide else []) + w, axis=1)
+
+    def sample(n):
+        return np.arange(n) if n <= max_rows else np.sort(np.random.default_rng(seed).choice(n, max_rows, replace=False))
+
+    lk, lk_hi = keys(N.ART_LMER_KEYS, N.ART_LMER_KEYS_HI)
+    vk, vk_hi = keys(N.ART_KMER_KEYS, N.ART_KMER_KEYS_HI)
+    o, ov = order(lk, lk_hi), order(vk, vk_hi)
+    rank = np.empty(vk.size, np.int64)
+    rank[ov] = np.arange(vk.size)
+    lrows, vrows = sample(lk.size), sample(vk.size)
+    li, vi = o[lrows], ov[vrows]
+    out = {
+        "counts": np.array([st.n_kmer_windows, st.n_lmer_windows, st.distinct_lmers, st.distinct_kmers, st.edge_count]),
+        "lmer_rows": lrows, "lmer_keys": words(lk[li], lk_hi[li] if wide else None),
+        "lmer_values": ctx.download(N.ART_LMER_VALUES)[li],
+        "edge_v1": rank[ctx.download(N.ART_EDGE_V1)[li]], "edge_v2": rank[ctx.download(N.ART_EDGE_V2)[li]],
+        "kmer_rows": vrows, "kmer_keys": words(vk[vi], vk_hi[vi] if wide else None),
+        "lcount": ctx.download(N.ART_LCOUNT).reshape(-1, 4)[vi], "ecount": ctx.download(N.ART_ECOUNT).reshape(-1, 4)[vi],
+    }
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
 
 
 class Runner:
@@ -436,12 +477,18 @@ def main():
     ap.add_argument("--no-extra", action="store_true", help="skip the extra BASELINE configs (configs[2..4]) reported under `extra`")
     ap.add_argument("--extra-scale", type=float, default=1.0,
                     help="development aid: scale the genome of the extra configs (0.25 on 2 GPUs = the per-rank size of the 8-GPU run)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the graph of the last one as DIR/<name>.npy (float64, key order; see dump_outputs)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or world > 1):
+        ap.error("--dump-outputs writes the outputs of the one-GPU path (--impl b200, one process)")
     wl = dict(WORKLOADS[args.workload])
     if args.k:
         wl["k"] = args.k
@@ -486,6 +533,8 @@ def main():
     m = runner.measure(args.steps, args.warmup)
     clocks = sampler.result()
     st, info, ms_max = m["st"], m["info"], m["ms"]
+    if args.dump_outputs:
+        dump_outputs(ctx, st, l, args.dump_outputs)
     nohint = None
     if world == 1 and hint:   # the same steady state without the genome-size hint (capacities learned from the previous run)
         m0 = runner.measure(max(3, args.steps // 4), 2, hint=0)

@@ -14,14 +14,6 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 PKG = os.path.join(ROOT, "pycuda-euler_b200")
 
 
-def _has_gpu():
-    try:
-        import torch
-        return torch.cuda.is_available()
-    except Exception:
-        return False
-
-
 def test_library_exports_every_declared_symbol():
     import __graft_entry__ as ge
     if not os.path.exists(ge.LIB):
@@ -37,14 +29,21 @@ def test_library_exports_every_declared_symbol():
 
 
 def test_no_cpu_fallback_without_a_device():
-    if _has_gpu():
-        pytest.skip("a GPU is present")
-    import _native
-    with pytest.raises(_native.EulerError):
-        _native.Context(0)
-    import eulercuda.eulercuda as ec
-    with pytest.raises(_native.EulerError):
-        ec.assemble2(9, buffer=["ACGTACGTACGTACGT"])
+    """In a child process that sees no CUDA device (none present, or hidden from it) the product path raises."""
+    code = r'''
+import sys
+sys.path[:0] = [%r, %r]
+import pytest, _native
+with pytest.raises(_native.EulerError):
+    _native.Context(0)
+import eulercuda.eulercuda as ec
+with pytest.raises(_native.EulerError):
+    ec.assemble2(9, buffer=["ACGTACGTACGTACGT"])
+print("ok")
+''' % (ROOT, PKG)
+    out = subprocess.run([sys.executable, "-c", code], env=dict(os.environ, CUDA_VISIBLE_DEVICES=""), capture_output=True,
+                         text=True, timeout=300)
+    assert out.returncode == 0 and out.stdout.strip() == "ok", out.stdout[-1000:] + out.stderr[-2000:]
 
 
 def test_product_never_imports_the_oracle():
@@ -133,27 +132,6 @@ def test_bench_reference_arm_runs_on_cpu():
     assert line["cpu_baseline"]["cores"] >= 1 and line["e2e"]["h2d_bytes_per_step"] == 0
 
 
-def test_reference_bytecode_is_the_reference():
-    """oracle/build_ref.py byte-compiles the unmodified reference module; loaded sourceless it gives the golden tables."""
-    import importlib.machinery
-    import importlib.util
-    import json
-    import types
-    from oracle import build_ref
-    pyc = build_ref.build()
-    if pyc is None:
-        pytest.skip("neither /root/reference nor oracle/_ref/ is present")
-    sys.modules.setdefault("dask", types.SimpleNamespace(delayed=lambda f=None, **kw: f))
-    loader = importlib.machinery.SourcelessFileLoader("ref_pyc_check", pyc)
-    mod = importlib.util.module_from_spec(importlib.util.spec_from_loader("ref_pyc_check", loader))
-    loader.exec_module(mod)
-    with open(os.path.join(ROOT, "tests", "golden", "g200.json")) as f:
-        fx = json.load(f)
-    case = next(c for c in fx["cases"] if c["k"] == 9 and c["limit"] == 1)
-    d = mod.build(fx["reads"], 9, 1)
-    assert sorted([km, c] for km, c in d.items()) == case["kmers"]
-
-
 def test_bench_line_guard_prints_once():
     """bench.py's watchdog: a stalled phase after the timed steps costs the extra keys, not the line."""
     code = r'''
@@ -174,6 +152,58 @@ print("main thread went on")
                           capture_output=True, text=True, timeout=60)
     lines = fine.stdout.strip().splitlines()
     assert fine.returncode == 0 and json.loads(lines[0])["value"] == 2 and lines[1] == "main thread went on" and len(lines) == 2
+
+
+@pytest.mark.parametrize("l", [12, 40])
+def test_bench_dump_outputs_do_not_depend_on_slot_order(tmp_path, l):
+    """bench.py --dump-outputs: the same graph with its ids in two different slot orders gives the same files, float64,
+    in key order (checked against the oracle's graph, whose ids are ranks in key order), sampled beyond max_rows."""
+    import importlib.util
+    import types
+    import _native as N
+    import oracle
+    from util import random_reads
+    spec = importlib.util.spec_from_file_location("bench", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    buf, off = oracle.pack_reads(random_reads(3, 200, genome_len=1500, lens=(60, 100), n_frac=0.0))
+    g = oracle.graph_build(buf, off, l, expand=False)
+    st = types.SimpleNamespace(n_kmer_windows=1, n_lmer_windows=2, distinct_lmers=g.nl, distinct_kmers=g.nv, edge_count=g.ne)
+
+    class SlotOrderContext:
+        def __init__(self, seed):
+            rng = np.random.default_rng(seed)
+            pl, pv = rng.permutation(g.nl), rng.permutation(g.nv)     # slot -> oracle id
+            inv = np.empty(g.nv, np.uint32)
+            inv[pv] = np.arange(g.nv)
+            self.arts = {N.ART_LMER_KEYS: g.lk_lo[pl], N.ART_LMER_KEYS_HI: g.lk_hi[pl], N.ART_LMER_VALUES: g.lvals[pl],
+                         N.ART_EDGE_V1: inv[g.ev1[pl]], N.ART_EDGE_V2: inv[g.ev2[pl]], N.ART_KMER_KEYS: g.vk_lo[pv],
+                         N.ART_KMER_KEYS_HI: g.vk_hi[pv], N.ART_LCOUNT: g.lcount.reshape(-1, 4)[pv].ravel(),
+                         N.ART_ECOUNT: g.ecount.reshape(-1, 4)[pv].ravel()}
+
+        def download(self, which):
+            return self.arts[which]
+
+    cap = g.nv // 2
+    for seed in (1, 2):
+        bench.dump_outputs(SlotOrderContext(seed), st, l, str(tmp_path / str(seed)), max_rows=cap)
+    names = sorted(os.listdir(tmp_path / "1"))
+    assert names == sorted(os.listdir(tmp_path / "2")) and len(names) == 10
+    d = {}
+    for n in names:
+        a, b = np.load(tmp_path / "1" / n), np.load(tmp_path / "2" / n)
+        assert a.dtype == np.float64 and np.array_equal(a, b), n
+        d[n[:-4]] = a.astype(np.uint64)
+    lr, vr = d["lmer_rows"], d["kmer_rows"]
+    assert lr.size == vr.size == cap and (np.diff(lr.astype(np.int64)) > 0).all()
+    words = [g.lk_hi >> np.uint64(32), g.lk_hi & np.uint64(0xFFFFFFFF)] if l > 32 else []
+    words += [g.lk_lo >> np.uint64(32), g.lk_lo & np.uint64(0xFFFFFFFF)]
+    assert np.array_equal(d["lmer_keys"], np.stack(words, axis=1)[lr])
+    assert np.array_equal(d["lmer_values"], g.lvals[lr])
+    assert np.array_equal(d["edge_v1"], g.ev1[lr]) and np.array_equal(d["edge_v2"], g.ev2[lr])
+    assert np.array_equal(d["kmer_keys"][:, -1], g.vk_lo[vr] & np.uint64(0xFFFFFFFF))
+    assert np.array_equal(d["lcount"], g.lcount.reshape(-1, 4)[vr]) and np.array_equal(d["ecount"], g.ecount.reshape(-1, 4)[vr])
+    assert d["counts"].tolist() == [1, 2, g.nl, g.nv, g.ne]
 
 
 def _bench_mock(args, world=1, stall=False, timeout=240):

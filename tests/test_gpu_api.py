@@ -435,3 +435,31 @@ def test_graph_equals_the_reference_derived_pins(ctx, name):
         check_graph_against_pins(pin, ctx.download(N.ART_KMER_KEYS), ctx.download(N.ART_LCOUNT), ctx.download(N.ART_ECOUNT),
                                  ctx.download(N.ART_LMER_KEYS), ctx.download(N.ART_LMER_VALUES), ctx.download(N.ART_EDGE_V1),
                                  ctx.download(N.ART_EDGE_V2), oracle.decode_key)
+
+
+def test_bench_dump_outputs_equal_the_oracle(tmp_path):
+    """bench.py --dump-outputs on the small workload: the files hold the graph of the oracle on the same reads, and a
+    second run with the same arguments writes the same files."""
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    for run in ("a", "b"):
+        subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--workload", "small_smoke", "--steps", "2", "--warmup", "1",
+                        "--no-e2e", "--no-cpu", "--no-extra", "--dump-outputs", str(tmp_path / run)], check=True, timeout=600,
+                       capture_output=True)
+    d = {}
+    for n in sorted(os.listdir(tmp_path / "a")):
+        a = np.load(tmp_path / "a" / n)
+        assert a.dtype == np.float64 and np.array_equal(a, np.load(tmp_path / "b" / n)), n
+        d[n[:-4]] = a.astype(np.uint64)
+    G, L, cov, l = 200_000, 100, 20, 32             # bench.py WORKLOADS["small_smoke"]
+    R = G * cov // L
+    g = oracle.graph_build(oracle.synth_reads(G, L, err_ppm=0, first=0, count=R), oracle.fixed_offsets(R, L), l, expand=False)
+    assert d["counts"].tolist() == [R * (L - l + 2), R * (L - l + 1), g.nl, g.nv, g.ne]
+    lr, vr = d["lmer_rows"], d["kmer_rows"]
+    assert lr.size == min(g.nl, 1 << 18) and vr.size == min(g.nv, 1 << 18)
+    assert np.array_equal(d["lmer_keys"], np.stack([g.lk_lo >> np.uint64(32), g.lk_lo & np.uint64(0xFFFFFFFF)], axis=1)[lr])
+    assert np.array_equal(d["lmer_values"], g.lvals[lr])
+    assert np.array_equal(d["edge_v1"], g.ev1[lr]) and np.array_equal(d["edge_v2"], g.ev2[lr])
+    assert np.array_equal(d["kmer_keys"], np.stack([g.vk_lo >> np.uint64(32), g.vk_lo & np.uint64(0xFFFFFFFF)], axis=1)[vr])
+    assert np.array_equal(d["lcount"], g.lcount.reshape(-1, 4)[vr]) and np.array_equal(d["ecount"], g.ecount.reshape(-1, 4)[vr])
