@@ -84,6 +84,12 @@ int euler_count_lmers(euler_ctx *ctx, const char *buf, const uint64_t *read_off,
  * (key,count) pairs with count > limit), ascending.  Same two-call protocol. len in [1,32]. */
 int euler_count_mers(euler_ctx *ctx, const char *buf, const uint64_t *read_off, uint64_t nreads,
                      uint32_t len, uint32_t limit, uint64_t *count, uint64_t *keys, uint32_t *values);
+/* euler_count_mers on two-word keys: bits 0..63 of each key in keys_lo, bits 64..127 in keys_hi, ascending in
+ * (hi, lo) order.  len in [1,64]; for len <= 32 keys_hi is all zero and the rest equals euler_count_mers.  Keys
+ * are canonical in the table, so len = 64 is counted although its poly-T key is all ones.  Same two-call protocol. */
+int euler_count_mers_wide(euler_ctx *ctx, const char *buf, const uint64_t *read_off, uint64_t nreads,
+                          uint32_t len, uint32_t limit, uint64_t *count, uint64_t *keys_lo, uint64_t *keys_hi,
+                          uint32_t *values);
 
 /* pygpuhash.create_hash_table_device (:262) / phase1 (:19) / copy_to_bucket (:77) / bucket_sort (:174):
  * open-addressing table.  capacity = euler_hash_capacity(n); TK/TV have `capacity` entries, empty
@@ -149,7 +155,9 @@ int euler_emit_contigs(euler_ctx *ctx, const euler_vertex *ev, uint32_t vcount, 
 /* referenceAssembler.build (:25-42) + all_contigs (:79-88) on device: unitigs of the both-strand
  * K-mer graph restricted to K-mers with count > limit.  Each unitig is written once, in one of its
  * two orientations; isolated cycles start at an implementation-chosen node.  '\n'-terminated
- * contigs; two-call protocol on out (NULL -> sizes).  K in [2,32]. */
+ * contigs; two-call protocol on out (NULL -> sizes).  K in [2,63]: K > 32 runs on two-word keys.
+ * K = 64 is refused because the two-word tables mark an empty slot with all ones, which is the
+ * poly-T 64-mer; every K-mer of K <= 63 bases leaves the top two bits of its high word clear. */
 int euler_unitigs(euler_ctx *ctx, const char *buf, const uint64_t *read_off, uint64_t nreads, uint32_t K,
                   uint32_t limit, char *out, uint64_t *out_bytes, uint64_t *ncontigs);
 
@@ -158,10 +166,16 @@ int euler_unitigs(euler_ctx *ctx, const char *buf, const uint64_t *read_off, uin
  * key present).  Output as euler_unitigs. */
 int euler_unitigs_from_kmers(euler_ctx *ctx, const uint64_t *keys, const uint32_t *counts, uint64_t n, uint32_t K,
                              char *out, uint64_t *out_bytes, uint64_t *ncontigs);
+/* the same on two-word keys (keys_lo / keys_hi as euler_count_mers_wide returns them).  K in [2,63]; for
+ * K <= 32 only keys_lo is read (keys_hi may be NULL) and the result is that of euler_unitigs_from_kmers. */
+int euler_unitigs_from_kmers_wide(euler_ctx *ctx, const uint64_t *keys_lo, const uint64_t *keys_hi, const uint32_t *counts,
+                                  uint64_t n, uint32_t K, char *out, uint64_t *out_bytes, uint64_t *ncontigs);
 /* Link graph G of referenceAssembler.all_contigs (:90-111) for n contigs: text = the contigs back to back
  * (no separators), off[n+1].  links: u32[16 n]; entry [16 i + 8 side + 2 base + o]: side 0 = candidates
  * fw(last K-mer of contig i), side 1 = fw(twin(first K-mer)); base = A,C,G,T; o = 0: contig whose head is the
- * candidate ('+'), o = 1: contig whose twin(tail) is ('-'); 0xffffffff = none.  K in [2,31]. */
+ * candidate ('+'), o = 1: contig whose twin(tail) is ('-'); 0xffffffff = none.  When two contigs share a head
+ * (or a twin(tail)), the later one is reported, as in the reference's dicts.  K in [2,63]: K >= 32 uses
+ * two-word end tables (the one-word tables' EMPTY key is the poly-T 32-mer; see euler_unitigs for 63). */
 int euler_unitig_links(euler_ctx *ctx, const char *text, const uint64_t *off, uint64_t n, uint32_t K, uint32_t *links);
 
 /* =========================================================================================

@@ -73,8 +73,10 @@ def load():
         "euler_compute_kmers": [vp, vp, u64, u64, vp, vp],
         "euler_count_lmers": [vp, vp, vp, u64, u32, vp, vp, vp, vp, vp, vp],
         "euler_count_mers": [vp, vp, vp, u64, u32, u32, vp, vp, vp],
+        "euler_count_mers_wide": [vp, vp, vp, u64, u32, u32, vp, vp, vp, vp],
         "euler_unitigs": [vp, vp, vp, u64, u32, u32, vp, vp, vp],
         "euler_unitigs_from_kmers": [vp, vp, vp, u64, u32, vp, vp, vp],
+        "euler_unitigs_from_kmers_wide": [vp, vp, vp, vp, u64, u32, vp, vp, vp],
         "euler_unitig_links": [vp, vp, vp, u64, u32, vp],
         "euler_hash_build": [vp, vp, vp, u64, u64, vp, vp],
         "euler_hash_lookup": [vp, vp, vp, u64, vp, u64, vp],
@@ -224,6 +226,21 @@ class Context:
                                                  C.byref(n), _p(keys), _p(vals)))
         return keys, vals
 
+    def count_mers_wide(self, buf, off, length, limit=0):
+        """count_mers for length 1..64: (keys_lo, keys_hi, vals), ascending in (hi, lo) order"""
+        buf = _arr(buf, np.uint8)
+        off = _arr(off, np.uint64)
+        n = C.c_uint64(0)
+        self.check(self.lib.euler_count_mers_wide(self.h, _p(buf), _p(off), len(off) - 1, int(length), int(limit),
+                                                  C.byref(n), None, None, None))
+        lo = np.zeros(n.value, np.uint64)
+        hi = np.zeros(n.value, np.uint64)
+        vals = np.zeros(n.value, np.uint32)
+        if n.value:
+            self.check(self.lib.euler_count_mers_wide(self.h, _p(buf), _p(off), len(off) - 1, int(length), int(limit),
+                                                      C.byref(n), _p(lo), _p(hi), _p(vals)))
+        return lo, hi, vals
+
     def unitigs(self, buf, off, K, limit=1):
         buf = _arr(buf, np.uint8)
         off = _arr(off, np.uint64)
@@ -238,19 +255,29 @@ class Context:
                                           C.byref(cap), C.byref(nc)))
         return out.tobytes().decode("ascii").split("\n")[:-1]
 
-    def unitigs_from_kmers(self, keys, counts, K):
-        """unitigs of a K-mer dictionary (packed keys, both-strand counts): referenceAssembler.all_contigs(d, k)"""
+    def unitigs_from_kmers(self, keys, counts, K, keys_hi=None):
+        """unitigs of a K-mer dictionary (packed keys, both-strand counts): referenceAssembler.all_contigs(d, k).
+        keys_hi: bits 64.. of the keys, needed when K > 32 (without it K > 32 is refused)."""
         keys = _arr(keys, np.uint64)
         counts = _arr(counts, np.uint32)
+        if keys_hi is None:
+            def call(out, nb, nc):
+                return self.lib.euler_unitigs_from_kmers(self.h, _p(keys), _p(counts), len(keys), int(K), out, nb, nc)
+        else:
+            keys_hi = _arr(keys_hi, np.uint64)
+            if keys_hi.size != keys.size:
+                raise EulerError("keys_hi has %d entries, keys %d" % (keys_hi.size, keys.size))
+
+            def call(out, nb, nc):
+                return self.lib.euler_unitigs_from_kmers_wide(self.h, _p(keys), _p(keys_hi), _p(counts), len(keys), int(K), out,
+                                                              nb, nc)
         nb, nc = C.c_uint64(0), C.c_uint64(0)
-        self.check(self.lib.euler_unitigs_from_kmers(self.h, _p(keys), _p(counts), len(keys), int(K), None, C.byref(nb),
-                                                     C.byref(nc)))
+        self.check(call(None, C.byref(nb), C.byref(nc)))
         if not nb.value:
             return []
         out = np.zeros(nb.value, np.uint8)
         cap = C.c_uint64(nb.value)
-        self.check(self.lib.euler_unitigs_from_kmers(self.h, _p(keys), _p(counts), len(keys), int(K), _p(out), C.byref(cap),
-                                                     C.byref(nc)))
+        self.check(call(_p(out), C.byref(cap), C.byref(nc)))
         return out.tobytes().decode("ascii").split("\n")[:-1]
 
     def unitig_links(self, contigs, K):

@@ -4,6 +4,7 @@
 (``src/cli_spark_gpu.py:37``: ``mapPartitions(assemble2)`` over read partitions), on the GPUs of one box.
 
     python assembler.py -i reads.fq -o contigs.fa -k 31                      # one GPU
+    python assembler.py -i reads.fq -o contigs.fa -k 63                      # one GPU, k up to 63
     python -m torch.distributed.run --nproc-per-node 8 --master-addr 127.0.0.1 \\
            assembler.py -i reads.fq -o contigs.fa -k 31                      # 8 GPUs, one assembly
 
@@ -19,7 +20,8 @@ Modes
                     graph and tour stages (euler_pipeline_run_lmers): same contigs as on one GPU.
   replicas          the reference's semantics: every rank assembles its own partition of the reads
                     independently and writes <out>.part<rank>.
-Outputs: FASTA contigs in -o, the GFA link graph in <out>.gfa (unitig mode).
+Outputs: FASTA contigs in -o, the GFA link graph in <out>.gfa (unitig mode).  k: 2..63 on one GPU and in
+replicas mode, 2..32 for one assembly across GPUs.
 """
 import argparse
 import logging
@@ -110,7 +112,7 @@ def main(argv=None):
     if world == 1 or args.mode == 'replicas':
         contigs = ctx.unitigs_ingested(K, args.limit) if nbases else []
         from referenceassembler import referenceAssembler as ram
-        G = ram.link_graph(contigs, K) if (contigs and K <= 31) else None
+        G = ram.link_graph(contigs, K) if (contigs and K <= 63) else None
         out = args.output_filename if world == 1 else "%s.part%d" % (args.output_filename, rank)
         write_outputs(out, contigs, G, K)
         log.info("rank %d: %d contigs -> %s", rank, len(contigs), out)
@@ -151,7 +153,7 @@ def main(argv=None):
                 contigs = ctx.pipeline_contigs()
         else:
             contigs = ctx.unitigs_from_kmers(all_k, all_v, K) if len(all_k) else []
-            G = ram.link_graph(contigs, K) if (contigs and K <= 31) else None
+            G = ram.link_graph(contigs, K) if (contigs and K <= 63) else None
         write_outputs(args.output_filename, contigs, G, K)
         log.info("%d k-mers joined, %d contigs -> %s", len(all_k), len(contigs), args.output_filename)
     dist.barrier()

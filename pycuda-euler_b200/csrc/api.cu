@@ -5,6 +5,7 @@
 #include "scan.cuh"
 #include "sort.cuh"
 #include "tmp.cuh"
+#include "wide.cuh"
 
 template <typename T>
 static int upload(euler_ctx *ctx, DevTmp<T> &d, const T *h, u64 n)
@@ -147,6 +148,64 @@ int euler_count_mers(euler_ctx *ctx, const char *buf, const uint64_t *read_off, 
     FINISH(ctx);
 }
 
+// euler_count_mers on two-word keys: len in [1,64]; len <= 32 is euler_count_mers with keys_hi all zero
+int euler_count_mers_wide(euler_ctx *ctx, const char *buf, const uint64_t *read_off, uint64_t nreads, uint32_t len,
+                          uint32_t limit, uint64_t *count, uint64_t *keys_lo, uint64_t *keys_hi, uint32_t *values)
+{
+    ENTER(ctx);
+    if (!read_off || !count) return euler_fail(ctx, EULER_ERR_ARG, "null argument");
+    if (len < 1 || len > 64) return euler_fail(ctx, EULER_ERR_ARG, "mer length %u out of range [1,64]", len);
+    const u64 out_cap = *count;
+    if (len <= 32) {
+        EULER_TRY(euler_count_mers(ctx, buf, read_off, nreads, len, limit, count, keys_lo, values));
+        if (keys_hi) {
+            if (out_cap < *count) return euler_fail(ctx, EULER_ERR_ARG, "output capacity too small (%llu < %llu)", out_cap, *count);
+            for (u64 i = 0; i < *count; i++) keys_hi[i] = 0;
+        }
+        return EULER_OK;
+    }
+    *count = 0;
+    const u64 B = read_off[nreads];
+    if (!B) return EULER_OK;
+    DevTmp<unsigned char> d_buf(ctx, B + 16);
+    DevTmp<u64> d_off(ctx, nreads + 1), d_stats(ctx, 8);
+    DevTmp<u32> d_bits(ctx, B / 32 + 2);
+    TMP_CHECK(ctx, d_bits); TMP_CHECK(ctx, d_stats);
+    EULER_TRY(upload(ctx, d_buf, (const unsigned char *)buf, B));
+    EULER_TRY(upload(ctx, d_off, (const u64 *)read_off, nreads + 1));
+    EULER_TRY(enc_mark_starts(ctx, d_off, nreads, B, d_bits));
+    const u64 cap = euler_hash_capacity(B);
+    DevTmp<K128> tk(ctx, cap);
+    DevTmp<u32> tc(ctx, cap), base(ctx, cap);
+    TMP_CHECK(ctx, tk); TMP_CHECK(ctx, tc); TMP_CHECK(ctx, base);
+    CUDA_TRY(ctx, cudaMemsetAsync(d_stats, 0, 8 * sizeof(u64), ctx->stream));
+    EULER_TRY(wide_table_clear(ctx, tk, tc, cap));
+    EULER_TRY(wide_count_tiled(ctx, d_buf, B, d_bits, len, tk, tc, cap, d_stats));
+    EULER_TRY(wide_slot_scan(ctx, tk, cap, len, base, d_stats.get() + 3));
+    u64 h[4];
+    EULER_TRY(read_u64s(ctx, d_stats, h, 4));
+    if (h[2]) return euler_fail(ctx, EULER_ERR_OVERFLOW, "count table overflow");
+    const u64 U = h[3];
+    if (!U) return EULER_OK;
+    DevTmp<u64> lo(ctx, U), hi(ctx, U), lo2(ctx, U), hi2(ctx, U);
+    DevTmp<u32> lv(ctx, U), lv2(ctx, U), fbase(ctx, U);
+    TMP_CHECK(ctx, lo); TMP_CHECK(ctx, hi); TMP_CHECK(ctx, lo2); TMP_CHECK(ctx, hi2); TMP_CHECK(ctx, lv); TMP_CHECK(ctx, lv2);
+    TMP_CHECK(ctx, fbase);
+    EULER_TRY(wide_compact_lmers(ctx, tk, tc, base, cap, len, lo, hi, lv));
+    EULER_TRY(wide_sort(ctx, lo, hi, lv, U, 2 * (int)len));
+    EULER_TRY(wide_filter_counts(ctx, lo, hi, lv, U, limit, fbase, lo2, hi2, lv2, d_stats.get() + 4));
+    u64 kept = 0;
+    EULER_TRY(read_u64(ctx, d_stats.get() + 4, &kept));
+    *count = kept;
+    if (keys_lo || keys_hi || values) {
+        if (out_cap < kept) return euler_fail(ctx, EULER_ERR_ARG, "output capacity too small (%llu < %llu)", out_cap, kept);
+        EULER_TRY(download(ctx, (u64 *)keys_lo, lo2.get(), kept));
+        EULER_TRY(download(ctx, (u64 *)keys_hi, hi2.get(), kept));
+        EULER_TRY(download(ctx, values, lv2.get(), kept));
+    }
+    FINISH(ctx);
+}
+
 static int unitigs_core(euler_ctx *ctx, const void *d_buf, const u64 *d_off, u64 nreads, u64 B, uint32_t K, uint32_t limit,
                         char *out, uint64_t *out_bytes, uint64_t *ncontigs)
 {
@@ -158,18 +217,31 @@ static int unitigs_core(euler_ctx *ctx, const void *d_buf, const u64 *d_off, u64
     TMP_CHECK(ctx, d_bits); TMP_CHECK(ctx, d_stats);
     EULER_TRY(enc_mark_starts(ctx, d_off, nreads, B, d_bits));
     const u64 cap = euler_hash_capacity(B);
-    DevTmp<u64> tk(ctx, cap);
-    DevTmp<u32> tc(ctx, cap);
-    TMP_CHECK(ctx, tk); TMP_CHECK(ctx, tc);
     CUDA_TRY(ctx, cudaMemsetAsync(d_stats, 0, 8 * sizeof(u64), ctx->stream));
-    EULER_TRY(graph_table_clear(ctx, tk, tc, cap));
-    EULER_TRY(enc_count_canonical(ctx, d_buf, B, d_bits, K, tk, tc, cap, TableHash{0, 0}, d_stats));
-    u64 h[3];
-    EULER_TRY(read_u64s(ctx, d_stats, h, 3));
-    if (h[2]) return euler_fail(ctx, EULER_ERR_OVERFLOW, "count table overflow");
     char *d_text = nullptr;
     u64 bytes = 0, nc = 0, nn = 0;
-    EULER_TRY(unitig_from_table(ctx, tk, tc, cap, K, limit, &d_text, &bytes, &nc, &nn));
+    if (K > 32) {
+        // two-word keys: the tiled 128-bit count of the pipeline (wide.cu) into a K128 table of the same capacity
+        DevTmp<K128> tk(ctx, cap);
+        DevTmp<u32> tc(ctx, cap);
+        TMP_CHECK(ctx, tk); TMP_CHECK(ctx, tc);
+        EULER_TRY(wide_table_clear(ctx, tk, tc, cap));
+        EULER_TRY(wide_count_tiled(ctx, d_buf, B, d_bits, K, tk, tc, cap, d_stats));
+        u64 h[3];
+        EULER_TRY(read_u64s(ctx, d_stats, h, 3));
+        if (h[2]) return euler_fail(ctx, EULER_ERR_OVERFLOW, "count table overflow");
+        EULER_TRY(wide_unitig_from_table(ctx, tk, tc, cap, K, limit, &d_text, &bytes, &nc, &nn));
+    } else {
+        DevTmp<u64> tk(ctx, cap);
+        DevTmp<u32> tc(ctx, cap);
+        TMP_CHECK(ctx, tk); TMP_CHECK(ctx, tc);
+        EULER_TRY(graph_table_clear(ctx, tk, tc, cap));
+        EULER_TRY(enc_count_canonical(ctx, d_buf, B, d_bits, K, tk, tc, cap, TableHash{0, 0}, d_stats));
+        u64 h[3];
+        EULER_TRY(read_u64s(ctx, d_stats, h, 3));
+        if (h[2]) return euler_fail(ctx, EULER_ERR_OVERFLOW, "count table overflow");
+        EULER_TRY(unitig_from_table(ctx, tk, tc, cap, K, limit, &d_text, &bytes, &nc, &nn));
+    }
     *out_bytes = bytes; *ncontigs = nc;
     if (out) {
         if (cap_out < bytes) return euler_fail(ctx, EULER_ERR_ARG, "output capacity too small");
@@ -184,7 +256,7 @@ int euler_unitigs(euler_ctx *ctx, const char *buf, const uint64_t *read_off, uin
 {
     ENTER(ctx);
     if (!read_off || !out_bytes || !ncontigs) return euler_fail(ctx, EULER_ERR_ARG, "null argument");
-    if (K < 2 || K > 32) return euler_fail(ctx, EULER_ERR_ARG, "K %u out of range [2,32]", K);
+    if (K < 2 || K > 63) return euler_fail(ctx, EULER_ERR_ARG, "K %u out of range [2,63]", K);
     const u64 B = read_off[nreads];
     DevTmp<unsigned char> d_buf(ctx, B + 16);
     DevTmp<u64> d_off(ctx, nreads + 1);
@@ -198,7 +270,7 @@ int euler_unitigs_ingested(euler_ctx *ctx, uint32_t K, uint32_t limit, char *out
 {
     ENTER(ctx);
     if (!out_bytes || !ncontigs) return euler_fail(ctx, EULER_ERR_ARG, "null argument");
-    if (K < 2 || K > 32) return euler_fail(ctx, EULER_ERR_ARG, "K %u out of range [2,32]", K);
+    if (K < 2 || K > 63) return euler_fail(ctx, EULER_ERR_ARG, "K %u out of range [2,63]", K);
     const void *d_buf; const u64 *d_off; u64 nr, nb;
     EULER_TRY(pipeline_resident_reads(ctx, &d_buf, &d_off, &nr, &nb));
     return unitigs_core(ctx, d_buf, d_off, nr, nb, K, limit, out, out_bytes, ncontigs);
@@ -237,6 +309,42 @@ int euler_unitigs_from_kmers(euler_ctx *ctx, const uint64_t *keys, const uint32_
     FINISH(ctx);
 }
 
+// euler_unitigs_from_kmers on two-word keys: K in [2,63]; K <= 32 reads keys_lo only (keys_hi may be NULL)
+int euler_unitigs_from_kmers_wide(euler_ctx *ctx, const uint64_t *keys_lo, const uint64_t *keys_hi, const uint32_t *counts,
+                                  uint64_t n, uint32_t K, char *out, uint64_t *out_bytes, uint64_t *ncontigs)
+{
+    ENTER(ctx);
+    if (K < 2 || K > 63) return euler_fail(ctx, EULER_ERR_ARG, "K %u out of range [2,63]", K);
+    if (K <= 32) return euler_unitigs_from_kmers(ctx, keys_lo, counts, n, K, out, out_bytes, ncontigs);
+    if (!out_bytes || !ncontigs || (n && (!keys_lo || !keys_hi || !counts))) return euler_fail(ctx, EULER_ERR_ARG, "null argument");
+    const u64 cap_out = *out_bytes;
+    *out_bytes = 0; *ncontigs = 0;
+    if (!n) return EULER_OK;
+    const u64 cap = euler_hash_capacity(n);
+    DevTmp<u64> dlo(ctx, n), dhi(ctx, n), flags(ctx, 1);
+    DevTmp<u32> dc(ctx, n), tc(ctx, cap);
+    DevTmp<K128> tk(ctx, cap);
+    TMP_CHECK(ctx, dlo); TMP_CHECK(ctx, dhi); TMP_CHECK(ctx, dc); TMP_CHECK(ctx, tk); TMP_CHECK(ctx, tc); TMP_CHECK(ctx, flags);
+    EULER_TRY(upload(ctx, dlo, (const u64 *)keys_lo, n));
+    EULER_TRY(upload(ctx, dhi, (const u64 *)keys_hi, n));
+    EULER_TRY(upload(ctx, dc, counts, n));
+    CUDA_TRY(ctx, cudaMemsetAsync(flags, 0, sizeof(u64), ctx->stream));
+    EULER_TRY(wide_table_clear(ctx, tk, tc, cap));
+    EULER_TRY(wide_unitig_dict_table(ctx, dlo, dhi, dc, n, K, tk, tc, cap, flags));
+    u64 f = 0;
+    EULER_TRY(read_u64(ctx, flags, &f));
+    if (f) return euler_fail(ctx, EULER_ERR_OVERFLOW, "K-mer table full");
+    char *d_text = nullptr;
+    u64 bytes = 0, nc = 0, nn = 0;
+    EULER_TRY(wide_unitig_from_table(ctx, tk, tc, cap, K, 0, &d_text, &bytes, &nc, &nn));
+    *out_bytes = bytes; *ncontigs = nc;
+    if (out) {
+        if (cap_out < bytes) return euler_fail(ctx, EULER_ERR_ARG, "output capacity too small");
+        EULER_TRY(download(ctx, out, (const char *)d_text, bytes));
+    }
+    FINISH(ctx);
+}
+
 // link graph G of referenceAssembler.all_contigs :90-111 for n contigs (text: the contigs back to back, no
 // separators; off[n+1]).  links: u32[16 n], entry [16 i + 8 side + 2 base + o]: side 0 = successors of the last
 // K-mer, side 1 = of twin(first K-mer); o = 0: the hit is a contig head ('+'), o = 1: a tail ('-'); 0xffffffff = none.
@@ -244,7 +352,7 @@ int euler_unitig_links(euler_ctx *ctx, const char *text, const uint64_t *off, ui
 {
     ENTER(ctx);
     if (n && (!text || !off || !links)) return euler_fail(ctx, EULER_ERR_ARG, "null argument");
-    if (K < 2 || K > 31) return euler_fail(ctx, EULER_ERR_ARG, "K %u out of range [2,31]", K);
+    if (K < 2 || K > 63) return euler_fail(ctx, EULER_ERR_ARG, "K %u out of range [2,63]", K);
     if (!n) return EULER_OK;
     if (n >= 0xfffffffeull) return euler_fail(ctx, EULER_ERR_RANGE, "too many contigs");
     const u64 B = off[n];
@@ -254,7 +362,9 @@ int euler_unitig_links(euler_ctx *ctx, const char *text, const uint64_t *off, ui
     TMP_CHECK(ctx, d_text); TMP_CHECK(ctx, d_off); TMP_CHECK(ctx, d_links);
     EULER_TRY(upload(ctx, d_text, text, B));
     EULER_TRY(upload(ctx, d_off, (const u64 *)off, n + 1));
-    EULER_TRY(unitig_link_graph(ctx, d_text, d_off, n, K, d_links));
+    // the 64-bit end tables use the all-ones word as EMPTY, which is the poly-T 32-mer: K >= 32 takes 128-bit tables
+    if (K >= 32) EULER_TRY(wide_unitig_link_graph(ctx, d_text, d_off, n, K, d_links));
+    else EULER_TRY(unitig_link_graph(ctx, d_text, d_off, n, K, d_links));
     EULER_TRY(download(ctx, links, d_links.get(), 16 * n));
     FINISH(ctx);
 }

@@ -149,6 +149,18 @@ int wide_assign_sorted_ids(euler_ctx *ctx, const u64 *vk_lo, const u64 *vk_hi, u
 int wide_degree_slots(euler_ctx *ctx, const u64 *lk_lo, const u64 *lk_hi, const u32 *lvals, u64 nl, u32 l, const K128 *vt_keys,
                       const u32 *id0, const u32 *id1, u64 vt_cap, u32 *lcount, u32 *ecount, u32 *ev1, u32 *ev2, unsigned char *tf);
 
+// ---- wide_unitig.cu (unitig stage, K = 33..63; link graph, K = 32..63)
+int wide_unitig_from_table(euler_ctx *ctx, const K128 *keys, const u32 *cnt, u64 cap, u32 K, u32 limit, char **d_out,
+                           u64 *out_bytes, u64 *ncontigs, u64 *n_nodes);
+// canonical count table from a both-strand K-mer dictionary (keys as lo / hi words, counts)
+int wide_unitig_dict_table(euler_ctx *ctx, const u64 *d_lo, const u64 *d_hi, const u32 *d_counts, u64 n, u32 K, K128 *tk, u32 *tc,
+                           u64 cap, u64 *d_flags);
+// links[16 i + 8 side + 2 base + (0 head '+' | 1 tail '-')] of n contigs (text without separators, off[n+1])
+int wide_unitig_link_graph(euler_ctx *ctx, const char *d_text, const u64 *d_off, u64 n, u32 K, u32 *d_links);
+// (key, count) filter: keep count > limit, compact
+int wide_filter_counts(euler_ctx *ctx, const u64 *lo, const u64 *hi, const u32 *vals, u64 n, u32 limit, u32 *d_base, u64 *out_lo,
+                       u64 *out_hi, u32 *out_vals, u64 *d_total);
+
 // ---- wide_dist.cu (k-mer-space partition over 16-byte keys)
 int wide_dist_scatter(euler_ctx *ctx, const void *d_buf, const u64 *d_off, u64 nreads, u32 l, u32 nranks, u64 *d_counts,
                       u64 *d_cursors, void *d_send, const u64 *d_seg_off, u64 seg_cap);

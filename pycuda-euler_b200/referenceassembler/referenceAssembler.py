@@ -4,11 +4,12 @@ with its hot loops on the GPU.
 Same names, arguments and return values as the reference:
 
 * ``build(reads, k=31, limit=1)`` (:25-42)  -> ``dict {kmer: count}`` over both strands, reads split at
-  ``N``, entries with ``count <= limit`` dropped.  Counting runs in ``euler_count_mers``.
+  ``N``, entries with ``count <= limit`` dropped.  Counting runs in ``euler_count_mers_wide``; k <= 64.
 * ``all_contigs(d, k)`` (:79-111)           -> ``(G, contigs)``.  The unitigs come from
-  ``euler_unitigs_from_kmers`` (each unitig once, in one of its two orientations; the reference's order
-  and orientation follow its dict order, so compare as orientation-free sets), the link graph ``G`` from
-  ``euler_unitig_links`` -- for a given contig list it is exactly the reference's ``G``.
+  ``euler_unitigs_from_kmers`` / ``_wide`` (each unitig once, in one of its two orientations; the reference's
+  order and orientation follow its dict order, so compare as orientation-free sets), the link graph ``G`` from
+  ``euler_unitig_links`` -- for a given contig list it is exactly the reference's ``G``.  k <= 63: the
+  library's two-word tables mark an empty slot with all ones, the key of the poly-T 64-mer.
 * ``get_contig`` / ``get_contig_forward`` (:47-77), string helpers ``twin kmers fw bw contig_to_string``
   (:7-23, :44-45), ``print_GFA`` / ``print_dbg`` (:115-130), ``runAssembler`` (:135-).
 
@@ -59,34 +60,55 @@ def _pack(reads):
     return buf, off
 
 
-def _decode(keys, k):
-    """packed 2-bit keys (MSB first) -> list of strings, vectorised"""
+_CODE_OF = np.full(256, 255, np.uint8)
+_CODE_OF[np.frombuffer(b"ACGT", np.uint8)] = np.arange(4, dtype=np.uint8)
+
+
+def _decode(keys, k, keys_hi=None):
+    """packed 2-bit keys (MSB first; bits 64.. in keys_hi when k > 32) -> list of strings, vectorised"""
     if len(keys) == 0:
         return []
     shifts = (2 * (k - 1 - np.arange(k))).astype(np.uint64)
-    codes = ((keys[:, None] >> shifts[None, :]) & np.uint64(3)).astype(np.uint8)
+    low = shifts < 64
+    codes = np.empty((len(keys), k), np.uint8)
+    codes[:, low] = (keys[:, None] >> shifts[None, low]) & np.uint64(3)
+    if not low.all():
+        codes[:, ~low] = (keys_hi[:, None] >> (shifts[None, ~low] - np.uint64(64))) & np.uint64(3)
     text = np.frombuffer(b"ACGT", dtype=np.uint8)[codes]
     return [row.tobytes().decode("ascii") for row in text]
 
 
 def _encode(kms, k):
-    out = np.zeros(len(kms), np.uint64)
-    for i, km in enumerate(kms):
-        x = 0
-        for ch in km:
-            x = (x << 2) | _CODE[ch]
-        out[i] = x
-    return out
+    """strings of length k -> (lo, hi): the 2-bit packed keys (MSB first), bits 64.. in hi, vectorised"""
+    n = len(kms)
+    lo = np.zeros(n, np.uint64)
+    hi = np.zeros(n, np.uint64)
+    if n == 0:
+        return lo, hi
+    data = "".join(kms).encode("ascii")
+    if len(data) != n * k:
+        raise ValueError("every k-mer must have length k = %d" % k)
+    codes = _CODE_OF[np.frombuffer(data, np.uint8).reshape(n, k)]
+    if (codes == 255).any():
+        raise ValueError("k-mers must be spelled in A, C, G, T")
+    codes = codes.astype(np.uint64)
+    for j in range(k):
+        s = 2 * (k - 1 - j)
+        if s < 64:
+            lo |= codes[:, j] << np.uint64(s)
+        else:
+            hi |= codes[:, j] << np.uint64(s - 64)
+    return lo, hi
 
 
 def build(reads, k=31, limit=1):
-    """referenceAssembler.build (:25-42) on the GPU"""
+    """referenceAssembler.build (:25-42) on the GPU; k <= 64"""
     reads = list(reads)
     buf, off = _pack(reads)
     if buf.size == 0:
         return {}
-    keys, vals = _native.default_context().count_mers(buf, off, int(k), int(limit))
-    return dict(zip(_decode(keys, int(k)), (int(v) for v in vals)))
+    lo, hi, vals = _native.default_context().count_mers_wide(buf, off, int(k), int(limit))
+    return dict(zip(_decode(lo, int(k), hi), (int(v) for v in vals)))
 
 
 def _links_to_G(links):
@@ -116,9 +138,9 @@ def all_contigs(d, k):
     if not d:
         return {}, []
     kms = list(d.keys())
-    keys = _encode(kms, k)
+    lo, hi = _encode(kms, k)
     counts = np.fromiter((int(d[x]) for x in kms), dtype=np.uint32, count=len(kms))
-    r = _native.default_context().unitigs_from_kmers(keys, counts, k)
+    r = _native.default_context().unitigs_from_kmers(lo, counts, k, keys_hi=hi if k > 32 else None)
     return link_graph(r, k), r
 
 
