@@ -178,6 +178,40 @@ int euler_unitigs_from_kmers_wide(euler_ctx *ctx, const uint64_t *keys_lo, const
  * two-word end tables (the one-word tables' EMPTY key is the poly-T 32-mer; see euler_unitigs for 63). */
 int euler_unitig_links(euler_ctx *ctx, const char *text, const uint64_t *off, uint64_t n, uint32_t K, uint32_t *links);
 
+/* Graph clean-up before the unitigs are written: tips, isolated fragments and bubble branches, the marks that
+ * sequencing errors leave in the graph of euler_unitigs.  Each round looks at every path unitig U = (h .. t) of the
+ * current node set on both strands, with L = its K-mers, cov = floor(65536 * sum of their both-strand counts / L),
+ * in = alive backward extensions of h, out = alive forward extensions of t, and removes U (and its twin) when
+ *   isolated:       in = out = {} and L <= isolated_len;
+ *   tip:            out = {}, in = {p}, L <= tip_len and cov < the largest cov of the unitigs headed by p's other
+ *                   successors (there must be one);
+ *   bubble branch:  in = {P}, out = {S}, L <= bubble_len and cov < the largest cov of the unitigs with the same
+ *                   (P, S) and L <= bubble_len.
+ * Cycles stay.  Every decision of a round sees the same node set; rounds repeat until one removes nothing or
+ * max_rounds have run.  Comparisons are strict and nothing depends on node ids or thread order, so the output set
+ * is a function of the K-mer counts alone.  A length of 0 turns its rule off; all three at 0 give euler_unitigs. */
+typedef struct { uint32_t tip_len, isolated_len, bubble_len, max_rounds; } euler_clean_params;
+typedef struct {
+    uint32_t rounds;            /* rounds that removed something */
+    uint64_t tips, isolated, bubble_branches;   /* unitigs removed, once per strand pair */
+    uint64_t kmers_removed;     /* canonical K-mers removed */
+} euler_clean_stats;
+/* euler_unitigs after the clean-up, plus kmer_sums[i] = sum of the both-strand counts of the K-mers of contig i (in
+ * output order; the mean K-mer coverage is kmer_sums[i] / (len - K + 1)).  Two-call protocol: with out and kmer_sums
+ * NULL the call returns the sizes; then out has *out_bytes bytes and kmer_sums *ncontigs entries.  stats may be
+ * NULL.  K in [2,63]. */
+int euler_unitigs_clean(euler_ctx *ctx, const char *buf, const uint64_t *read_off, uint64_t nreads, uint32_t K,
+                        uint32_t limit, const euler_clean_params *params, char *out, uint64_t *out_bytes,
+                        uint64_t *ncontigs, uint64_t *kmer_sums, euler_clean_stats *stats);
+/* the same on the reads left on the device by euler_ingest */
+int euler_unitigs_clean_ingested(euler_ctx *ctx, uint32_t K, uint32_t limit, const euler_clean_params *params, char *out,
+                                 uint64_t *out_bytes, uint64_t *ncontigs, uint64_t *kmer_sums, euler_clean_stats *stats);
+/* the same on a K-mer dictionary, as euler_unitigs_from_kmers_wide (K <= 32 reads keys_lo only) */
+int euler_unitigs_clean_from_kmers_wide(euler_ctx *ctx, const uint64_t *keys_lo, const uint64_t *keys_hi,
+                                        const uint32_t *counts, uint64_t n, uint32_t K, const euler_clean_params *params,
+                                        char *out, uint64_t *out_bytes, uint64_t *ncontigs, uint64_t *kmer_sums,
+                                        euler_clean_stats *stats);
+
 /* =========================================================================================
  * Fused device-resident pipeline (the measured hot path)
  * ======================================================================================= */

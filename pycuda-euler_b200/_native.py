@@ -52,6 +52,18 @@ class Stats(C.Structure):
         return {k: getattr(self, k) for k, _ in self._fields_}
 
 
+class CleanParams(C.Structure):
+    _fields_ = [("tip_len", C.c_uint32), ("isolated_len", C.c_uint32), ("bubble_len", C.c_uint32), ("max_rounds", C.c_uint32)]
+
+
+class CleanStats(C.Structure):
+    _fields_ = [("rounds", C.c_uint32), ("tips", C.c_uint64), ("isolated", C.c_uint64), ("bubble_branches", C.c_uint64),
+                ("kmers_removed", C.c_uint64)]
+
+    def as_dict(self):
+        return {k: int(getattr(self, k)) for k, _ in self._fields_}
+
+
 _lib = None
 
 
@@ -78,6 +90,9 @@ def load():
         "euler_unitigs_from_kmers": [vp, vp, vp, u64, u32, vp, vp, vp],
         "euler_unitigs_from_kmers_wide": [vp, vp, vp, vp, u64, u32, vp, vp, vp],
         "euler_unitig_links": [vp, vp, vp, u64, u32, vp],
+        "euler_unitigs_clean": [vp, vp, vp, u64, u32, u32, vp, vp, vp, vp, vp, vp],
+        "euler_unitigs_clean_ingested": [vp, u32, u32, vp, vp, vp, vp, vp, vp],
+        "euler_unitigs_clean_from_kmers_wide": [vp, vp, vp, vp, u64, u32, vp, vp, vp, vp, vp, vp],
         "euler_hash_build": [vp, vp, vp, u64, u64, vp, vp],
         "euler_hash_lookup": [vp, vp, vp, u64, vp, u64, vp],
         "euler_exclusive_scan_u32": [vp, vp, u64, vp],
@@ -279,6 +294,55 @@ class Context:
         cap = C.c_uint64(nb.value)
         self.check(call(_p(out), C.byref(cap), C.byref(nc)))
         return out.tobytes().decode("ascii").split("\n")[:-1]
+
+    def _clean_call(self, call, K, tip_len, isolated_len, bubble_len, max_rounds):
+        """two-call protocol of the euler_unitigs_clean* entry points -> (contigs, kmer_sums, stats dict)"""
+        dflt = 2 * int(K)
+        p = CleanParams(dflt if tip_len is None else int(tip_len), dflt if isolated_len is None else int(isolated_len),
+                        dflt if bubble_len is None else int(bubble_len), int(max_rounds))
+        st = CleanStats()
+        nb, nc = C.c_uint64(0), C.c_uint64(0)
+        self.check(call(C.byref(p), None, C.byref(nb), C.byref(nc), None, C.byref(st)))
+        if not nb.value:
+            return [], np.zeros(0, np.uint64), st.as_dict()
+        out = np.zeros(nb.value, np.uint8)
+        sums = np.zeros(nc.value, np.uint64)
+        cap, nc2 = C.c_uint64(nb.value), C.c_uint64(nc.value)
+        self.check(call(C.byref(p), _p(out), C.byref(cap), C.byref(nc2), _p(sums), C.byref(st)))
+        return out.tobytes().decode("ascii").split("\n")[:-1], sums, st.as_dict()
+
+    def unitigs_clean(self, buf, off, K, limit=1, tip_len=None, isolated_len=None, bubble_len=None, max_rounds=10):
+        """unitigs after clipping tips, dropping isolated fragments and popping bubbles (euler_unitigs_clean):
+        (contigs, kmer_sums, stats).  kmer_sums[i] = sum of the both-strand counts of contig i's K-mers.  A length of
+        None means 2 K, 0 turns its rule off."""
+        buf = _arr(buf, np.uint8)
+        off = _arr(off, np.uint64)
+
+        def call(p, out, nb, nc, sums, st):
+            return self.lib.euler_unitigs_clean(self.h, _p(buf), _p(off), len(off) - 1, int(K), int(limit), p, out, nb, nc,
+                                                sums, st)
+        return self._clean_call(call, K, tip_len, isolated_len, bubble_len, max_rounds)
+
+    def unitigs_clean_ingested(self, K, limit=1, tip_len=None, isolated_len=None, bubble_len=None, max_rounds=10):
+        """unitigs_clean on the reads left resident by ingest"""
+        def call(p, out, nb, nc, sums, st):
+            return self.lib.euler_unitigs_clean_ingested(self.h, int(K), int(limit), p, out, nb, nc, sums, st)
+        return self._clean_call(call, K, tip_len, isolated_len, bubble_len, max_rounds)
+
+    def unitigs_clean_from_kmers(self, keys, counts, K, keys_hi=None, tip_len=None, isolated_len=None, bubble_len=None,
+                                 max_rounds=10):
+        """unitigs_clean on a K-mer dictionary (as unitigs_from_kmers; keys_hi is needed when K > 32)"""
+        keys = _arr(keys, np.uint64)
+        counts = _arr(counts, np.uint32)
+        if keys_hi is not None:
+            keys_hi = _arr(keys_hi, np.uint64)
+            if keys_hi.size != keys.size:
+                raise EulerError("keys_hi has %d entries, keys %d" % (keys_hi.size, keys.size))
+
+        def call(p, out, nb, nc, sums, st):
+            return self.lib.euler_unitigs_clean_from_kmers_wide(self.h, _p(keys), _p(keys_hi), _p(counts), len(keys), int(K), p,
+                                                                out, nb, nc, sums, st)
+        return self._clean_call(call, K, tip_len, isolated_len, bubble_len, max_rounds)
 
     def unitig_links(self, contigs, K):
         """(n, 16) uint32 link table of referenceAssembler.all_contigs' G (see euler_unitig_links)"""

@@ -5,6 +5,7 @@
 
     python assembler.py -i reads.fq -o contigs.fa -k 31                      # one GPU
     python assembler.py -i reads.fq -o contigs.fa -k 63                      # one GPU, k up to 63
+    python assembler.py -i reads.fq -o contigs.fa -k 31 --clean              # clip tips, pop bubbles first
     python -m torch.distributed.run --nproc-per-node 8 --master-addr 127.0.0.1 \\
            assembler.py -i reads.fq -o contigs.fa -k 31                      # 8 GPUs, one assembly
 
@@ -22,6 +23,12 @@ Modes
                     independently and writes <out>.part<rank>.
 Outputs: FASTA contigs in -o, the GFA link graph in <out>.gfa (unitig mode).  k: 2..63 on one GPU and in
 replicas mode, 2..32 for one assembly across GPUs.
+
+--clean (unitig and replicas modes) removes what sequencing errors leave in the graph before the unitigs are
+written: tips (dead-end branches), isolated fragments and the weaker branches of bubbles, each up to a length in
+K-mers (--tip-len, --isolated-len, --bubble-len; default 2k, 0 turns a rule off), for up to --clean-rounds rounds
+(rules: include/euler_b200.h, euler_unitigs_clean).  The GFA's S lines then carry KC:i:<sum of the contig's K-mer
+counts>, and the log gets a line with the rounds and the removals.
 """
 import argparse
 import logging
@@ -67,13 +74,22 @@ def split_records(data, world, fmt):
     return [(cuts[r], cuts[r + 1]) for r in range(world)]
 
 
-def write_outputs(path, contigs, G, k):
+def write_outputs(path, contigs, G, k, kc=None):
     from referenceassembler import referenceAssembler as ram
     with open(path, "w") as f:
         ram.write_fasta(contigs, f)
     if G is not None:
         with open(path + ".gfa", "w") as f:
-            ram.write_gfa(G, contigs, k, f)
+            ram.write_gfa(G, contigs, k, f, kc=kc)
+
+
+def clean_kwargs(args):
+    return dict(tip_len=args.tip_len, isolated_len=args.isolated_len, bubble_len=args.bubble_len, max_rounds=args.clean_rounds)
+
+
+def log_clean(log, rank, st):
+    log.info("rank %d: clean-up: %d rounds, %d tips, %d isolated, %d bubble branches, %d K-mers removed", rank, st["rounds"],
+             st["tips"], st["isolated"], st["bubble_branches"], st["kmers_removed"])
 
 
 def main(argv=None):
@@ -84,6 +100,11 @@ def main(argv=None):
     ap.add_argument('-d', action='store_true', default=False, help='Use DDFS (accepted for compatibility; ignored)')
     ap.add_argument('--limit', type=int, default=1, help='keep k-mers with both-strand count > limit (build() default 1)')
     ap.add_argument('--mode', choices=['unitig', 'euler', 'replicas'], default='unitig')
+    ap.add_argument('--clean', action='store_true', help='clip tips, drop isolated fragments and pop bubbles (unitig routes)')
+    ap.add_argument('--tip-len', type=int, default=None, help='longest tip removed, in K-mers (default 2k; 0 = off)')
+    ap.add_argument('--isolated-len', type=int, default=None, help='longest isolated fragment removed, in K-mers (default 2k)')
+    ap.add_argument('--bubble-len', type=int, default=None, help='longest bubble branch removed, in K-mers (default 2k)')
+    ap.add_argument('--clean-rounds', type=int, default=10, help='most clean-up rounds')
     args = ap.parse_args(argv)
     logging.basicConfig(level=logging.INFO, format='%(asctime)s %(levelname)s %(message)s')
     log = logging.getLogger("assembler")
@@ -110,11 +131,17 @@ def main(argv=None):
         log.info("%d contigs -> %s", len(contigs), args.output_filename)
         return 0
     if world == 1 or args.mode == 'replicas':
-        contigs = ctx.unitigs_ingested(K, args.limit) if nbases else []
+        kc = None
+        if args.clean:
+            contigs, kc, st = ctx.unitigs_clean_ingested(K, args.limit, **clean_kwargs(args)) if nbases else ([], None, None)
+            if st:
+                log_clean(log, rank, st)
+        else:
+            contigs = ctx.unitigs_ingested(K, args.limit) if nbases else []
         from referenceassembler import referenceAssembler as ram
         G = ram.link_graph(contigs, K) if (contigs and K <= 63) else None
         out = args.output_filename if world == 1 else "%s.part%d" % (args.output_filename, rank)
-        write_outputs(out, contigs, G, K)
+        write_outputs(out, contigs, G, K, kc)
         log.info("rank %d: %d contigs -> %s", rank, len(contigs), out)
         return 0
 
@@ -146,15 +173,20 @@ def main(argv=None):
         all_k = np.concatenate([g[0] for g in gathered])
         all_v = np.concatenate([g[1] for g in gathered])
         from referenceassembler import referenceAssembler as ram
+        kc = None
         if args.mode == 'euler':
             contigs, G = [], None
             if len(all_k):
                 ctx.run_lmers(all_k, all_v, K, N.RUN_CANONICAL_IDS | N.RUN_EXPAND_EDGES)
                 contigs = ctx.pipeline_contigs()
         else:
-            contigs = ctx.unitigs_from_kmers(all_k, all_v, K) if len(all_k) else []
+            if args.clean and len(all_k):
+                contigs, kc, st = ctx.unitigs_clean_from_kmers(all_k, all_v, K, **clean_kwargs(args))
+                log_clean(log, rank, st)
+            else:
+                contigs = ctx.unitigs_from_kmers(all_k, all_v, K) if len(all_k) else []
             G = ram.link_graph(contigs, K) if (contigs and K <= 63) else None
-        write_outputs(args.output_filename, contigs, G, K)
+        write_outputs(args.output_filename, contigs, G, K, kc)
         log.info("%d k-mers joined, %d contigs -> %s", len(all_k), len(contigs), args.output_filename)
     dist.barrier()
     dist.destroy_process_group()

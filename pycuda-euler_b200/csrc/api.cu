@@ -206,10 +206,13 @@ int euler_count_mers_wide(euler_ctx *ctx, const char *buf, const uint64_t *read_
     FINISH(ctx);
 }
 
+// cp != NULL: the unitigs after the graph clean-up (clean.cu), with per-contig count sums (sums: *ncontigs entries on
+// entry, may be NULL) and stats
 static int unitigs_core(euler_ctx *ctx, const void *d_buf, const u64 *d_off, u64 nreads, u64 B, uint32_t K, uint32_t limit,
-                        char *out, uint64_t *out_bytes, uint64_t *ncontigs)
+                        char *out, uint64_t *out_bytes, uint64_t *ncontigs, const euler_clean_params *cp = nullptr,
+                        uint64_t *sums = nullptr, euler_clean_stats *st = nullptr)
 {
-    const u64 cap_out = *out_bytes;
+    const u64 cap_out = *out_bytes, cap_sums = *ncontigs;
     *out_bytes = 0; *ncontigs = 0;
     if (!B) return EULER_OK;
     DevTmp<u64> d_stats(ctx, 8);
@@ -230,7 +233,8 @@ static int unitigs_core(euler_ctx *ctx, const void *d_buf, const u64 *d_off, u64
         u64 h[3];
         EULER_TRY(read_u64s(ctx, d_stats, h, 3));
         if (h[2]) return euler_fail(ctx, EULER_ERR_OVERFLOW, "count table overflow");
-        EULER_TRY(wide_unitig_from_table(ctx, tk, tc, cap, K, limit, &d_text, &bytes, &nc, &nn));
+        if (cp) EULER_TRY(wide_unitig_clean_from_table(ctx, tk, tc, cap, K, limit, *cp, &d_text, &bytes, &nc, (u64 *)sums, cap_sums, st));
+        else EULER_TRY(wide_unitig_from_table(ctx, tk, tc, cap, K, limit, &d_text, &bytes, &nc, &nn));
     } else {
         DevTmp<u64> tk(ctx, cap);
         DevTmp<u32> tc(ctx, cap);
@@ -240,7 +244,8 @@ static int unitigs_core(euler_ctx *ctx, const void *d_buf, const u64 *d_off, u64
         u64 h[3];
         EULER_TRY(read_u64s(ctx, d_stats, h, 3));
         if (h[2]) return euler_fail(ctx, EULER_ERR_OVERFLOW, "count table overflow");
-        EULER_TRY(unitig_from_table(ctx, tk, tc, cap, K, limit, &d_text, &bytes, &nc, &nn));
+        if (cp) EULER_TRY(unitig_clean_from_table(ctx, tk, tc, cap, K, limit, *cp, &d_text, &bytes, &nc, (u64 *)sums, cap_sums, st));
+        else EULER_TRY(unitig_from_table(ctx, tk, tc, cap, K, limit, &d_text, &bytes, &nc, &nn));
     }
     *out_bytes = bytes; *ncontigs = nc;
     if (out) {
@@ -338,6 +343,96 @@ int euler_unitigs_from_kmers_wide(euler_ctx *ctx, const uint64_t *keys_lo, const
     u64 bytes = 0, nc = 0, nn = 0;
     EULER_TRY(wide_unitig_from_table(ctx, tk, tc, cap, K, 0, &d_text, &bytes, &nc, &nn));
     *out_bytes = bytes; *ncontigs = nc;
+    if (out) {
+        if (cap_out < bytes) return euler_fail(ctx, EULER_ERR_ARG, "output capacity too small");
+        EULER_TRY(download(ctx, out, (const char *)d_text, bytes));
+    }
+    FINISH(ctx);
+}
+
+static int clean_args(euler_ctx *ctx, uint32_t K, const euler_clean_params *params, uint64_t *out_bytes, uint64_t *ncontigs,
+                      euler_clean_stats *stats)
+{
+    if (!params || !out_bytes || !ncontigs) return euler_fail(ctx, EULER_ERR_ARG, "null argument");
+    if (K < 2 || K > 63) return euler_fail(ctx, EULER_ERR_ARG, "K %u out of range [2,63]", K);
+    if (stats) *stats = euler_clean_stats{};
+    return EULER_OK;
+}
+
+int euler_unitigs_clean(euler_ctx *ctx, const char *buf, const uint64_t *read_off, uint64_t nreads, uint32_t K, uint32_t limit,
+                        const euler_clean_params *params, char *out, uint64_t *out_bytes, uint64_t *ncontigs,
+                        uint64_t *kmer_sums, euler_clean_stats *stats)
+{
+    ENTER(ctx);
+    if (!read_off) return euler_fail(ctx, EULER_ERR_ARG, "null argument");
+    EULER_TRY(clean_args(ctx, K, params, out_bytes, ncontigs, stats));
+    euler_clean_stats st{};
+    const u64 B = read_off[nreads];
+    DevTmp<unsigned char> d_buf(ctx, B + 16);
+    DevTmp<u64> d_off(ctx, nreads + 1);
+    EULER_TRY(upload(ctx, d_buf, (const unsigned char *)buf, B));
+    EULER_TRY(upload(ctx, d_off, (const u64 *)read_off, nreads + 1));
+    EULER_TRY(unitigs_core(ctx, d_buf, d_off, nreads, B, K, limit, out, out_bytes, ncontigs, params, kmer_sums, &st));
+    if (stats) *stats = st;
+    return EULER_OK;
+}
+
+int euler_unitigs_clean_ingested(euler_ctx *ctx, uint32_t K, uint32_t limit, const euler_clean_params *params, char *out,
+                                 uint64_t *out_bytes, uint64_t *ncontigs, uint64_t *kmer_sums, euler_clean_stats *stats)
+{
+    ENTER(ctx);
+    EULER_TRY(clean_args(ctx, K, params, out_bytes, ncontigs, stats));
+    euler_clean_stats st{};
+    const void *d_buf; const u64 *d_off; u64 nr, nb;
+    EULER_TRY(pipeline_resident_reads(ctx, &d_buf, &d_off, &nr, &nb));
+    EULER_TRY(unitigs_core(ctx, d_buf, d_off, nr, nb, K, limit, out, out_bytes, ncontigs, params, kmer_sums, &st));
+    if (stats) *stats = st;
+    return EULER_OK;
+}
+
+// the dictionary's counts are all kept (limit 0), as in euler_unitigs_from_kmers
+int euler_unitigs_clean_from_kmers_wide(euler_ctx *ctx, const uint64_t *keys_lo, const uint64_t *keys_hi, const uint32_t *counts,
+                                        uint64_t n, uint32_t K, const euler_clean_params *params, char *out, uint64_t *out_bytes,
+                                        uint64_t *ncontigs, uint64_t *kmer_sums, euler_clean_stats *stats)
+{
+    ENTER(ctx);
+    EULER_TRY(clean_args(ctx, K, params, out_bytes, ncontigs, stats));
+    if (n && (!keys_lo || !counts || (K > 32 && !keys_hi))) return euler_fail(ctx, EULER_ERR_ARG, "null argument");
+    const u64 cap_out = *out_bytes, cap_sums = *ncontigs;
+    *out_bytes = 0; *ncontigs = 0;
+    if (!n) return EULER_OK;
+    const u64 cap = euler_hash_capacity(n);
+    DevTmp<u64> dlo(ctx, n), flags(ctx, 1);
+    DevTmp<u32> dc(ctx, n), tc(ctx, cap);
+    TMP_CHECK(ctx, dlo); TMP_CHECK(ctx, dc); TMP_CHECK(ctx, tc); TMP_CHECK(ctx, flags);
+    EULER_TRY(upload(ctx, dlo, (const u64 *)keys_lo, n));
+    EULER_TRY(upload(ctx, dc, counts, n));
+    CUDA_TRY(ctx, cudaMemsetAsync(flags, 0, sizeof(u64), ctx->stream));
+    char *d_text = nullptr;
+    u64 bytes = 0, nc = 0, f = 0;
+    euler_clean_stats st{};
+    if (K > 32) {
+        DevTmp<u64> dhi(ctx, n);
+        DevTmp<K128> tk(ctx, cap);
+        TMP_CHECK(ctx, dhi); TMP_CHECK(ctx, tk);
+        EULER_TRY(upload(ctx, dhi, (const u64 *)keys_hi, n));
+        EULER_TRY(wide_table_clear(ctx, tk, tc, cap));
+        EULER_TRY(wide_unitig_dict_table(ctx, dlo, dhi, dc, n, K, tk, tc, cap, flags));
+        EULER_TRY(read_u64(ctx, flags, &f));
+        if (f) return euler_fail(ctx, EULER_ERR_OVERFLOW, "K-mer table full");
+        EULER_TRY(wide_unitig_clean_from_table(ctx, tk, tc, cap, K, 0, *params, &d_text, &bytes, &nc, (u64 *)kmer_sums, cap_sums,
+                                               &st));
+    } else {
+        DevTmp<u64> tk(ctx, cap);
+        TMP_CHECK(ctx, tk);
+        EULER_TRY(graph_table_clear(ctx, tk, tc, cap));
+        EULER_TRY(unitig_dict_table(ctx, dlo, dc, n, K, tk, tc, cap, flags));
+        EULER_TRY(read_u64(ctx, flags, &f));
+        if (f) return euler_fail(ctx, EULER_ERR_OVERFLOW, "K-mer table full");
+        EULER_TRY(unitig_clean_from_table(ctx, tk, tc, cap, K, 0, *params, &d_text, &bytes, &nc, (u64 *)kmer_sums, cap_sums, &st));
+    }
+    *out_bytes = bytes; *ncontigs = nc;
+    if (stats) *stats = st;
     if (out) {
         if (cap_out < bytes) return euler_fail(ctx, EULER_ERR_ARG, "output capacity too small");
         EULER_TRY(download(ctx, out, (const char *)d_text, bytes));

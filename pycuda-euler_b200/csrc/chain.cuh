@@ -141,56 +141,83 @@ static __global__ void __launch_bounds__(CH_TB) ch_widen_kernel(const u32 *__res
     if (t < n) out[t] = in[t];
 }
 
-// Emits into ctx->text_buf.  Total text must stay below 4 GiB (u32 scan); larger jobs are split
-// by the caller.
+// The ranking half of chain_emit, kept in one place for the callers that also need the ranks (clean.cu): predecessor
+// scatter, components, head kinds and anc.  After chain_rank, anc is ancA or ancB.
+struct ChainRanks {
+    DevTmp<u32> pred, D, has_start, head_kind, ord1, ord2, changed;
+    DevTmp<euler_succ_vertex> sv;
+    DevTmp<u64> ancA, ancB, totals;
+    u64 *anc = nullptr;
+    ChainRanks(euler_ctx *ctx, u32 n)
+        : pred(ctx, n), D(ctx, n), has_start(ctx, n), head_kind(ctx, n), ord1(ctx, n), ord2(ctx, n), changed(ctx, 1), sv(ctx, n),
+          ancA(ctx, n), ancB(ctx, n), totals(ctx, 4)
+    {
+    }
+    bool ok() const
+    {
+        return pred.ok() && D.ok() && has_start.ok() && head_kind.ok() && ord1.ok() && ord2.ok() && changed.ok() && sv.ok() &&
+               ancA.ok() && ancB.ok() && totals.ok();
+    }
+};
+#define CHAIN_RANKS_CHECK(ctx, r)                                                                   \
+    do {                                                                                           \
+        if (!(r).ok()) return euler_fail((ctx), EULER_ERR_NOMEM, "%s:%d device temp alloc failed", __FILE__, __LINE__); \
+    } while (0)
+
 template <typename M>
-static int chain_emit(euler_ctx *ctx, M m, u32 n, u32 k, char **d_out, u64 *out_bytes, u64 *ncontigs)
+static int chain_rank(euler_ctx *ctx, M m, u32 n, ChainRanks &r)
 {
-    *d_out = nullptr; *out_bytes = 0; *ncontigs = 0;
-    if (!n) return EULER_OK;
-    DevTmp<u32> pred(ctx, n), D(ctx, n), has_start(ctx, n), head_kind(ctx, n), ord1(ctx, n), ord2(ctx, n), changed(ctx, 1);
-    DevTmp<euler_succ_vertex> sv(ctx, n);
-    DevTmp<u64> ancA(ctx, n), ancB(ctx, n), totals(ctx, 4);
-    TMP_CHECK(ctx, pred); TMP_CHECK(ctx, D); TMP_CHECK(ctx, has_start); TMP_CHECK(ctx, head_kind); TMP_CHECK(ctx, ord1);
-    TMP_CHECK(ctx, ord2); TMP_CHECK(ctx, changed); TMP_CHECK(ctx, sv); TMP_CHECK(ctx, ancA); TMP_CHECK(ctx, ancB);
-    TMP_CHECK(ctx, totals);
     const unsigned g = grid_for(n, CH_TB);
     cudaStream_t s = ctx->stream;
-    ch_fill_kernel<<<g, CH_TB, 0, s>>>(pred, n, n);
-    ch_pred_kernel<<<g, CH_TB, 0, s>>>(m, n, pred);
-    ch_succ_vertex_kernel<<<g, CH_TB, 0, s>>>(m, pred, n, sv);
-    EULER_TRY(tour_components(ctx, sv, n, D));
-    CUDA_TRY(ctx, cudaMemsetAsync(has_start, 0, (size_t)n * 4, s));
-    ch_has_start_kernel<<<g, CH_TB, 0, s>>>(pred, D, n, has_start);
-    ch_rank_init_kernel<<<g, CH_TB, 0, s>>>(m, pred, D, has_start, n, ancA, head_kind);
+    ch_fill_kernel<<<g, CH_TB, 0, s>>>(r.pred, n, n);
+    ch_pred_kernel<<<g, CH_TB, 0, s>>>(m, n, r.pred);
+    ch_succ_vertex_kernel<<<g, CH_TB, 0, s>>>(m, r.pred, n, r.sv);
+    EULER_TRY(tour_components(ctx, r.sv, n, r.D));
+    CUDA_TRY(ctx, cudaMemsetAsync(r.has_start, 0, (size_t)n * 4, s));
+    ch_has_start_kernel<<<g, CH_TB, 0, s>>>(r.pred, r.D, n, r.has_start);
+    ch_rank_init_kernel<<<g, CH_TB, 0, s>>>(m, r.pred, r.D, r.has_start, n, r.ancA, r.head_kind);
     CUDA_TRY(ctx, cudaGetLastError());
-    u64 *cur = ancA, *nxt = ancB;
+    u64 *cur = r.ancA, *nxt = r.ancB;
     for (int round = 0; round < 40; round++) {
-        CUDA_TRY(ctx, cudaMemsetAsync(changed, 0, 4, s));
-        ch_rank_step_kernel<<<g, CH_TB, 0, s>>>(cur, nxt, n, changed);
-        CUDA_TRY(ctx, cudaMemcpyAsync(ctx->h_pinned, changed.get(), 4, cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(ctx, cudaMemsetAsync(r.changed, 0, 4, s));
+        ch_rank_step_kernel<<<g, CH_TB, 0, s>>>(cur, nxt, n, r.changed);
+        CUDA_TRY(ctx, cudaMemcpyAsync(ctx->h_pinned, r.changed.get(), 4, cudaMemcpyDeviceToHost, s));
         CUDA_TRY(ctx, cudaStreamSynchronize(s));
         u64 *t = cur; cur = nxt; nxt = t;
         if (!*(u32 *)ctx->h_pinned) break;
     }
-    EULER_TRY(scan_exclusive(ctx, ChKindIn{head_kind, 1u}, n, ord1.get(), totals.get() + 0));
-    EULER_TRY(scan_exclusive(ctx, ChKindIn{head_kind, 2u}, n, ord2.get(), totals.get() + 1));
+    r.anc = cur;
+    return EULER_OK;
+}
+
+// The emitting half on ranks of the same model: contig order (ord1 / ord2, *n_starts = number of path contigs),
+// lengths, text.  Emits into ctx->text_buf.
+template <typename M>
+static int chain_spell(euler_ctx *ctx, M m, u32 n, u32 k, ChainRanks &r, char **d_out, u64 *out_bytes, u64 *ncontigs,
+                       u32 *n_starts = nullptr)
+{
+    const unsigned g = grid_for(n, CH_TB);
+    cudaStream_t s = ctx->stream;
+    u64 *cur = r.anc;
+    EULER_TRY(scan_exclusive(ctx, ChKindIn{r.head_kind, 1u}, n, r.ord1.get(), r.totals.get() + 0));
+    EULER_TRY(scan_exclusive(ctx, ChKindIn{r.head_kind, 2u}, n, r.ord2.get(), r.totals.get() + 1));
     u64 h[2];
-    EULER_TRY(read_u64s(ctx, totals, h, 2));
+    EULER_TRY(read_u64s(ctx, r.totals, h, 2));
+    if (n_starts) *n_starts = (u32)h[0];
     const u64 nc = h[0] + h[1];
     if (!nc) return EULER_OK;
     DevTmp<u32> len_by_ord(ctx, nc), off32(ctx, nc);
     DevTmp<u64> off_by_ord(ctx, nc);
     TMP_CHECK(ctx, len_by_ord); TMP_CHECK(ctx, off32); TMP_CHECK(ctx, off_by_ord);
-    ch_len_kernel<<<g, CH_TB, 0, s>>>(m, head_kind, cur, ord1, ord2, (u32)h[0], n, k, len_by_ord);
-    EULER_TRY(scan_exclusive(ctx, ChLenIn{len_by_ord}, nc, off32.get(), totals.get() + 2));
+    ch_len_kernel<<<g, CH_TB, 0, s>>>(m, r.head_kind, cur, r.ord1, r.ord2, (u32)h[0], n, k, len_by_ord);
+    EULER_TRY(scan_exclusive(ctx, ChLenIn{len_by_ord}, nc, off32.get(), r.totals.get() + 2));
     u64 bytes = 0;
-    EULER_TRY(read_u64(ctx, totals.get() + 2, &bytes));
+    EULER_TRY(read_u64(ctx, r.totals.get() + 2, &bytes));
     if (bytes >= 0xffffffffull)
         return euler_fail(ctx, EULER_ERR_RANGE, "contig text of %llu bytes exceeds the 4 GiB emission limit", bytes);
     ch_widen_kernel<<<grid_for(nc, CH_TB), CH_TB, 0, s>>>(off32, nc, off_by_ord);
     EULER_TRY(dev_reserve(ctx, ctx->text_buf, bytes));
-    ch_write_kernel<<<g, CH_TB, 0, s>>>(m, head_kind, cur, ord1, ord2, (u32)h[0], n, k, off_by_ord, len_by_ord,
+    ch_write_kernel<<<g, CH_TB, 0, s>>>(m, r.head_kind, cur, r.ord1, r.ord2, (u32)h[0], n, k, off_by_ord, len_by_ord,
                                         (char *)ctx->text_buf.p);
     CUDA_TRY(ctx, cudaGetLastError());
     CUDA_TRY(ctx, cudaStreamSynchronize(s));
@@ -199,4 +226,17 @@ static int chain_emit(euler_ctx *ctx, M m, u32 n, u32 k, char **d_out, u64 *out_
     *out_bytes = bytes;
     *ncontigs = nc;
     return EULER_OK;
+}
+
+// Emits into ctx->text_buf.  Total text must stay below 4 GiB (u32 scan); larger jobs are split
+// by the caller.
+template <typename M>
+static int chain_emit(euler_ctx *ctx, M m, u32 n, u32 k, char **d_out, u64 *out_bytes, u64 *ncontigs)
+{
+    *d_out = nullptr; *out_bytes = 0; *ncontigs = 0;
+    if (!n) return EULER_OK;
+    ChainRanks r(ctx, n);
+    CHAIN_RANKS_CHECK(ctx, r);
+    EULER_TRY(chain_rank(ctx, m, n, r));
+    return chain_spell(ctx, m, n, k, r, d_out, out_bytes, ncontigs);
 }

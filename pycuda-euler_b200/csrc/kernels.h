@@ -109,10 +109,22 @@ int synth_reads(euler_ctx *ctx, u64 G, u32 L, u32 err_ppm, u64 first, u64 nreads
 int unitig_from_table(euler_ctx *ctx, const u64 *keys, const u32 *cnt, u64 cap, u32 K, u32 limit, char **d_out,
                       u64 *out_bytes, u64 *ncontigs, u64 *n_nodes);
 
+// unitig_from_table after the graph clean-up of clean.cu; h_sums (host, sums_cap entries, may be NULL): per-contig
+// sums of the both-strand counts, in output order
+int unitig_clean_from_table(euler_ctx *ctx, const u64 *keys, const u32 *cnt, u64 cap, u32 K, u32 limit,
+                            const euler_clean_params &p, char **d_out, u64 *out_bytes, u64 *ncontigs, u64 *h_sums,
+                            u64 sums_cap, euler_clean_stats *st);
+
 // canonical count table from a both-strand K-mer dictionary (keys, counts)
 int unitig_dict_table(euler_ctx *ctx, const u64 *d_keys, const u32 *d_counts, u64 n, u32 K, u64 *tk, u32 *tc, u64 cap, u64 *d_flags);
 // link graph of n contigs (text without separators, off[n+1]): links[16 i + 8 side + 2 base + (0 head '+' | 1 tail '-')]
 int unitig_link_graph(euler_ctx *ctx, const char *d_text, const u64 *d_off, u64 n, u32 K, u32 *d_links);
+
+// ---- clean.cu (key-independent): n nodes with forward extensions nbr[4 n], twin_id[n], both-strand counts cnt[n] and
+// keys of key_stride 64-bit words each (low word first)
+int clean_unitigs(euler_ctx *ctx, u32 n, u32 K, const u64 *key_words, u32 key_stride, const u32 *nbr, const u32 *twin_id,
+                  const u32 *cnt, const euler_clean_params &p, char **d_out, u64 *out_bytes, u64 *ncontigs, u64 *h_sums,
+                  u64 sums_cap, euler_clean_stats *st);
 
 // ---- graph.cu, fused fast path
 // pair scan over l-mer table slots: base = distinct both-strand l-mer index, eoff = edge offset;

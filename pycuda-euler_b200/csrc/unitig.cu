@@ -136,6 +136,44 @@ int unitig_from_table(euler_ctx *ctx, const u64 *keys, const u32 *cnt, u64 cap, 
     return chain_emit(ctx, m, (u32)n, K, d_out, out_bytes, ncontigs);
 }
 
+// clean.cu's view of the node graph: the node ids of the four forward extensions, the twin and the both-strand count
+__global__ void __launch_bounds__(UB) unitig_nbr_kernel(const u64 *__restrict__ keys, const u32 *__restrict__ cnt,
+                                                        const u32 *__restrict__ base, u64 cap, u32 K, u32 limit,
+                                                        const u64 *__restrict__ nkeys, u32 n, u32 *__restrict__ nbr,
+                                                        u32 *__restrict__ twin_id, u32 *__restrict__ ncnt)
+{
+    const u32 i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const u64 x = nkeys[i];
+    const u64 mask = key_mask_d(K);
+    twin_id[i] = node_of(keys, cnt, base, cap, K, limit, revcomp64(x, K));
+    for (u32 b = 0; b < 4; b++) nbr[4ull * i + b] = node_of(keys, cnt, base, cap, K, limit, ((x << 2) | b) & mask);
+    ncnt[i] = both_count(keys, cnt, table_find(keys, cap, canon_k(x, K)), K);
+}
+
+// unitig_from_table after the graph clean-up of clean.cu; h_sums (may be NULL): per-contig count sums
+int unitig_clean_from_table(euler_ctx *ctx, const u64 *keys, const u32 *cnt, u64 cap, u32 K, u32 limit,
+                            const euler_clean_params &p, char **d_out, u64 *out_bytes, u64 *ncontigs, u64 *h_sums,
+                            u64 sums_cap, euler_clean_stats *st)
+{
+    *d_out = nullptr; *out_bytes = 0; *ncontigs = 0; *st = euler_clean_stats{};
+    DevTmp<u32> base(ctx, cap);
+    DevTmp<u64> total(ctx, 1);
+    TMP_CHECK(ctx, base); TMP_CHECK(ctx, total);
+    EULER_TRY(scan_exclusive(ctx, NodeWeight{keys, cnt, K, limit}, cap, base.get(), total.get()));
+    u64 n = 0;
+    EULER_TRY(read_u64(ctx, total, &n));
+    if (!n) return EULER_OK;
+    if (n >= 0xffffffffull) return euler_fail(ctx, EULER_ERR_RANGE, "unitig node count exceeds u32");
+    DevTmp<u64> nkeys(ctx, n);
+    DevTmp<u32> nbr(ctx, 4 * n), twin_id(ctx, n), ncnt(ctx, n);
+    TMP_CHECK(ctx, nkeys); TMP_CHECK(ctx, nbr); TMP_CHECK(ctx, twin_id); TMP_CHECK(ctx, ncnt);
+    unitig_nodes_kernel<<<grid_for(cap, UB), UB, 0, ctx->stream>>>(keys, cnt, base, cap, K, limit, nkeys);
+    unitig_nbr_kernel<<<grid_for(n, UB), UB, 0, ctx->stream>>>(keys, cnt, base, cap, K, limit, nkeys, (u32)n, nbr, twin_id, ncnt);
+    CUDA_TRY(ctx, cudaGetLastError());
+    return clean_unitigs(ctx, (u32)n, K, nkeys, 1, nbr, twin_id, ncnt, p, d_out, out_bytes, ncontigs, h_sums, sums_cap, st);
+}
+
 // ---- a K-mer dictionary as input (referenceAssembler.all_contigs(d, k) takes the dict of build()) -------
 __global__ void __launch_bounds__(UB) kmer_dict_insert_kernel(const u64 *__restrict__ keys, const u32 *__restrict__ counts, u64 n,
                                                                u32 K, u64 *__restrict__ tk, u32 *__restrict__ tc, u64 cap, u64 *flags)

@@ -152,6 +152,10 @@ int wide_degree_slots(euler_ctx *ctx, const u64 *lk_lo, const u64 *lk_hi, const 
 // ---- wide_unitig.cu (unitig stage, K = 33..63; link graph, K = 32..63)
 int wide_unitig_from_table(euler_ctx *ctx, const K128 *keys, const u32 *cnt, u64 cap, u32 K, u32 limit, char **d_out,
                            u64 *out_bytes, u64 *ncontigs, u64 *n_nodes);
+// the same after the graph clean-up of clean.cu (unitig_clean_from_table)
+int wide_unitig_clean_from_table(euler_ctx *ctx, const K128 *keys, const u32 *cnt, u64 cap, u32 K, u32 limit,
+                                 const euler_clean_params &p, char **d_out, u64 *out_bytes, u64 *ncontigs, u64 *h_sums,
+                                 u64 sums_cap, euler_clean_stats *st);
 // canonical count table from a both-strand K-mer dictionary (keys as lo / hi words, counts)
 int wide_unitig_dict_table(euler_ctx *ctx, const u64 *d_lo, const u64 *d_hi, const u32 *d_counts, u64 n, u32 K, K128 *tk, u32 *tc,
                            u64 cap, u64 *d_flags);

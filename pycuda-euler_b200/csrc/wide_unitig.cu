@@ -130,6 +130,50 @@ int wide_unitig_from_table(euler_ctx *ctx, const K128 *keys, const u32 *cnt, u64
     return chain_emit(ctx, m, (u32)n, K, d_out, out_bytes, ncontigs);
 }
 
+// clean.cu's view of the node graph, as unitig_nbr_kernel
+__global__ void __launch_bounds__(WUB) wide_unitig_nbr_kernel(const K128 *__restrict__ keys, const u32 *__restrict__ cnt,
+                                                               const u32 *__restrict__ base, u64 cap, u32 K, u32 limit,
+                                                               const K128 *__restrict__ nkeys, u32 n, u32 *__restrict__ nbr,
+                                                               u32 *__restrict__ twin_id, u32 *__restrict__ ncnt)
+{
+    const u32 i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const K128 x = nkeys[i];
+    const K128 mask = mask128(K);
+    const K128 tw = revcomp128(x, K);
+    twin_id[i] = wide_node_of(keys, cnt, base, cap, K, limit, tw);
+    for (u32 b = 0; b < 4; b++) nbr[4ull * i + b] = wide_node_of(keys, cnt, base, cap, K, limit, and128(shl2_or(x, b), mask));
+    const u64 slot = wide_find(keys, cap, lt128(tw, x) ? tw : x);
+    ncnt[i] = eq128(x, tw) ? 2u * cnt[slot] : cnt[slot];
+}
+
+// wide_unitig_from_table after the graph clean-up of clean.cu
+int wide_unitig_clean_from_table(euler_ctx *ctx, const K128 *keys, const u32 *cnt, u64 cap, u32 K, u32 limit,
+                                 const euler_clean_params &p, char **d_out, u64 *out_bytes, u64 *ncontigs, u64 *h_sums,
+                                 u64 sums_cap, euler_clean_stats *st)
+{
+    *d_out = nullptr; *out_bytes = 0; *ncontigs = 0; *st = euler_clean_stats{};
+    DevTmp<u32> weight(ctx, cap), base(ctx, cap);
+    DevTmp<u64> total(ctx, 1);
+    TMP_CHECK(ctx, weight); TMP_CHECK(ctx, base); TMP_CHECK(ctx, total);
+    wide_node_weight_kernel<<<grid_for(cap, WUB), WUB, 0, ctx->stream>>>(keys, cnt, cap, K, limit, weight);
+    CUDA_TRY(ctx, cudaGetLastError());
+    EULER_TRY(scan_exclusive(ctx, ScanInU32{weight}, cap, base.get(), total.get()));
+    u64 n = 0;
+    EULER_TRY(read_u64(ctx, total, &n));
+    if (!n) return EULER_OK;
+    if (n >= 0xffffffffull) return euler_fail(ctx, EULER_ERR_RANGE, "unitig node count exceeds u32");
+    DevTmp<K128> nkeys(ctx, n);
+    DevTmp<u32> nbr(ctx, 4 * n), twin_id(ctx, n), ncnt(ctx, n);
+    TMP_CHECK(ctx, nkeys); TMP_CHECK(ctx, nbr); TMP_CHECK(ctx, twin_id); TMP_CHECK(ctx, ncnt);
+    wide_unitig_nodes_kernel<<<grid_for(cap, WUB), WUB, 0, ctx->stream>>>(keys, cnt, base, cap, K, limit, nkeys);
+    wide_unitig_nbr_kernel<<<grid_for(n, WUB), WUB, 0, ctx->stream>>>(keys, cnt, base, cap, K, limit, nkeys, (u32)n, nbr, twin_id,
+                                                                      ncnt);
+    CUDA_TRY(ctx, cudaGetLastError());
+    return clean_unitigs(ctx, (u32)n, K, (const u64 *)nkeys.get(), 2, nbr, twin_id, ncnt, p, d_out, out_bytes, ncontigs, h_sums,
+                         sums_cap, st);
+}
+
 // ---- a K-mer dictionary as input (referenceAssembler.all_contigs(d, k) takes the dict of build()) -------
 __global__ void __launch_bounds__(WUB) wide_kmer_dict_insert_kernel(const u64 *__restrict__ keys_lo, const u64 *__restrict__ keys_hi,
                                                                      const u32 *__restrict__ counts, u64 n, u32 K,

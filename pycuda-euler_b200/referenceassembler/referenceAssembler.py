@@ -196,12 +196,16 @@ def get_contig(d, km):
     return contig_to_string(c), c
 
 
-def write_gfa(G, cs, k, out=None):
-    """GFA 1.0 records of the link graph (the intent of print_GFA :115-125)"""
+def write_gfa(G, cs, k, out=None, kc=None):
+    """GFA 1.0 records of the link graph (the intent of print_GFA :115-125).  kc: per-contig K-mer count sums; when
+    given, every S line ends in the KC:i: tag (total K-mer coverage, which graph viewers such as Bandage read)."""
     out = out or sys.stdout
     out.write("H\tVN:Z:1.0\n")
     for i, x in enumerate(cs):
-        out.write("S\t%d\t%s\t*\n" % (i, x))
+        if kc is None:
+            out.write("S\t%d\t%s\t*\n" % (i, x))
+        else:
+            out.write("S\t%d\t%s\t*\tKC:i:%d\n" % (i, x, int(kc[i])))
     for i in G:
         for j, o in G[i][0]:
             out.write("L\t%d\t+\t%d\t%s\t%dM\n" % (i, j, o, k - 1))

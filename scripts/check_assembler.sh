@@ -32,6 +32,18 @@ print('single-GPU contigs', len(a), 'multi-GPU contigs', len(b), 'equal sets:', 
 assert a == b and len(a) > 0
 print('gfa links:', sum(1 for l in open('/tmp/multi.fa.gfa') if l[0] == 'L'), 'vs', sum(1 for l in open('/tmp/one.fa.gfa') if l[0] == 'L'))
 PY
+# --clean: the contig set of one assembly across GPUs (clean-up on the joined table) equals the single-GPU one
+python pycuda-euler_b200/assembler.py -i /tmp/reads.fq -o /tmp/one_c.fa -k 31 --clean
+python -m torch.distributed.run --nnodes=1 --nproc-per-node $N --master-addr 127.0.0.1 --master-port 29533 \
+    pycuda-euler_b200/assembler.py -i /tmp/reads.fq -o /tmp/multi_c.fa -k 31 --clean
+python - <<'PY'
+def canon(path):
+    comp = str.maketrans('ACGT', 'TGCA')
+    return sorted(min(c, c.translate(comp)[::-1]) for c in (l.strip() for l in open(path)) if c and c[0] != '>')
+a, b = canon('/tmp/one_c.fa'), canon('/tmp/multi_c.fa')
+print('--clean: single-GPU contigs', len(a), 'multi-GPU contigs', len(b), 'equal sets:', a == b)
+assert a == b and len(a) > 0
+PY
 # Euler mode: identical contig LIST (canonical ids make the tour deterministic)
 python pycuda-euler_b200/assembler.py -i /tmp/reads.fq -o /tmp/one_e.fa -k 32 --mode euler
 python -m torch.distributed.run --nnodes=1 --nproc-per-node $N --master-addr 127.0.0.1 --master-port 29532 \
