@@ -206,7 +206,10 @@ int euler_unitigs_clean(euler_ctx *ctx, const char *buf, const uint64_t *read_of
 /* the same on the reads left on the device by euler_ingest */
 int euler_unitigs_clean_ingested(euler_ctx *ctx, uint32_t K, uint32_t limit, const euler_clean_params *params, char *out,
                                  uint64_t *out_bytes, uint64_t *ncontigs, uint64_t *kmer_sums, euler_clean_stats *stats);
-/* the same on a K-mer dictionary, as euler_unitigs_from_kmers_wide (K <= 32 reads keys_lo only) */
+/* the same on a K-mer dictionary, as euler_unitigs_from_kmers_wide (K <= 32 reads keys_lo only).  The clean-up
+ * compares coverages, so here the counts must be both-strand counts as euler_count_mers(_wide) returns them: even on a
+ * palindrome, and equal on a key and its reverse complement when both are given.  Other counts are refused with
+ * EULER_ERR_ARG (euler_unitigs_from_kmers(_wide), whose output depends only on which keys are present, takes any). */
 int euler_unitigs_clean_from_kmers_wide(euler_ctx *ctx, const uint64_t *keys_lo, const uint64_t *keys_hi,
                                         const uint32_t *counts, uint64_t n, uint32_t K, const euler_clean_params *params,
                                         char *out, uint64_t *out_bytes, uint64_t *ncontigs, uint64_t *kmer_sums,

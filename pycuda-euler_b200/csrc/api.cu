@@ -390,7 +390,17 @@ int euler_unitigs_clean_ingested(euler_ctx *ctx, uint32_t K, uint32_t limit, con
     return EULER_OK;
 }
 
-// the dictionary's counts are all kept (limit 0), as in euler_unitigs_from_kmers
+// flags of the dictionary insert and check: 1 the table is full, 2 a count is not a both-strand count
+static int dict_flags(euler_ctx *ctx, u64 f)
+{
+    if (f & 1) return euler_fail(ctx, EULER_ERR_OVERFLOW, "K-mer table full");
+    if (f & 2) return euler_fail(ctx, EULER_ERR_ARG, "K-mer counts are not both-strand counts (an odd count on a palindrome, "
+                                                     "or a key and its reverse complement with different counts)");
+    return EULER_OK;
+}
+
+// the dictionary's counts are all kept (limit 0), as in euler_unitigs_from_kmers; they must be both-strand counts,
+// because the clean-up compares them
 int euler_unitigs_clean_from_kmers_wide(euler_ctx *ctx, const uint64_t *keys_lo, const uint64_t *keys_hi, const uint32_t *counts,
                                         uint64_t n, uint32_t K, const euler_clean_params *params, char *out, uint64_t *out_bytes,
                                         uint64_t *ncontigs, uint64_t *kmer_sums, euler_clean_stats *stats)
@@ -418,8 +428,9 @@ int euler_unitigs_clean_from_kmers_wide(euler_ctx *ctx, const uint64_t *keys_lo,
         EULER_TRY(upload(ctx, dhi, (const u64 *)keys_hi, n));
         EULER_TRY(wide_table_clear(ctx, tk, tc, cap));
         EULER_TRY(wide_unitig_dict_table(ctx, dlo, dhi, dc, n, K, tk, tc, cap, flags));
+        EULER_TRY(wide_unitig_dict_check(ctx, dlo, dhi, dc, n, K, tk, tc, cap, flags));
         EULER_TRY(read_u64(ctx, flags, &f));
-        if (f) return euler_fail(ctx, EULER_ERR_OVERFLOW, "K-mer table full");
+        EULER_TRY(dict_flags(ctx, f));
         EULER_TRY(wide_unitig_clean_from_table(ctx, tk, tc, cap, K, 0, *params, &d_text, &bytes, &nc, (u64 *)kmer_sums, cap_sums,
                                                &st));
     } else {
@@ -427,8 +438,9 @@ int euler_unitigs_clean_from_kmers_wide(euler_ctx *ctx, const uint64_t *keys_lo,
         TMP_CHECK(ctx, tk);
         EULER_TRY(graph_table_clear(ctx, tk, tc, cap));
         EULER_TRY(unitig_dict_table(ctx, dlo, dc, n, K, tk, tc, cap, flags));
+        EULER_TRY(unitig_dict_check(ctx, dlo, dc, n, K, tk, tc, cap, flags));
         EULER_TRY(read_u64(ctx, flags, &f));
-        if (f) return euler_fail(ctx, EULER_ERR_OVERFLOW, "K-mer table full");
+        EULER_TRY(dict_flags(ctx, f));
         EULER_TRY(unitig_clean_from_table(ctx, tk, tc, cap, K, 0, *params, &d_text, &bytes, &nc, (u64 *)kmer_sums, cap_sums, &st));
     }
     *out_bytes = bytes; *ncontigs = nc;

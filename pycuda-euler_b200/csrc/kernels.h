@@ -117,6 +117,9 @@ int unitig_clean_from_table(euler_ctx *ctx, const u64 *keys, const u32 *cnt, u64
 
 // canonical count table from a both-strand K-mer dictionary (keys, counts)
 int unitig_dict_table(euler_ctx *ctx, const u64 *d_keys, const u32 *d_counts, u64 n, u32 K, u64 *tk, u32 *tc, u64 cap, u64 *d_flags);
+// after unitig_dict_table: sets bit 2 of *d_flags when a count is not the both-strand count of its key in the table
+int unitig_dict_check(euler_ctx *ctx, const u64 *d_keys, const u32 *d_counts, u64 n, u32 K, const u64 *tk, const u32 *tc, u64 cap,
+                      u64 *d_flags);
 // link graph of n contigs (text without separators, off[n+1]): links[16 i + 8 side + 2 base + (0 head '+' | 1 tail '-')]
 int unitig_link_graph(euler_ctx *ctx, const char *d_text, const u64 *d_off, u64 n, u32 K, u32 *d_links);
 

@@ -196,6 +196,29 @@ int unitig_dict_table(euler_ctx *ctx, const u64 *d_keys, const u32 *d_counts, u6
     return EULER_OK;
 }
 
+// after kmer_dict_insert_kernel: flag 2 when a key's count is not the both-strand count the table now gives it (an
+// odd count on a palindrome, or a key and its twin given with different counts)
+__global__ void __launch_bounds__(UB) kmer_dict_check_kernel(const u64 *__restrict__ keys, const u32 *__restrict__ counts, u64 n,
+                                                              u32 K, const u64 *__restrict__ tk, const u32 *__restrict__ tc,
+                                                              u64 cap, u64 *flags)
+{
+    const u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const u64 x = keys[i] & key_mask_d(K), r = revcomp64(x, K);
+    const u64 slot = table_find(tk, cap, x < r ? x : r);
+    if (slot == EULER_NO_SLOT) return;   // the insert has flagged a full table
+    const u32 v = counts[i];
+    if ((x == r && (v & 1u)) || both_count(tk, tc, slot, K) != v) atomicOr((unsigned long long *)flags, 2ull);
+}
+int unitig_dict_check(euler_ctx *ctx, const u64 *d_keys, const u32 *d_counts, u64 n, u32 K, const u64 *tk, const u32 *tc, u64 cap,
+                      u64 *d_flags)
+{
+    if (!n) return EULER_OK;
+    kmer_dict_check_kernel<<<grid_for(n, UB), UB, 0, ctx->stream>>>(d_keys, d_counts, n, K, tk, tc, cap, d_flags);
+    CUDA_TRY(ctx, cudaGetLastError());
+    return EULER_OK;
+}
+
 // ---- link graph of the contigs: referenceAssembler.all_contigs :90-111 ------------------------------------
 // heads[x[:k]] = (i,'+'), tails[twin(x[-k:])] = (i,'-') (a later contig overwrites an earlier one: max i);
 // G[i][0] = for y in fw(x[-k:]): heads hit, tails hit; G[i][1] = for z in fw(twin(x[:k])): heads hit, tails hit.

@@ -159,6 +159,9 @@ int wide_unitig_clean_from_table(euler_ctx *ctx, const K128 *keys, const u32 *cn
 // canonical count table from a both-strand K-mer dictionary (keys as lo / hi words, counts)
 int wide_unitig_dict_table(euler_ctx *ctx, const u64 *d_lo, const u64 *d_hi, const u32 *d_counts, u64 n, u32 K, K128 *tk, u32 *tc,
                            u64 cap, u64 *d_flags);
+// after wide_unitig_dict_table: sets bit 2 of *d_flags as unitig_dict_check
+int wide_unitig_dict_check(euler_ctx *ctx, const u64 *d_lo, const u64 *d_hi, const u32 *d_counts, u64 n, u32 K, const K128 *tk,
+                           const u32 *tc, u64 cap, u64 *d_flags);
 // links[16 i + 8 side + 2 base + (0 head '+' | 1 tail '-')] of n contigs (text without separators, off[n+1])
 int wide_unitig_link_graph(euler_ctx *ctx, const char *d_text, const u64 *d_off, u64 n, u32 K, u32 *d_links);
 // (key, count) filter: keep count > limit, compact

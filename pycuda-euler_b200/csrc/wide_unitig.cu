@@ -197,6 +197,30 @@ int wide_unitig_dict_table(euler_ctx *ctx, const u64 *d_lo, const u64 *d_hi, con
     return EULER_OK;
 }
 
+// after wide_kmer_dict_insert_kernel: flag 2 as kmer_dict_check_kernel
+__global__ void __launch_bounds__(WUB) wide_kmer_dict_check_kernel(const u64 *__restrict__ keys_lo, const u64 *__restrict__ keys_hi,
+                                                                    const u32 *__restrict__ counts, u64 n, u32 K,
+                                                                    const K128 *__restrict__ tk, const u32 *__restrict__ tc, u64 cap,
+                                                                    u64 *flags)
+{
+    const u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const K128 x = and128(K128{keys_lo[i], keys_hi[i]}, mask128(K)), r = revcomp128(x, K);
+    const u64 slot = wide_find(tk, cap, lt128(r, x) ? r : x);
+    if (slot == EULER_NO_SLOT) return;   // the insert has flagged a full table
+    const u32 v = counts[i];
+    const bool pal = eq128(x, r);
+    if ((pal && (v & 1u)) || (pal ? 2u * tc[slot] : tc[slot]) != v) atomicOr((unsigned long long *)flags, 2ull);
+}
+int wide_unitig_dict_check(euler_ctx *ctx, const u64 *d_lo, const u64 *d_hi, const u32 *d_counts, u64 n, u32 K, const K128 *tk,
+                           const u32 *tc, u64 cap, u64 *d_flags)
+{
+    if (!n) return EULER_OK;
+    wide_kmer_dict_check_kernel<<<grid_for(n, WUB), WUB, 0, ctx->stream>>>(d_lo, d_hi, d_counts, n, K, tk, tc, cap, d_flags);
+    CUDA_TRY(ctx, cudaGetLastError());
+    return EULER_OK;
+}
+
 // ---- link graph of the contigs (referenceAssembler.all_contigs :90-111), as unitig_link_graph --------------
 __device__ __forceinline__ K128 encode_text_kmer128(const char *s, u32 K)
 {
