@@ -253,8 +253,10 @@ static int pipeline_run_wide(euler_ctx *ctx, Pipeline *P, u32 l, u32 flags, u64 
         EULER_TRY(read_u64s(ctx, P->stats.ptr(), h, 6));
         if ((h[2] & 3) == 0) break;
         if (++retries > 10) return euler_fail(ctx, EULER_ERR_OVERFLOW, "hash table overflow after %u regrows", retries);
-        if (h[2] & 1) lt_cap *= 2;
-        if (h[2] & 2) vt_cap *= 2;
+        // The window counts are complete even when a table overflowed, and they bound the distinct counts: one regrow
+        // is enough however small the hint or the learned size was (doubling alone gave up after 10 on large inputs).
+        if (h[2] & 1) lt_cap = std::max(2 * lt_cap, cap_for(h[0]));
+        if (h[2] & 2) vt_cap = std::max(2 * vt_cap, cap_for(h[1]));
     }
     const u64 N_l = h[0], N_k = h[1], U_l = h[3], V = h[4];
     const u64 E = 2 * N_l;
