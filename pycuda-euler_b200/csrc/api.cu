@@ -193,7 +193,9 @@ int euler_count_mers_wide(euler_ctx *ctx, const char *buf, const uint64_t *read_
     TMP_CHECK(ctx, fbase);
     EULER_TRY(wide_compact_lmers(ctx, tk, tc, base, cap, len, lo, hi, lv));
     EULER_TRY(wide_sort(ctx, lo, hi, lv, U, 2 * (int)len));
-    EULER_TRY(wide_filter_counts(ctx, lo, hi, lv, U, limit, fbase, lo2, hi2, lv2, d_stats.get() + 4));
+    // graph.cu's one-word filter (keep count > limit), once per key word: both passes keep the same entries
+    EULER_TRY(graph_filter_counts(ctx, lo, lv, U, limit, fbase, lo2, lv2, d_stats.get() + 4));
+    EULER_TRY(graph_filter_counts(ctx, hi, lv, U, limit, fbase, hi2, lv2, d_stats.get() + 4));
     u64 kept = 0;
     EULER_TRY(read_u64(ctx, d_stats.get() + 4, &kept));
     *count = kept;
@@ -207,52 +209,25 @@ int euler_count_mers_wide(euler_ctx *ctx, const char *buf, const uint64_t *read_
 }
 
 // cp != NULL: the unitigs after the graph clean-up (clean.cu), with per-contig count sums (sums: *ncontigs entries on
-// entry, may be NULL) and stats
+// entry, may be NULL) and stats (may be NULL; written on success)
 static int unitigs_core(euler_ctx *ctx, const void *d_buf, const u64 *d_off, u64 nreads, u64 B, uint32_t K, uint32_t limit,
                         char *out, uint64_t *out_bytes, uint64_t *ncontigs, const euler_clean_params *cp = nullptr,
-                        uint64_t *sums = nullptr, euler_clean_stats *st = nullptr)
+                        uint64_t *sums = nullptr, euler_clean_stats *stats = nullptr)
 {
     const u64 cap_out = *out_bytes, cap_sums = *ncontigs;
     *out_bytes = 0; *ncontigs = 0;
     if (!B) return EULER_OK;
-    DevTmp<u64> d_stats(ctx, 8);
-    DevTmp<u32> d_bits(ctx, B / 32 + 2);
-    TMP_CHECK(ctx, d_bits); TMP_CHECK(ctx, d_stats);
-    EULER_TRY(enc_mark_starts(ctx, d_off, nreads, B, d_bits));
-    const u64 cap = euler_hash_capacity(B);
-    CUDA_TRY(ctx, cudaMemsetAsync(d_stats, 0, 8 * sizeof(u64), ctx->stream));
     char *d_text = nullptr;
-    u64 bytes = 0, nc = 0, nn = 0;
-    if (K > 32) {
-        // two-word keys: the tiled 128-bit count of the pipeline (wide.cu) into a K128 table of the same capacity
-        DevTmp<K128> tk(ctx, cap);
-        DevTmp<u32> tc(ctx, cap);
-        TMP_CHECK(ctx, tk); TMP_CHECK(ctx, tc);
-        EULER_TRY(wide_table_clear(ctx, tk, tc, cap));
-        EULER_TRY(wide_count_tiled(ctx, d_buf, B, d_bits, K, tk, tc, cap, d_stats));
-        u64 h[3];
-        EULER_TRY(read_u64s(ctx, d_stats, h, 3));
-        if (h[2]) return euler_fail(ctx, EULER_ERR_OVERFLOW, "count table overflow");
-        if (cp) EULER_TRY(wide_unitig_clean_from_table(ctx, tk, tc, cap, K, limit, *cp, &d_text, &bytes, &nc, (u64 *)sums, cap_sums, st));
-        else EULER_TRY(wide_unitig_from_table(ctx, tk, tc, cap, K, limit, &d_text, &bytes, &nc, &nn));
-    } else {
-        DevTmp<u64> tk(ctx, cap);
-        DevTmp<u32> tc(ctx, cap);
-        TMP_CHECK(ctx, tk); TMP_CHECK(ctx, tc);
-        EULER_TRY(graph_table_clear(ctx, tk, tc, cap));
-        EULER_TRY(enc_count_canonical(ctx, d_buf, B, d_bits, K, tk, tc, cap, TableHash{0, 0}, d_stats));
-        u64 h[3];
-        EULER_TRY(read_u64s(ctx, d_stats, h, 3));
-        if (h[2]) return euler_fail(ctx, EULER_ERR_OVERFLOW, "count table overflow");
-        if (cp) EULER_TRY(unitig_clean_from_table(ctx, tk, tc, cap, K, limit, *cp, &d_text, &bytes, &nc, (u64 *)sums, cap_sums, st));
-        else EULER_TRY(unitig_from_table(ctx, tk, tc, cap, K, limit, &d_text, &bytes, &nc, &nn));
-    }
+    u64 bytes = 0, nc = 0;
+    euler_clean_stats st{};
+    EULER_TRY(unitigs_from_reads(ctx, d_buf, d_off, nreads, B, K, limit, cp, &d_text, &bytes, &nc, (u64 *)sums, cap_sums, &st));
     *out_bytes = bytes; *ncontigs = nc;
     if (out) {
         if (cap_out < bytes) return euler_fail(ctx, EULER_ERR_ARG, "output capacity too small");
         EULER_TRY(download(ctx, out, (const char *)d_text, bytes));
     }
     CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+    if (stats) *stats = st;
     return EULER_OK;
 }
 
@@ -281,37 +256,42 @@ int euler_unitigs_ingested(euler_ctx *ctx, uint32_t K, uint32_t limit, char *out
     return unitigs_core(ctx, d_buf, d_off, nr, nb, K, limit, out, out_bytes, ncontigs);
 }
 
-// referenceAssembler.all_contigs(d, k) :79-88 on a K-mer dictionary (the output of build / euler_count_mers)
+// referenceAssembler.all_contigs(d, k) :79-88 on a K-mer dictionary (the output of build / euler_count_mers), every
+// count kept (limit 0); keys_hi is read for K > 32 only.  cp != NULL: after the graph clean-up, with sums and stats
+// (may be NULL) as unitigs_core.
+static int unitigs_dict_core(euler_ctx *ctx, const uint64_t *keys_lo, const uint64_t *keys_hi, const uint32_t *counts, uint64_t n,
+                             uint32_t K, char *out, uint64_t *out_bytes, uint64_t *ncontigs, const euler_clean_params *cp = nullptr,
+                             uint64_t *sums = nullptr, euler_clean_stats *stats = nullptr)
+{
+    const u64 cap_out = *out_bytes, cap_sums = *ncontigs;
+    *out_bytes = 0; *ncontigs = 0;
+    if (!n) return EULER_OK;
+    DevTmp<u64> dlo(ctx, n), dhi(ctx, K > 32 ? n : 0);
+    DevTmp<u32> dc(ctx, n);
+    TMP_CHECK(ctx, dlo); TMP_CHECK(ctx, dhi); TMP_CHECK(ctx, dc);
+    EULER_TRY(upload(ctx, dlo, (const u64 *)keys_lo, n));
+    if (K > 32) EULER_TRY(upload(ctx, dhi, (const u64 *)keys_hi, n));
+    EULER_TRY(upload(ctx, dc, counts, n));
+    char *d_text = nullptr;
+    u64 bytes = 0, nc = 0;
+    euler_clean_stats st{};
+    EULER_TRY(unitigs_from_dict(ctx, dlo, dhi, dc, n, K, cp, &d_text, &bytes, &nc, (u64 *)sums, cap_sums, &st));
+    *out_bytes = bytes; *ncontigs = nc;
+    if (stats) *stats = st;
+    if (out) {
+        if (cap_out < bytes) return euler_fail(ctx, EULER_ERR_ARG, "output capacity too small");
+        EULER_TRY(download(ctx, out, (const char *)d_text, bytes));
+    }
+    FINISH(ctx);
+}
+
 int euler_unitigs_from_kmers(euler_ctx *ctx, const uint64_t *keys, const uint32_t *counts, uint64_t n, uint32_t K, char *out,
                              uint64_t *out_bytes, uint64_t *ncontigs)
 {
     ENTER(ctx);
     if (!out_bytes || !ncontigs || (n && (!keys || !counts))) return euler_fail(ctx, EULER_ERR_ARG, "null argument");
     if (K < 2 || K > 32) return euler_fail(ctx, EULER_ERR_ARG, "K %u out of range [2,32]", K);
-    const u64 cap_out = *out_bytes;
-    *out_bytes = 0; *ncontigs = 0;
-    if (!n) return EULER_OK;
-    const u64 cap = euler_hash_capacity(n);
-    DevTmp<u64> dk(ctx, n), tk(ctx, cap), flags(ctx, 1);
-    DevTmp<u32> dc(ctx, n), tc(ctx, cap);
-    TMP_CHECK(ctx, dk); TMP_CHECK(ctx, dc); TMP_CHECK(ctx, tk); TMP_CHECK(ctx, tc); TMP_CHECK(ctx, flags);
-    EULER_TRY(upload(ctx, dk, (const u64 *)keys, n));
-    EULER_TRY(upload(ctx, dc, counts, n));
-    CUDA_TRY(ctx, cudaMemsetAsync(flags, 0, sizeof(u64), ctx->stream));
-    EULER_TRY(graph_table_clear(ctx, tk, tc, cap));
-    EULER_TRY(unitig_dict_table(ctx, dk, dc, n, K, tk, tc, cap, flags));
-    u64 f = 0;
-    EULER_TRY(read_u64(ctx, flags, &f));
-    if (f) return euler_fail(ctx, EULER_ERR_OVERFLOW, "K-mer table full");
-    char *d_text = nullptr;
-    u64 bytes = 0, nc = 0, nn = 0;
-    EULER_TRY(unitig_from_table(ctx, tk, tc, cap, K, 0, &d_text, &bytes, &nc, &nn));
-    *out_bytes = bytes; *ncontigs = nc;
-    if (out) {
-        if (cap_out < bytes) return euler_fail(ctx, EULER_ERR_ARG, "output capacity too small");
-        EULER_TRY(download(ctx, out, (const char *)d_text, bytes));
-    }
-    FINISH(ctx);
+    return unitigs_dict_core(ctx, keys, nullptr, counts, n, K, out, out_bytes, ncontigs);
 }
 
 // euler_unitigs_from_kmers on two-word keys: K in [2,63]; K <= 32 reads keys_lo only (keys_hi may be NULL)
@@ -320,34 +300,9 @@ int euler_unitigs_from_kmers_wide(euler_ctx *ctx, const uint64_t *keys_lo, const
 {
     ENTER(ctx);
     if (K < 2 || K > 63) return euler_fail(ctx, EULER_ERR_ARG, "K %u out of range [2,63]", K);
-    if (K <= 32) return euler_unitigs_from_kmers(ctx, keys_lo, counts, n, K, out, out_bytes, ncontigs);
-    if (!out_bytes || !ncontigs || (n && (!keys_lo || !keys_hi || !counts))) return euler_fail(ctx, EULER_ERR_ARG, "null argument");
-    const u64 cap_out = *out_bytes;
-    *out_bytes = 0; *ncontigs = 0;
-    if (!n) return EULER_OK;
-    const u64 cap = euler_hash_capacity(n);
-    DevTmp<u64> dlo(ctx, n), dhi(ctx, n), flags(ctx, 1);
-    DevTmp<u32> dc(ctx, n), tc(ctx, cap);
-    DevTmp<K128> tk(ctx, cap);
-    TMP_CHECK(ctx, dlo); TMP_CHECK(ctx, dhi); TMP_CHECK(ctx, dc); TMP_CHECK(ctx, tk); TMP_CHECK(ctx, tc); TMP_CHECK(ctx, flags);
-    EULER_TRY(upload(ctx, dlo, (const u64 *)keys_lo, n));
-    EULER_TRY(upload(ctx, dhi, (const u64 *)keys_hi, n));
-    EULER_TRY(upload(ctx, dc, counts, n));
-    CUDA_TRY(ctx, cudaMemsetAsync(flags, 0, sizeof(u64), ctx->stream));
-    EULER_TRY(wide_table_clear(ctx, tk, tc, cap));
-    EULER_TRY(wide_unitig_dict_table(ctx, dlo, dhi, dc, n, K, tk, tc, cap, flags));
-    u64 f = 0;
-    EULER_TRY(read_u64(ctx, flags, &f));
-    if (f) return euler_fail(ctx, EULER_ERR_OVERFLOW, "K-mer table full");
-    char *d_text = nullptr;
-    u64 bytes = 0, nc = 0, nn = 0;
-    EULER_TRY(wide_unitig_from_table(ctx, tk, tc, cap, K, 0, &d_text, &bytes, &nc, &nn));
-    *out_bytes = bytes; *ncontigs = nc;
-    if (out) {
-        if (cap_out < bytes) return euler_fail(ctx, EULER_ERR_ARG, "output capacity too small");
-        EULER_TRY(download(ctx, out, (const char *)d_text, bytes));
-    }
-    FINISH(ctx);
+    if (!out_bytes || !ncontigs || (n && (!keys_lo || !counts || (K > 32 && !keys_hi))))
+        return euler_fail(ctx, EULER_ERR_ARG, "null argument");
+    return unitigs_dict_core(ctx, keys_lo, keys_hi, counts, n, K, out, out_bytes, ncontigs);
 }
 
 static int clean_args(euler_ctx *ctx, uint32_t K, const euler_clean_params *params, uint64_t *out_bytes, uint64_t *ncontigs,
@@ -366,15 +321,12 @@ int euler_unitigs_clean(euler_ctx *ctx, const char *buf, const uint64_t *read_of
     ENTER(ctx);
     if (!read_off) return euler_fail(ctx, EULER_ERR_ARG, "null argument");
     EULER_TRY(clean_args(ctx, K, params, out_bytes, ncontigs, stats));
-    euler_clean_stats st{};
     const u64 B = read_off[nreads];
     DevTmp<unsigned char> d_buf(ctx, B + 16);
     DevTmp<u64> d_off(ctx, nreads + 1);
     EULER_TRY(upload(ctx, d_buf, (const unsigned char *)buf, B));
     EULER_TRY(upload(ctx, d_off, (const u64 *)read_off, nreads + 1));
-    EULER_TRY(unitigs_core(ctx, d_buf, d_off, nreads, B, K, limit, out, out_bytes, ncontigs, params, kmer_sums, &st));
-    if (stats) *stats = st;
-    return EULER_OK;
+    return unitigs_core(ctx, d_buf, d_off, nreads, B, K, limit, out, out_bytes, ncontigs, params, kmer_sums, stats);
 }
 
 int euler_unitigs_clean_ingested(euler_ctx *ctx, uint32_t K, uint32_t limit, const euler_clean_params *params, char *out,
@@ -382,21 +334,9 @@ int euler_unitigs_clean_ingested(euler_ctx *ctx, uint32_t K, uint32_t limit, con
 {
     ENTER(ctx);
     EULER_TRY(clean_args(ctx, K, params, out_bytes, ncontigs, stats));
-    euler_clean_stats st{};
     const void *d_buf; const u64 *d_off; u64 nr, nb;
     EULER_TRY(pipeline_resident_reads(ctx, &d_buf, &d_off, &nr, &nb));
-    EULER_TRY(unitigs_core(ctx, d_buf, d_off, nr, nb, K, limit, out, out_bytes, ncontigs, params, kmer_sums, &st));
-    if (stats) *stats = st;
-    return EULER_OK;
-}
-
-// flags of the dictionary insert and check: 1 the table is full, 2 a count is not a both-strand count
-static int dict_flags(euler_ctx *ctx, u64 f)
-{
-    if (f & 1) return euler_fail(ctx, EULER_ERR_OVERFLOW, "K-mer table full");
-    if (f & 2) return euler_fail(ctx, EULER_ERR_ARG, "K-mer counts are not both-strand counts (an odd count on a palindrome, "
-                                                     "or a key and its reverse complement with different counts)");
-    return EULER_OK;
+    return unitigs_core(ctx, d_buf, d_off, nr, nb, K, limit, out, out_bytes, ncontigs, params, kmer_sums, stats);
 }
 
 // the dictionary's counts are all kept (limit 0), as in euler_unitigs_from_kmers; they must be both-strand counts,
@@ -408,48 +348,7 @@ int euler_unitigs_clean_from_kmers_wide(euler_ctx *ctx, const uint64_t *keys_lo,
     ENTER(ctx);
     EULER_TRY(clean_args(ctx, K, params, out_bytes, ncontigs, stats));
     if (n && (!keys_lo || !counts || (K > 32 && !keys_hi))) return euler_fail(ctx, EULER_ERR_ARG, "null argument");
-    const u64 cap_out = *out_bytes, cap_sums = *ncontigs;
-    *out_bytes = 0; *ncontigs = 0;
-    if (!n) return EULER_OK;
-    const u64 cap = euler_hash_capacity(n);
-    DevTmp<u64> dlo(ctx, n), flags(ctx, 1);
-    DevTmp<u32> dc(ctx, n), tc(ctx, cap);
-    TMP_CHECK(ctx, dlo); TMP_CHECK(ctx, dc); TMP_CHECK(ctx, tc); TMP_CHECK(ctx, flags);
-    EULER_TRY(upload(ctx, dlo, (const u64 *)keys_lo, n));
-    EULER_TRY(upload(ctx, dc, counts, n));
-    CUDA_TRY(ctx, cudaMemsetAsync(flags, 0, sizeof(u64), ctx->stream));
-    char *d_text = nullptr;
-    u64 bytes = 0, nc = 0, f = 0;
-    euler_clean_stats st{};
-    if (K > 32) {
-        DevTmp<u64> dhi(ctx, n);
-        DevTmp<K128> tk(ctx, cap);
-        TMP_CHECK(ctx, dhi); TMP_CHECK(ctx, tk);
-        EULER_TRY(upload(ctx, dhi, (const u64 *)keys_hi, n));
-        EULER_TRY(wide_table_clear(ctx, tk, tc, cap));
-        EULER_TRY(wide_unitig_dict_table(ctx, dlo, dhi, dc, n, K, tk, tc, cap, flags));
-        EULER_TRY(wide_unitig_dict_check(ctx, dlo, dhi, dc, n, K, tk, tc, cap, flags));
-        EULER_TRY(read_u64(ctx, flags, &f));
-        EULER_TRY(dict_flags(ctx, f));
-        EULER_TRY(wide_unitig_clean_from_table(ctx, tk, tc, cap, K, 0, *params, &d_text, &bytes, &nc, (u64 *)kmer_sums, cap_sums,
-                                               &st));
-    } else {
-        DevTmp<u64> tk(ctx, cap);
-        TMP_CHECK(ctx, tk);
-        EULER_TRY(graph_table_clear(ctx, tk, tc, cap));
-        EULER_TRY(unitig_dict_table(ctx, dlo, dc, n, K, tk, tc, cap, flags));
-        EULER_TRY(unitig_dict_check(ctx, dlo, dc, n, K, tk, tc, cap, flags));
-        EULER_TRY(read_u64(ctx, flags, &f));
-        EULER_TRY(dict_flags(ctx, f));
-        EULER_TRY(unitig_clean_from_table(ctx, tk, tc, cap, K, 0, *params, &d_text, &bytes, &nc, (u64 *)kmer_sums, cap_sums, &st));
-    }
-    *out_bytes = bytes; *ncontigs = nc;
-    if (stats) *stats = st;
-    if (out) {
-        if (cap_out < bytes) return euler_fail(ctx, EULER_ERR_ARG, "output capacity too small");
-        EULER_TRY(download(ctx, out, (const char *)d_text, bytes));
-    }
-    FINISH(ctx);
+    return unitigs_dict_core(ctx, keys_lo, keys_hi, counts, n, K, out, out_bytes, ncontigs, params, kmer_sums, stats);
 }
 
 // link graph G of referenceAssembler.all_contigs :90-111 for n contigs (text: the contigs back to back, no
@@ -469,9 +368,7 @@ int euler_unitig_links(euler_ctx *ctx, const char *text, const uint64_t *off, ui
     TMP_CHECK(ctx, d_text); TMP_CHECK(ctx, d_off); TMP_CHECK(ctx, d_links);
     EULER_TRY(upload(ctx, d_text, text, B));
     EULER_TRY(upload(ctx, d_off, (const u64 *)off, n + 1));
-    // the 64-bit end tables use the all-ones word as EMPTY, which is the poly-T 32-mer: K >= 32 takes 128-bit tables
-    if (K >= 32) EULER_TRY(wide_unitig_link_graph(ctx, d_text, d_off, n, K, d_links));
-    else EULER_TRY(unitig_link_graph(ctx, d_text, d_off, n, K, d_links));
+    EULER_TRY(unitig_link_graph(ctx, d_text, d_off, n, K, d_links));
     EULER_TRY(download(ctx, links, d_links.get(), 16 * n));
     FINISH(ctx);
 }

@@ -1,13 +1,14 @@
-// clean.cu -- tip clipping, isolated-fragment removal and bubble popping on the unitig node graph, then emission.
+// clean.cu -- the link rule of unitig mode, and tip clipping, isolated-fragment removal and bubble popping on the
+// unitig node graph, then emission.  With zero rounds it spells the plain unitigs.
 //
-// Key-independent: the key-width-specific files (unitig.cu, wide_unitig.cu) describe their node graph once, as
+// Key-independent: unitig.cu describes the node graph once, for either key width, as
 //   nbr[4 i + b]  node id of the forward extension of node i by base b, or EULER_NO_ID (absent or filtered),
 //   twin_id[i]    node id of the reverse complement,
-//   cnt[i]        both-strand count,
+//   cnt[i]        both-strand count (read only by the rounds and the sums),
 // and the keys as 64-bit words (key_stride words per node, low word first) for spelling.  From then on everything
 // is node ids.  Every round works on one snapshot of the alive mask:
-//   1. succ: the link rule of unitig.cu on alive nodes (the backward degree of y is the alive forward degree of
-//      twin(y); the hairpin stop is cand == twin(x));
+//   1. succ: the link rule on alive nodes (the backward degree of y is the alive forward degree of twin(y); the
+//      hairpin stop is cand == twin(x));
 //   2. chain_rank (chain.cuh): every node knows its chain head and its distance to it;
 //   3. per path unitig (indexed by its head): sum of counts, tail, L, cov, bubble end point;
 //   4. decisions (rules in euler_b200.h), taken per head on the snapshot;
@@ -46,6 +47,8 @@ __device__ __forceinline__ u32 alive_fw(const u32 *nbr, const unsigned char *ali
     return d;
 }
 
+// referenceAssembler.get_contig_forward :59-77, one step, for every alive node: x -> y iff y is the only alive forward
+// extension of x, x the only alive backward extension of y, and y is not twin(x) (hairpin stop, :70-71)
 __global__ void __launch_bounds__(CB) clean_succ_kernel(const u32 *__restrict__ nbr, const u32 *__restrict__ twin_id,
                                                         const unsigned char *__restrict__ alive, u32 n, u32 *__restrict__ succ)
 {
@@ -191,9 +194,10 @@ int clean_unitigs(euler_ctx *ctx, u32 n, u32 K, const u64 *key_words, u32 key_st
     *d_out = nullptr; *out_bytes = 0; *ncontigs = 0;
     *st = euler_clean_stats{};
     if (!n) return EULER_OK;
-    DevTmp<unsigned char> alive(ctx, n), rm(ctx, n);
-    DevTmp<u32> succ(ctx, n), utail(ctx, n), uS(ctx, n);
-    DevTmp<u64> ucov(ctx, n), stats(ctx, 4);
+    const u32 nr = p.max_rounds ? n : 0;   // rm, utail, uS and ucov serve the rounds only
+    DevTmp<unsigned char> alive(ctx, n), rm(ctx, nr);
+    DevTmp<u32> succ(ctx, n), utail(ctx, nr), uS(ctx, nr);
+    DevTmp<u64> ucov(ctx, nr), stats(ctx, 4);
     TMP_CHECK(ctx, alive); TMP_CHECK(ctx, rm); TMP_CHECK(ctx, succ); TMP_CHECK(ctx, utail); TMP_CHECK(ctx, uS);
     TMP_CHECK(ctx, ucov); TMP_CHECK(ctx, stats);
     ChainRanks r(ctx, n);

@@ -105,26 +105,25 @@ int tour_emit_contigs(euler_ctx *ctx, const euler_vertex *ev, u32 vcount, const 
 // ---- synth.cu
 int synth_reads(euler_ctx *ctx, u64 G, u32 L, u32 err_ppm, u64 first, u64 nreads, void *d_out);
 
-// ---- unitig.cu
-int unitig_from_table(euler_ctx *ctx, const u64 *keys, const u32 *cnt, u64 cap, u32 K, u32 limit, char **d_out,
-                      u64 *out_bytes, u64 *ncontigs, u64 *n_nodes);
-
-// unitig_from_table after the graph clean-up of clean.cu; h_sums (host, sums_cap entries, may be NULL): per-contig
-// sums of the both-strand counts, in output order
-int unitig_clean_from_table(euler_ctx *ctx, const u64 *keys, const u32 *cnt, u64 cap, u32 K, u32 limit,
-                            const euler_clean_params &p, char **d_out, u64 *out_bytes, u64 *ncontigs, u64 *h_sums,
-                            u64 sums_cap, euler_clean_stats *st);
-
-// canonical count table from a both-strand K-mer dictionary (keys, counts)
+// ---- unitig.cu (K = 2..63; the key width follows from K there)
+// unitigs of the reads (d_off[nreads + 1], B bases), text in ctx->text_buf.  cp == NULL: plain; else after the graph
+// clean-up of clean.cu, with h_sums (host, sums_cap entries, may be NULL) the per-contig sums of the both-strand counts
+// in output order
+int unitigs_from_reads(euler_ctx *ctx, const void *d_buf, const u64 *d_off, u64 nreads, u64 B, u32 K, u32 limit,
+                       const euler_clean_params *cp, char **d_out, u64 *out_bytes, u64 *ncontigs, u64 *h_sums, u64 sums_cap,
+                       euler_clean_stats *st);
+// the same on a both-strand K-mer dictionary of n > 0 keys (low words d_lo, high words d_hi read for K > 32), all kept;
+// with cp the counts must be both-strand counts
+int unitigs_from_dict(euler_ctx *ctx, const u64 *d_lo, const u64 *d_hi, const u32 *d_counts, u64 n, u32 K,
+                      const euler_clean_params *cp, char **d_out, u64 *out_bytes, u64 *ncontigs, u64 *h_sums, u64 sums_cap,
+                      euler_clean_stats *st);
+// canonical count table (one-word keys, K <= 32) from a both-strand K-mer dictionary (keys, counts)
 int unitig_dict_table(euler_ctx *ctx, const u64 *d_keys, const u32 *d_counts, u64 n, u32 K, u64 *tk, u32 *tc, u64 cap, u64 *d_flags);
-// after unitig_dict_table: sets bit 2 of *d_flags when a count is not the both-strand count of its key in the table
-int unitig_dict_check(euler_ctx *ctx, const u64 *d_keys, const u32 *d_counts, u64 n, u32 K, const u64 *tk, const u32 *tc, u64 cap,
-                      u64 *d_flags);
 // link graph of n contigs (text without separators, off[n+1]): links[16 i + 8 side + 2 base + (0 head '+' | 1 tail '-')]
 int unitig_link_graph(euler_ctx *ctx, const char *d_text, const u64 *d_off, u64 n, u32 K, u32 *d_links);
 
-// ---- clean.cu (key-independent): n nodes with forward extensions nbr[4 n], twin_id[n], both-strand counts cnt[n] and
-// keys of key_stride 64-bit words each (low word first)
+// ---- clean.cu (key-independent): n nodes with forward extensions nbr[4 n], twin_id[n], both-strand counts cnt[n]
+// (read only with rounds or sums) and keys of key_stride 64-bit words each (low word first)
 int clean_unitigs(euler_ctx *ctx, u32 n, u32 K, const u64 *key_words, u32 key_stride, const u32 *nbr, const u32 *twin_id,
                   const u32 *cnt, const euler_clean_params &p, char **d_out, u64 *out_bytes, u64 *ncontigs, u64 *h_sums,
                   u64 sums_cap, euler_clean_stats *st);
