@@ -215,6 +215,39 @@ int euler_unitigs_clean_from_kmers_wide(euler_ctx *ctx, const uint64_t *keys_lo,
                                         char *out, uint64_t *out_bytes, uint64_t *ncontigs, uint64_t *kmer_sums,
                                         euler_clean_stats *stats);
 
+/* Multi-k unitigs.  One K cannot serve both ends of the trade-off: a small K keeps the graph connected where coverage
+ * is thin, a large K resolves repeats.  So, as multi-k assemblers (IDBA, SPAdes, MEGAHIT) do, the contigs of each step
+ * spell the K-mers of the next, larger K that the reads cover too thinly.  Input: the reads, ks[0] < ... < ks[nk - 1]
+ * (1 <= nk <= EULER_MULTIK_MAX, each K in [2,63]), limit, params[nk].  Step i:
+ *   1. counts the both-strand ks[i]-mers of the reads as euler_unitigs_clean does;
+ *   2. for i > 0, gives every contig C written by step i - 1 the weight w_C = max(limit + 1, floor(kmer_sum_C / L_C)),
+ *      L_C = C's number of ks[i - 1]-mers;
+ *   3. every ks[i]-mer x that C spells, in either orientation, gets the count max(count(x), w_C), the maximum taken
+ *      over all contigs that spell x; on a palindromic x the count is rounded up to even (the table keeps ceil(w / 2),
+ *      as for a dictionary input), so counts stay both-strand counts;
+ *   4. a contig of fewer than ks[i] bases spells nothing;
+ *   5. a contig step i - 1 wrote as a cycle spells the ks[i]-mers of its cyclic sequence, all L_C rotations, so step i
+ *      does not depend on where the cycle was cut;
+ *   6. the nodes are the K-mers with count > limit; they are cleaned with params[i] and written as in
+ *      euler_unitigs_clean.
+ * The output is the last step's contigs and kmer_sums (the sums include the raised counts).  With nk = 1 it is
+ * euler_unitigs_clean.  Nothing depends on thread order or slot layout, so the output set is a function of the reads
+ * and the parameters.  Two-call protocol as euler_unitigs_clean; steps (nk entries, may be NULL) reports each step. */
+#define EULER_MULTIK_MAX 16
+typedef struct {
+    uint32_t K;
+    uint64_t contigs, bases;      /* that step's contigs and their bases (without the '\n') */
+    uint64_t nodes_added;         /* canonical K-mers that are nodes only because of the previous step's contigs */
+    euler_clean_stats clean;      /* that step's clean-up */
+} euler_multik_step;
+int euler_unitigs_multik(euler_ctx *ctx, const char *buf, const uint64_t *read_off, uint64_t nreads, const uint32_t *ks,
+                         uint32_t nk, uint32_t limit, const euler_clean_params *params, char *out, uint64_t *out_bytes,
+                         uint64_t *ncontigs, uint64_t *kmer_sums, euler_multik_step *steps);
+/* the same on the reads left on the device by euler_ingest */
+int euler_unitigs_multik_ingested(euler_ctx *ctx, const uint32_t *ks, uint32_t nk, uint32_t limit,
+                                  const euler_clean_params *params, char *out, uint64_t *out_bytes, uint64_t *ncontigs,
+                                  uint64_t *kmer_sums, euler_multik_step *steps);
+
 /* =========================================================================================
  * Fused device-resident pipeline (the measured hot path)
  * ======================================================================================= */

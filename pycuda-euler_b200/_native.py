@@ -64,6 +64,18 @@ class CleanStats(C.Structure):
         return {k: int(getattr(self, k)) for k, _ in self._fields_}
 
 
+class MultikStep(C.Structure):
+    """euler_multik_step"""
+    _fields_ = [("K", C.c_uint32), ("contigs", C.c_uint64), ("bases", C.c_uint64), ("nodes_added", C.c_uint64),
+                ("clean", CleanStats)]
+
+    def as_dict(self):
+        return {"K": int(self.K), "contigs": int(self.contigs), "bases": int(self.bases),
+                "nodes_added": int(self.nodes_added), "clean": self.clean.as_dict()}
+
+
+MULTIK_MAX = 16   # EULER_MULTIK_MAX
+
 _lib = None
 
 
@@ -93,6 +105,8 @@ def load():
         "euler_unitigs_clean": [vp, vp, vp, u64, u32, u32, vp, vp, vp, vp, vp, vp],
         "euler_unitigs_clean_ingested": [vp, u32, u32, vp, vp, vp, vp, vp, vp],
         "euler_unitigs_clean_from_kmers_wide": [vp, vp, vp, vp, u64, u32, vp, vp, vp, vp, vp, vp],
+        "euler_unitigs_multik": [vp, vp, vp, u64, vp, u32, u32, vp, vp, vp, vp, vp, vp],
+        "euler_unitigs_multik_ingested": [vp, vp, u32, u32, vp, vp, vp, vp, vp, vp],
         "euler_hash_build": [vp, vp, vp, u64, u64, vp, vp],
         "euler_hash_lookup": [vp, vp, vp, u64, vp, u64, vp],
         "euler_exclusive_scan_u32": [vp, vp, u64, vp],
@@ -343,6 +357,49 @@ class Context:
             return self.lib.euler_unitigs_clean_from_kmers_wide(self.h, _p(keys), _p(keys_hi), _p(counts), len(keys), int(K), p,
                                                                 out, nb, nc, sums, st)
         return self._clean_call(call, K, tip_len, isolated_len, bubble_len, max_rounds)
+
+    def _multik_call(self, call, ks, clean, tip_len, isolated_len, bubble_len, max_rounds):
+        """two-call protocol of the euler_unitigs_multik* entry points -> (contigs, kmer_sums, list of step dicts)"""
+        ks = [int(k) for k in ks]
+        nk = len(ks)
+        karr = (C.c_uint32 * max(nk, 1))(*ks)
+        P = (CleanParams * max(nk, 1))()
+        for i, k in enumerate(ks):
+            d = lambda v: 0 if not clean else (2 * k if v is None else int(v))
+            P[i] = CleanParams(d(tip_len), d(isolated_len), d(bubble_len), int(max_rounds) if clean else 0)
+        st = (MultikStep * max(nk, 1))()
+        nb, nc = C.c_uint64(0), C.c_uint64(0)
+        self.check(call(karr, nk, P, None, C.byref(nb), C.byref(nc), None, st))
+        if nb.value:
+            out = np.zeros(nb.value, np.uint8)
+            sums = np.zeros(nc.value, np.uint64)
+            cap, nc2 = C.c_uint64(nb.value), C.c_uint64(nc.value)
+            self.check(call(karr, nk, P, _p(out), C.byref(cap), C.byref(nc2), _p(sums), st))
+            contigs = out.tobytes().decode("ascii").split("\n")[:-1]
+        else:
+            contigs, sums = [], np.zeros(0, np.uint64)
+        return contigs, sums, [st[i].as_dict() for i in range(nk)]
+
+    def unitigs_multik(self, buf, off, ks, limit=1, clean=True, tip_len=None, isolated_len=None, bubble_len=None,
+                       max_rounds=10):
+        """multi-k unitigs (euler_unitigs_multik): for ks strictly increasing, each step's contigs add their K-mers to
+        the next step's graph -> (contigs, kmer_sums, steps), the contigs and sums of the last step and one dict per
+        step (K, contigs, bases, nodes_added, clean).  A length of None means 2 K at each step; clean=False runs no
+        round at any step (plain unitigs per step)."""
+        buf = _arr(buf, np.uint8)
+        off = _arr(off, np.uint64)
+
+        def call(ka, nk, p, out, nb, nc, sums, st):
+            return self.lib.euler_unitigs_multik(self.h, _p(buf), _p(off), len(off) - 1, ka, nk, int(limit), p, out, nb, nc,
+                                                 sums, st)
+        return self._multik_call(call, ks, clean, tip_len, isolated_len, bubble_len, max_rounds)
+
+    def unitigs_multik_ingested(self, ks, limit=1, clean=True, tip_len=None, isolated_len=None, bubble_len=None,
+                                max_rounds=10):
+        """unitigs_multik on the reads left resident by ingest"""
+        def call(ka, nk, p, out, nb, nc, sums, st):
+            return self.lib.euler_unitigs_multik_ingested(self.h, ka, nk, int(limit), p, out, nb, nc, sums, st)
+        return self._multik_call(call, ks, clean, tip_len, isolated_len, bubble_len, max_rounds)
 
     def unitig_links(self, contigs, K):
         """(n, 16) uint32 link table of referenceAssembler.all_contigs' G (see euler_unitig_links)"""

@@ -6,6 +6,7 @@
     python assembler.py -i reads.fq -o contigs.fa -k 31                      # one GPU
     python assembler.py -i reads.fq -o contigs.fa -k 63                      # one GPU, k up to 63
     python assembler.py -i reads.fq -o contigs.fa -k 31 --clean              # clip tips, pop bubbles first
+    python assembler.py -i reads.fq -o contigs.fa --k-list 21,41,63 --clean  # multi-k: one GPU or replicas
     python -m torch.distributed.run --nproc-per-node 8 --master-addr 127.0.0.1 \\
            assembler.py -i reads.fq -o contigs.fa -k 31                      # 8 GPUs, one assembly
 
@@ -29,6 +30,12 @@ written: tips (dead-end branches), isolated fragments and the weaker branches of
 K-mers (--tip-len, --isolated-len, --bubble-len; default 2k, 0 turns a rule off), for up to --clean-rounds rounds
 (rules: include/euler_b200.h, euler_unitigs_clean).  The GFA's S lines then carry KC:i:<sum of the contig's K-mer
 counts>, and the log gets a line with the rounds and the removals.
+
+--k-list k1,k2,... (strictly increasing, 2..63, at most 16; in place of -k) assembles at each K in turn and adds the
+K-mers of each step's contigs to the graph of the next (rule: include/euler_b200.h, euler_unitigs_multik), so a small
+K bridges thinly covered places and a large K resolves repeats.  With --clean every step is cleaned up (the lengths
+default to 2k at each step).  One GPU and replicas mode only.  The log gets one line per step; the FASTA and the GFA
+(link graph at the last K, KC:i: from the last step's sums) are those of the last step.
 """
 import argparse
 import logging
@@ -92,11 +99,20 @@ def log_clean(log, rank, st):
              st["tips"], st["isolated"], st["bubble_branches"], st["kmers_removed"])
 
 
+def log_step(log, rank, s, clean):
+    c = s["clean"]
+    log.info("rank %d: K = %d: %d contigs, %d bases, %d K-mers added from the previous contigs%s", rank, s["K"],
+             s["contigs"], s["bases"], s["nodes_added"],
+             "; clean-up: %d rounds, %d tips, %d isolated, %d bubble branches, %d K-mers removed" %
+             (c["rounds"], c["tips"], c["isolated"], c["bubble_branches"], c["kmers_removed"]) if clean else "")
+
+
 def main(argv=None):
     ap = argparse.ArgumentParser(description=__doc__, formatter_class=argparse.RawDescriptionHelpFormatter)
     ap.add_argument('-i', dest='input_filename', required=True, help='Input File Name (FASTA / FASTQ)')
     ap.add_argument('-o', dest='output_filename', required=True, help='Output File Name')
-    ap.add_argument('-k', dest='k', type=int, default=31, help='kmer size')
+    ap.add_argument('-k', dest='k', type=int, default=None, help='kmer size (default 31)')
+    ap.add_argument('--k-list', default=None, help='multi-k: strictly increasing K values, e.g. 21,41,63 (not with -k)')
     ap.add_argument('-d', action='store_true', default=False, help='Use DDFS (accepted for compatibility; ignored)')
     ap.add_argument('--limit', type=int, default=1, help='keep k-mers with both-strand count > limit (build() default 1)')
     ap.add_argument('--mode', choices=['unitig', 'euler', 'replicas'], default='unitig')
@@ -106,6 +122,24 @@ def main(argv=None):
     ap.add_argument('--bubble-len', type=int, default=None, help='longest bubble branch removed, in K-mers (default 2k)')
     ap.add_argument('--clean-rounds', type=int, default=10, help='most clean-up rounds')
     args = ap.parse_args(argv)
+    ks = None
+    if args.k_list is not None:
+        if args.k is not None:
+            ap.error("give either -k or --k-list, not both")
+        try:
+            ks = [int(x) for x in args.k_list.split(",")]
+        except ValueError:
+            ap.error("--k-list takes comma-separated integers, got %r" % args.k_list)
+        if args.mode == 'euler':
+            ap.error("--k-list is a unitig-mode option; --mode euler takes one -k")
+        if not 1 <= len(ks) <= 16:   # EULER_MULTIK_MAX
+            ap.error("--k-list takes 1 to 16 values, got %d" % len(ks))
+        if any(k < 2 or k > 63 for k in ks):
+            ap.error("--k-list values must be in [2, 63], got %s" % args.k_list)
+        if any(b <= a for a, b in zip(ks, ks[1:])):
+            ap.error("--k-list must be strictly increasing, got %s" % args.k_list)
+    if args.k is None:
+        args.k = 31 if ks is None else ks[-1]
     logging.basicConfig(level=logging.INFO, format='%(asctime)s %(levelname)s %(message)s')
     log = logging.getLogger("assembler")
 
@@ -130,9 +164,16 @@ def main(argv=None):
         write_outputs(args.output_filename, contigs, None, K)
         log.info("%d contigs -> %s", len(contigs), args.output_filename)
         return 0
+    if ks is not None and world > 1 and args.mode != 'replicas':
+        raise SystemExit("--k-list runs on one GPU or in replicas mode; one assembly across GPUs takes one -k")
     if world == 1 or args.mode == 'replicas':
         kc = None
-        if args.clean:
+        if ks is not None:
+            contigs, kc, steps = ctx.unitigs_multik_ingested(ks, args.limit, clean=args.clean, **clean_kwargs(args)) \
+                if nbases else ([], None, [])
+            for s in steps:
+                log_step(log, rank, s, args.clean)
+        elif args.clean:
             contigs, kc, st = ctx.unitigs_clean_ingested(K, args.limit, **clean_kwargs(args)) if nbases else ([], None, None)
             if st:
                 log_clean(log, rank, st)

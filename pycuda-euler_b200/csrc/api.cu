@@ -351,6 +351,67 @@ int euler_unitigs_clean_from_kmers_wide(euler_ctx *ctx, const uint64_t *keys_lo,
     return unitigs_dict_core(ctx, keys_lo, keys_hi, counts, n, K, out, out_bytes, ncontigs, params, kmer_sums, stats);
 }
 
+static int multik_args(euler_ctx *ctx, const uint32_t *ks, uint32_t nk, const euler_clean_params *params, uint64_t *out_bytes,
+                       uint64_t *ncontigs, euler_multik_step *steps)
+{
+    if (!ks || !params || !out_bytes || !ncontigs) return euler_fail(ctx, EULER_ERR_ARG, "null argument");
+    if (nk < 1 || nk > EULER_MULTIK_MAX)
+        return euler_fail(ctx, EULER_ERR_ARG, "K list of %u entries, expected 1 to %d", nk, EULER_MULTIK_MAX);
+    for (u32 i = 0; i < nk; i++) {
+        if (ks[i] < 2 || ks[i] > 63) return euler_fail(ctx, EULER_ERR_ARG, "K %u out of range [2,63]", ks[i]);
+        if (i && ks[i] <= ks[i - 1])
+            return euler_fail(ctx, EULER_ERR_ARG, "K list is not strictly increasing (%u after %u)", ks[i], ks[i - 1]);
+    }
+    if (steps)
+        for (u32 i = 0; i < nk; i++) steps[i] = euler_multik_step{ks[i], 0, 0, 0, euler_clean_stats{}};
+    return EULER_OK;
+}
+
+// two-call protocol as unitigs_core; the work runs on both calls
+static int multik_core(euler_ctx *ctx, const void *d_buf, const u64 *d_off, u64 nreads, u64 B, const uint32_t *ks, uint32_t nk,
+                       uint32_t limit, const euler_clean_params *params, char *out, uint64_t *out_bytes, uint64_t *ncontigs,
+                       uint64_t *sums, euler_multik_step *steps)
+{
+    const u64 cap_out = *out_bytes, cap_sums = *ncontigs;
+    *out_bytes = 0; *ncontigs = 0;
+    if (!B) return EULER_OK;
+    char *d_text = nullptr;
+    u64 bytes = 0, nc = 0;
+    EULER_TRY(unitigs_multik(ctx, d_buf, d_off, nreads, B, ks, nk, limit, params, &d_text, &bytes, &nc, (u64 *)sums, cap_sums, steps));
+    *out_bytes = bytes; *ncontigs = nc;
+    if (out) {
+        if (cap_out < bytes) return euler_fail(ctx, EULER_ERR_ARG, "output capacity too small");
+        EULER_TRY(download(ctx, out, (const char *)d_text, bytes));
+    }
+    FINISH(ctx);
+}
+
+int euler_unitigs_multik(euler_ctx *ctx, const char *buf, const uint64_t *read_off, uint64_t nreads, const uint32_t *ks,
+                         uint32_t nk, uint32_t limit, const euler_clean_params *params, char *out, uint64_t *out_bytes,
+                         uint64_t *ncontigs, uint64_t *kmer_sums, euler_multik_step *steps)
+{
+    ENTER(ctx);
+    if (!read_off) return euler_fail(ctx, EULER_ERR_ARG, "null argument");
+    EULER_TRY(multik_args(ctx, ks, nk, params, out_bytes, ncontigs, steps));
+    const u64 B = read_off[nreads];
+    DevTmp<unsigned char> d_buf(ctx, B + 16);
+    DevTmp<u64> d_off(ctx, nreads + 1);
+    EULER_TRY(upload(ctx, d_buf, (const unsigned char *)buf, B));
+    EULER_TRY(upload(ctx, d_off, (const u64 *)read_off, nreads + 1));
+    return multik_core(ctx, d_buf, d_off, nreads, B, ks, nk, limit, params, out, out_bytes, ncontigs, kmer_sums, steps);
+}
+
+int euler_unitigs_multik_ingested(euler_ctx *ctx, const uint32_t *ks, uint32_t nk, uint32_t limit,
+                                  const euler_clean_params *params, char *out, uint64_t *out_bytes, uint64_t *ncontigs,
+                                  uint64_t *kmer_sums, euler_multik_step *steps)
+{
+    ENTER(ctx);
+    EULER_TRY(multik_args(ctx, ks, nk, params, out_bytes, ncontigs, steps));
+    const void *d_buf; const u64 *d_off; u64 nr, nb;
+    EULER_TRY(pipeline_resident_reads(ctx, &d_buf, &d_off, &nr, &nb));
+    return multik_core(ctx, d_buf, d_off, nr, nb, ks, nk, limit, params, out, out_bytes, ncontigs, kmer_sums, steps);
+}
+
 // link graph G of referenceAssembler.all_contigs :90-111 for n contigs (text: the contigs back to back, no
 // separators; off[n+1]).  links: u32[16 n], entry [16 i + 8 side + 2 base + o]: side 0 = successors of the last
 // K-mer, side 1 = of twin(first K-mer); o = 0: the hit is a contig head ('+'), o = 1: a tail ('-'); 0xffffffff = none.

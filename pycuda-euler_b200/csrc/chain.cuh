@@ -191,10 +191,11 @@ static int chain_rank(euler_ctx *ctx, M m, u32 n, ChainRanks &r)
 }
 
 // The emitting half on ranks of the same model: contig order (ord1 / ord2, *n_starts = number of path contigs),
-// lengths, text.  Emits into ctx->text_buf.
+// lengths, text.  Emits into ctx->text_buf.  keep_off (may be NULL): the contig offsets on the device, with the text
+// bytes as entry ncontigs.
 template <typename M>
 static int chain_spell(euler_ctx *ctx, M m, u32 n, u32 k, ChainRanks &r, char **d_out, u64 *out_bytes, u64 *ncontigs,
-                       u32 *n_starts = nullptr)
+                       u32 *n_starts = nullptr, DevArr<u64> *keep_off = nullptr)
 {
     const unsigned g = grid_for(n, CH_TB);
     cudaStream_t s = ctx->stream;
@@ -220,6 +221,11 @@ static int chain_spell(euler_ctx *ctx, M m, u32 n, u32 k, ChainRanks &r, char **
     ch_write_kernel<<<g, CH_TB, 0, s>>>(m, r.head_kind, cur, r.ord1, r.ord2, (u32)h[0], n, k, off_by_ord, len_by_ord,
                                         (char *)ctx->text_buf.p);
     CUDA_TRY(ctx, cudaGetLastError());
+    if (keep_off) {
+        EULER_TRY(keep_off->reserve(ctx, nc + 1));
+        CUDA_TRY(ctx, cudaMemcpyAsync(keep_off->ptr(), off_by_ord.get(), nc * sizeof(u64), cudaMemcpyDeviceToDevice, s));
+        CUDA_TRY(ctx, cudaMemcpyAsync(keep_off->ptr() + nc, r.totals.get() + 2, sizeof(u64), cudaMemcpyDeviceToDevice, s));
+    }
     CUDA_TRY(ctx, cudaStreamSynchronize(s));
     ctx->text_gen++;
     *d_out = (char *)ctx->text_buf.p;

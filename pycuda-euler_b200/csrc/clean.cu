@@ -189,9 +189,10 @@ static __global__ void __launch_bounds__(CB) clean_fill_kernel(unsigned char *p,
 
 int clean_unitigs(euler_ctx *ctx, u32 n, u32 K, const u64 *key_words, u32 key_stride, const u32 *nbr, const u32 *twin_id,
                   const u32 *cnt, const euler_clean_params &p, char **d_out, u64 *out_bytes, u64 *ncontigs, u64 *h_sums,
-                  u64 sums_cap, euler_clean_stats *st)
+                  u64 sums_cap, euler_clean_stats *st, UnitigsKept *keep)
 {
     *d_out = nullptr; *out_bytes = 0; *ncontigs = 0;
+    if (keep) keep->n_starts = 0;
     *st = euler_clean_stats{};
     if (!n) return EULER_OK;
     const u32 nr = p.max_rounds ? n : 0;   // rm, utail, uS and ucov serve the rounds only
@@ -234,15 +235,19 @@ int clean_unitigs(euler_ctx *ctx, u32 n, u32 K, const u64 *key_words, u32 key_st
         EULER_TRY(chain_rank(ctx, m, n, r));
     }
     u32 n_starts = 0;
-    EULER_TRY(chain_spell(ctx, m, n, K, r, d_out, out_bytes, ncontigs, &n_starts));
-    if (!h_sums || !*ncontigs) return EULER_OK;
-    if (sums_cap < *ncontigs) return euler_fail(ctx, EULER_ERR_ARG, "kmer_sums capacity too small (%llu < %llu)", sums_cap, *ncontigs);
-    DevTmp<u64> sums(ctx, *ncontigs);
-    TMP_CHECK(ctx, sums);
+    EULER_TRY(chain_spell(ctx, m, n, K, r, d_out, out_bytes, ncontigs, &n_starts, keep ? &keep->off : nullptr));
+    if (keep) keep->n_starts = n_starts;
+    if ((!h_sums && !keep) || !*ncontigs) return EULER_OK;
+    if (h_sums && sums_cap < *ncontigs)
+        return euler_fail(ctx, EULER_ERR_ARG, "kmer_sums capacity too small (%llu < %llu)", sums_cap, *ncontigs);
+    DevTmp<u64> tmp_sums(ctx, keep ? 0 : *ncontigs);
+    TMP_CHECK(ctx, tmp_sums);
+    if (keep) EULER_TRY(keep->sums.reserve(ctx, *ncontigs));
+    u64 *sums = keep ? keep->sums.ptr() : tmp_sums.get();
     CUDA_TRY(ctx, cudaMemsetAsync(sums, 0, *ncontigs * sizeof(u64), s));
     clean_contig_sums_kernel<<<g, CB, 0, s>>>(r.anc, r.head_kind, r.ord1, r.ord2, n_starts, cnt, n, sums);
     CUDA_TRY(ctx, cudaGetLastError());
-    CUDA_TRY(ctx, cudaMemcpyAsync(h_sums, sums.get(), *ncontigs * sizeof(u64), cudaMemcpyDeviceToHost, s));
+    if (h_sums) CUDA_TRY(ctx, cudaMemcpyAsync(h_sums, sums, *ncontigs * sizeof(u64), cudaMemcpyDeviceToHost, s));
     CUDA_TRY(ctx, cudaStreamSynchronize(s));
     return EULER_OK;
 }

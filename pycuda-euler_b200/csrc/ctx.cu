@@ -58,7 +58,7 @@ int scan_state_reserve(euler_ctx *ctx, u64 ntiles, ScanState **state, u64 **coun
 
 extern "C" {
 
-int euler_version(void) { return 102; }
+int euler_version(void) { return 103; }
 
 int euler_ctx_create(int device, euler_ctx **out)
 {

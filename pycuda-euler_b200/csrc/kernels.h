@@ -121,12 +121,26 @@ int unitigs_from_dict(euler_ctx *ctx, const u64 *d_lo, const u64 *d_hi, const u3
 int unitig_dict_table(euler_ctx *ctx, const u64 *d_keys, const u32 *d_counts, u64 n, u32 K, u64 *tk, u32 *tc, u64 cap, u64 *d_flags);
 // link graph of n contigs (text without separators, off[n+1]): links[16 i + 8 side + 2 base + (0 head '+' | 1 tail '-')]
 int unitig_link_graph(euler_ctx *ctx, const char *d_text, const u64 *d_off, u64 n, u32 K, u32 *d_links);
+// multi-k unitigs (the rule in euler_b200.h) of the reads for ks[0] < .. < ks[nk - 1]: the last step's text in
+// ctx->text_buf, its sums in h_sums (may be NULL), one euler_multik_step per step in steps (may be NULL)
+int unitigs_multik(euler_ctx *ctx, const void *d_buf, const u64 *d_off, u64 nreads, u64 B, const u32 *ks, u32 nk, u32 limit,
+                   const euler_clean_params *params, char **d_out, u64 *out_bytes, u64 *ncontigs, u64 *h_sums, u64 sums_cap,
+                   euler_multik_step *steps);
+
+// clean_unitigs' output left on the device for the caller: contig i is ctx->text_buf[off[i], off[i + 1]) with its '\n'
+// (off[ncontigs] = the text bytes), sums[i] its count sum; contigs from n_starts on are cycles.  The buffers grow only.
+struct UnitigsKept {
+    DevArr<u64> off, sums;
+    u32 n_starts = 0;
+    void free() { off.free(); sums.free(); }
+};
 
 // ---- clean.cu (key-independent): n nodes with forward extensions nbr[4 n], twin_id[n], both-strand counts cnt[n]
-// (read only with rounds or sums) and keys of key_stride 64-bit words each (low word first)
+// (read only with rounds, sums or keep) and keys of key_stride 64-bit words each (low word first).  keep (may be NULL):
+// leave offsets, sums and n_starts on the device as well
 int clean_unitigs(euler_ctx *ctx, u32 n, u32 K, const u64 *key_words, u32 key_stride, const u32 *nbr, const u32 *twin_id,
                   const u32 *cnt, const euler_clean_params &p, char **d_out, u64 *out_bytes, u64 *ncontigs, u64 *h_sums,
-                  u64 sums_cap, euler_clean_stats *st);
+                  u64 sums_cap, euler_clean_stats *st, UnitigsKept *keep = nullptr);
 
 // ---- graph.cu, fused fast path
 // pair scan over l-mer table slots: base = distinct both-strand l-mer index, eoff = edge offset;

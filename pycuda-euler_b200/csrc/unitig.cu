@@ -124,7 +124,7 @@ __global__ void __launch_bounds__(UB) unitig_nbr_kernel(const Key *__restrict__ 
 template <typename Key>
 static int unitigs_from_table(euler_ctx *ctx, const Key *keys, const u32 *cnt, u64 cap, u32 K, u32 limit,
                               const euler_clean_params *cp, char **d_out, u64 *out_bytes, u64 *ncontigs, u64 *h_sums,
-                              u64 sums_cap, euler_clean_stats *st)
+                              u64 sums_cap, euler_clean_stats *st, UnitigsKept *keep = nullptr)
 {
     *d_out = nullptr; *out_bytes = 0; *ncontigs = 0; *st = euler_clean_stats{};
     DevTmp<u32> base(ctx, cap);
@@ -136,7 +136,7 @@ static int unitigs_from_table(euler_ctx *ctx, const Key *keys, const u32 *cnt, u
     if (!n) return EULER_OK;
     if (n >= 0xffffffffull) return euler_fail(ctx, EULER_ERR_RANGE, "unitig node count exceeds u32");
     const euler_clean_params p = cp ? *cp : euler_clean_params{};   // plain unitigs: no round
-    const bool counts = p.max_rounds || h_sums;
+    const bool counts = p.max_rounds || h_sums || keep;
     DevTmp<Key> nkeys(ctx, n);
     DevTmp<u32> nbr(ctx, 4 * n), twin_id(ctx, n), ncnt(ctx, counts ? n : 0);
     TMP_CHECK(ctx, nkeys); TMP_CHECK(ctx, nbr); TMP_CHECK(ctx, twin_id); TMP_CHECK(ctx, ncnt);
@@ -145,7 +145,7 @@ static int unitigs_from_table(euler_ctx *ctx, const Key *keys, const u32 *cnt, u
                                                                 counts ? ncnt.get() : nullptr);
     CUDA_TRY(ctx, cudaGetLastError());
     return clean_unitigs(ctx, (u32)n, K, (const u64 *)nkeys.get(), sizeof(Key) / sizeof(u64), nbr, twin_id,
-                         counts ? ncnt.get() : nullptr, p, d_out, out_bytes, ncontigs, h_sums, sums_cap, st);
+                         counts ? ncnt.get() : nullptr, p, d_out, out_bytes, ncontigs, h_sums, sums_cap, st, keep);
 }
 
 template <typename Key>
@@ -327,4 +327,129 @@ int unitig_link_graph(euler_ctx *ctx, const char *d_text, const u64 *d_off, u64 
     if (!n) return EULER_OK;
     if (K <= 31) return link_graph_w<u64>(ctx, d_text, d_off, n, K, d_links);
     return link_graph_w<K128>(ctx, d_text, d_off, n, K, d_links);
+}
+
+// ---- multi-k: the contigs of step i - 1 raise the counts of step i (rule in euler_b200.h) -----------------------
+__device__ __forceinline__ u64 rc_push(u64 r, u32 code, u32 K) { return (r >> 2) | ((u64)(3u - code) << (2 * (K - 1))); }
+__device__ __forceinline__ K128 rc_push(K128 r, u32 code, u32 K) { return shr2_or_top(r, 3u - code, 2 * (K - 1)); }
+__device__ __forceinline__ u32 text_code(const char *s, u64 i)
+{
+    const unsigned char c = (unsigned char)s[i];
+    return ((c >> 1) ^ (c >> 2)) & 3u;
+}
+
+#define MK_RUN 64   // window starts per thread
+
+// Every K-window of the previous step's contigs (text, off[nc + 1] with '\n' terminators, count sums, contigs from
+// n_starts on are cycles written on Kp-mers): count = max(count, w_C) with w_C = max(limit + 1, sum / L_C), ceil(w / 2)
+// on a palindrome.  A thread covers MK_RUN consecutive text positions, rolling both strands through each contig's run.
+// A cycle of L_C K-mers is read as its cyclic sequence text[0, L_C) from its start, so it gives all L_C rotations.
+// stats[2] |= 1 on a full table; stats[4] += canonical K-mers whose count crosses limit here.
+template <typename Key>
+__global__ void __launch_bounds__(UB) multik_contig_kmers_kernel(const char *__restrict__ text, const u64 *__restrict__ off,
+                                                                  const u64 *__restrict__ sums, u64 nc, u64 n_starts, u32 Kp,
+                                                                  u32 K, u32 limit, Key *__restrict__ tk, u32 *__restrict__ tc,
+                                                                  u64 cap, u64 *__restrict__ stats)
+{
+    const u64 p0 = ((u64)blockIdx.x * blockDim.x + threadIdx.x) * MK_RUN;
+    const u64 bytes = off[nc];
+    if (p0 >= bytes) return;
+    const u64 p1 = p0 + MK_RUN < bytes ? p0 + MK_RUN : bytes;
+    u64 lo = 0, hi = nc;   // the contig holding p0: the last c with off[c] <= p0
+    while (hi - lo > 1) {
+        const u64 mid = (lo + hi) / 2;
+        if (off[mid] <= p0) lo = mid; else hi = mid;
+    }
+    u64 added = 0;
+    bool full = false;
+    for (u64 c = lo; c < nc && off[c] < p1; c++) {
+        const u64 b = off[c], n = off[c + 1] - b - 1, L = n - Kp + 1;   // bases, Kp-mers
+        if (n < K) continue;
+        const bool cyc = c >= n_starts;
+        const u64 s = p0 > b ? p0 - b : 0, e0 = cyc ? L : n - K + 1, e = p1 - b < e0 ? p1 - b : e0;   // window starts [s, e)
+        if (s >= e) continue;
+        const u64 wm = sums[c] / L;
+        const u32 w = (u32)(wm > (u64)limit + 1 ? (wm < 0xffffffffull ? wm : 0xffffffffull) : (u64)limit + 1);
+        Key x{}, r{};
+        for (u64 j = s; j < s + K - 1; j++) {
+            const u32 code = text_code(text + b, j < n ? j : j % L);
+            x = shl_base(x, code);
+            r = rc_push(r, code, K);
+        }
+        for (u64 i = s; i < e; i++) {
+            const u64 j = i + K - 1;
+            const u32 code = text_code(text + b, j < n ? j : j % L);
+            x = push_base(x, code, K);
+            r = rc_push(r, code, K);
+            const bool pal = x == r;
+            const u64 slot = key_insert(tk, cap, r < x ? r : x);
+            if (slot == EULER_NO_SLOT) { full = true; continue; }
+            const u32 v = pal ? (u32)(((u64)w + 1u) / 2u) : w;   // in u64: w may be 0xffffffff
+            const u32 old = atomicMax(tc + slot, v);
+            // counts only grow, so exactly one update takes a K-mer from <= limit to > limit
+            if ((pal ? 2ull * old : old) <= limit && (pal ? 2ull * v : v) > limit) added++;
+        }
+    }
+    if (added) atomicAdd((unsigned long long *)(stats + 4), (unsigned long long)added);
+    if (full) atomicOr((unsigned long long *)(stats + 2), 1ull);
+}
+
+// one step: the count table of the reads at K, raised by the previous contigs (prev_nc of them, Kp-mers, on the device
+// in ctx->text_buf and prev), then clean_unitigs.  keep: where this step's contigs stay for the next one.
+template <typename Key>
+static int multik_step_w(euler_ctx *ctx, const void *d_buf, u64 B, const u32 *d_bits, u32 K, u32 Kp, u32 limit,
+                         const euler_clean_params &cp, const UnitigsKept &prev, u64 prev_nc, u64 prev_bytes, UnitigsKept *keep,
+                         char **d_out, u64 *out_bytes, u64 *ncontigs, u64 *h_sums, u64 sums_cap, euler_clean_stats *st,
+                         u64 *nodes_added)
+{
+    const u64 cap = euler_hash_capacity(B + prev_bytes);
+    DevTmp<u64> d_stats(ctx, 8);
+    DevTmp<u32> tc(ctx, cap);
+    DevTmp<Key> tk(ctx, cap);
+    TMP_CHECK(ctx, d_stats); TMP_CHECK(ctx, tk); TMP_CHECK(ctx, tc);
+    CUDA_TRY(ctx, cudaMemsetAsync(d_stats, 0, 8 * sizeof(u64), ctx->stream));
+    EULER_TRY(key_table_clear(ctx, tk.get(), tc, cap));
+    if (B) EULER_TRY(key_count(ctx, d_buf, B, d_bits, K, tk.get(), tc, cap, d_stats));
+    if (prev_nc) {
+        multik_contig_kmers_kernel<Key><<<grid_for((prev_bytes + MK_RUN - 1) / MK_RUN, UB), UB, 0, ctx->stream>>>(
+            (const char *)ctx->text_buf.p, prev.off.ptr(), prev.sums.ptr(), prev_nc, prev.n_starts, Kp, K, limit, tk.get(), tc.get(),
+            cap, d_stats.get());
+        CUDA_TRY(ctx, cudaGetLastError());
+    }
+    u64 h[5];
+    EULER_TRY(read_u64s(ctx, d_stats, h, 5));
+    if (h[2]) return euler_fail(ctx, EULER_ERR_OVERFLOW, "count table overflow");
+    *nodes_added = h[4];
+    return unitigs_from_table(ctx, tk.get(), tc.get(), cap, K, limit, &cp, d_out, out_bytes, ncontigs, h_sums, sums_cap, st, keep);
+}
+
+int unitigs_multik(euler_ctx *ctx, const void *d_buf, const u64 *d_off, u64 nreads, u64 B, const u32 *ks, u32 nk, u32 limit,
+                   const euler_clean_params *params, char **d_out, u64 *out_bytes, u64 *ncontigs, u64 *h_sums, u64 sums_cap,
+                   euler_multik_step *steps)
+{
+    *d_out = nullptr; *out_bytes = 0; *ncontigs = 0;
+    DevTmp<u32> d_bits(ctx, B / 32 + 2);
+    TMP_CHECK(ctx, d_bits);
+    if (B) EULER_TRY(enc_mark_starts(ctx, d_off, nreads, B, d_bits));
+    UnitigsKept kept;   // offsets and sums of the previous step; its text is ctx->text_buf until this step spells
+    u64 nc = 0, bytes = 0;
+    int rc = EULER_OK;
+    for (u32 i = 0; i < nk && rc == EULER_OK; i++) {
+        const bool last = i + 1 == nk;
+        const u32 K = ks[i], Kp = i ? ks[i - 1] : 0;
+        char *text = nullptr;
+        u64 nb = 0, n = 0, added = 0;
+        euler_clean_stats st{};
+        if (K <= 32)
+            rc = multik_step_w<u64>(ctx, d_buf, B, d_bits, K, Kp, limit, params[i], kept, nc, bytes, last ? nullptr : &kept, &text,
+                                    &nb, &n, last ? h_sums : nullptr, sums_cap, &st, &added);
+        else
+            rc = multik_step_w<K128>(ctx, d_buf, B, d_bits, K, Kp, limit, params[i], kept, nc, bytes, last ? nullptr : &kept, &text,
+                                     &nb, &n, last ? h_sums : nullptr, sums_cap, &st, &added);
+        nc = n; bytes = nb;
+        if (steps) steps[i] = euler_multik_step{K, n, nb - n, added, st};
+        if (last) { *d_out = text; *out_bytes = nb; *ncontigs = n; }
+    }
+    kept.free();
+    return rc;
 }
