@@ -20,9 +20,24 @@ typedef unsigned int u32;
 // ---------------------------------------------------------------------------------------
 // context
 // ---------------------------------------------------------------------------------------
+// Owns its device memory: freed on destruction, so the device it was allocated on must be current then.  Move-only.
 struct DevBuf {
     void *p = nullptr;
     size_t cap = 0;
+    DevBuf() = default;
+    DevBuf(const DevBuf &) = delete;
+    DevBuf &operator=(const DevBuf &) = delete;
+    DevBuf(DevBuf &&o) noexcept : p(o.p), cap(o.cap) { o.p = nullptr; o.cap = 0; }
+    DevBuf &operator=(DevBuf &&o) noexcept
+    {
+        if (this != &o) {
+            if (p) cudaFree(p);
+            p = o.p; cap = o.cap;
+            o.p = nullptr; o.cap = 0;
+        }
+        return *this;
+    }
+    ~DevBuf() { if (p) cudaFree(p); }
 };
 
 struct Pipeline;
@@ -65,14 +80,12 @@ int euler_fail(euler_ctx *ctx, int code, const char *fmt, ...);
 
 // grow-only device buffer
 int dev_reserve(euler_ctx *ctx, DevBuf &b, size_t bytes);
-void dev_free(DevBuf &b);
 
 template <typename T>
 struct DevArr {
     DevBuf b;
     T *ptr() const { return (T *)b.p; }
     int reserve(euler_ctx *ctx, size_t n) { return dev_reserve(ctx, b, (n ? n : 1) * sizeof(T)); }
-    void free() { dev_free(b); }
 };
 
 static inline unsigned grid_for(u64 n, unsigned block)

@@ -41,13 +41,6 @@ int dev_reserve(euler_ctx *ctx, DevBuf &b, size_t bytes)
     return EULER_OK;
 }
 
-void dev_free(DevBuf &b)
-{
-    if (b.p) cudaFree(b.p);
-    b.p = nullptr;
-    b.cap = 0;
-}
-
 int scan_state_reserve(euler_ctx *ctx, u64 ntiles, ScanState **state, u64 **counter)
 {
     EULER_TRY(dev_reserve(ctx, ctx->scan_state, (ntiles + 1) * sizeof(ScanState)));
@@ -102,9 +95,6 @@ void euler_ctx_destroy(euler_ctx *ctx)
     cudaSetDevice(ctx->device);
     if (ctx->stream) cudaStreamSynchronize(ctx->stream);
     if (ctx->pipe) pipeline_destroy(ctx->pipe);
-    dev_free(ctx->scan_state);
-    dev_free(ctx->cg_buf);
-    dev_free(ctx->text_buf);
     for (int i = 0; i < 8; i++) if (ctx->ev[i]) cudaEventDestroy(ctx->ev[i]);
     if (ctx->h_pinned) cudaFreeHost(ctx->h_pinned);
     if (ctx->own_stream && ctx->stream) cudaStreamDestroy(ctx->stream);

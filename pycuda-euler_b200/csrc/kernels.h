@@ -132,7 +132,6 @@ int unitigs_multik(euler_ctx *ctx, const void *d_buf, const u64 *d_off, u64 nrea
 struct UnitigsKept {
     DevArr<u64> off, sums;
     u32 n_starts = 0;
-    void free() { off.free(); sums.free(); }
 };
 
 // ---- clean.cu (key-independent): n nodes with forward extensions nbr[4 n], twin_id[n], both-strand counts cnt[n]

@@ -122,21 +122,12 @@ struct Pipeline {
     euler_stats st = {};
 };
 
+// the device buffers free themselves; only the IPC-exported allocations are raw
 void pipeline_destroy(Pipeline *p)
 {
     if (!p) return;
-    p->in_buf.free(); p->in_off.free(); p->start_bits.free();
-    dev_free(p->lt.b); p->lt_packed.free(); p->side_keys.free(); p->side_cnt.free(); p->lt_base.free(); p->lt_eoff.free(); p->lt_own.free();
-    p->vt_keys.free(); p->vt_id0.free(); p->vt_id1.free(); p->stats.free();
-    p->lkeys.free(); p->vkeys.free(); p->lvals.free(); p->loffs.free(); p->ev1.free(); p->ev2.free();
-    p->lcount.free(); p->ecount.free(); p->lstart.free(); p->estart.free(); p->ev.free(); p->ee.free();
     if (p->recv_buf) cudaFree(p->recv_buf);
-    p->lev.free(); p->ent.free(); p->sort_k.free(); p->sort_v.free(); p->sort_hist.free();
-    p->blk_keys.free(); p->blk_cur.free(); p->deg.free(); p->vt_bbase.free(); p->lt_merged.free(); p->tbl_keys.free(); p->tbl_cnt.free();
-    p->wlt_keys.free(); p->wvt_keys.free(); p->wlt_cnt.free(); p->lkeys_hi.free(); p->vkeys_hi.free(); p->tf.free();
     for (int i = 0; i < 2; i++) if (p->bk_area[i]) cudaFree(p->bk_area[i]);
-    dev_free(p->bk_records); dev_free(p->bk_state); p->bk_cursors.free(); p->bk_bvals.free(); p->bk_perm.free(); p->bk_newid.free();
-    p->bk_tmp32a.free(); p->bk_tmp32b.free(); p->bk_tmp32c.free(); p->bk_rows_a.free(); p->bk_rows_b.free(); p->bk_bkeys.free(); p->bk_dst.free(); p->bk_scursors.free();
     delete p;
 }
 
@@ -204,21 +195,114 @@ static bool use_merged_table()
 }
 static u64 cap_for(u64 n) { return round_up((u64)((double)(n < 64 ? 64 : n) / table_load()) + 1, 1024); }
 
+// ---- stages shared by the graph builds --------------------------------------------------------------------------------
+// start of a build: the previous graph, its contig text and its stats are gone
+static void begin_run(Pipeline *P, u32 l, u32 flags, bool wide, u64 nreads, u64 n_bases)
+{
+    P->l = l; P->flags = flags; P->wide = wide;
+    P->have_graph = false; P->expanded = false; P->text_valid = false;
+    memset(&P->st, 0, sizeof(P->st));
+    P->st.n_reads = nreads; P->st.n_bases = n_bases;
+}
+
+// expected distinct canonical l-mers / k-mers of B bases of reads: the hint, else what the last run of this size
+// counted, else B
+static void estimate_from_reads(const Pipeline *P, u64 B, u64 hint, u64 &est_l, u64 &est_v)
+{
+    if (hint) { est_l = hint; est_v = hint + hint / 16; }
+    else if (P->learned_bases == B && P->learned_lc) { est_l = P->learned_lc + P->learned_lc / 32; est_v = P->learned_vc + P->learned_vc / 32; }
+    else { est_l = B ? B : 1; est_v = est_l; }
+}
+
+// table capacities for nkeys received keys: from the hint, else from what the last build of as many keys counted, else
+// one l-mer per key
+static void caps_from_keys(const Pipeline *P, u64 nkeys, u64 hint, u64 &lt_cap, u64 &vt_cap)
+{
+    const bool learned = !hint && P->learned_bases == nkeys && P->learned_lc;
+    const u64 est = hint ? hint : (learned ? P->learned_lc : (nkeys ? nkeys : 1));
+    lt_cap = cap_for(est); vt_cap = cap_for(learned ? P->learned_vc : est);
+}
+
+// the graph artefacts for ucap both-strand l-mers and vcap vertices; two-word keys add the high words and tf
+static int reserve_graph(euler_ctx *ctx, Pipeline *P, u64 ucap, u64 vcap, bool wide)
+{
+    EULER_TRY(P->lkeys.reserve(ctx, ucap)); EULER_TRY(P->lvals.reserve(ctx, ucap)); EULER_TRY(P->loffs.reserve(ctx, ucap));
+    EULER_TRY(P->ev1.reserve(ctx, ucap)); EULER_TRY(P->ev2.reserve(ctx, ucap));
+    EULER_TRY(P->vkeys.reserve(ctx, vcap));
+    EULER_TRY(P->lcount.reserve(ctx, 4 * vcap + 4)); EULER_TRY(P->ecount.reserve(ctx, 4 * vcap + 4));
+    EULER_TRY(P->lstart.reserve(ctx, 4 * vcap + 4)); EULER_TRY(P->estart.reserve(ctx, 4 * vcap + 4));
+    EULER_TRY(P->ev.reserve(ctx, vcap));
+    if (wide) {
+        EULER_TRY(P->lkeys_hi.reserve(ctx, ucap)); EULER_TRY(P->vkeys_hi.reserve(ctx, vcap));
+        EULER_TRY(P->tf.reserve(ctx, ucap + 16));
+    }
+    return EULER_OK;
+}
+
+// zero what the edge kernels count degrees into: the paired regions (common.cuh, DegOut) or lcount / ecount
+static int clear_degrees(euler_ctx *ctx, Pipeline *P, u64 V, bool paired)
+{
+    cudaStream_t s = ctx->stream;
+    if (paired) {
+        EULER_TRY(P->deg.reserve(ctx, 8 * V + 8));
+        CUDA_TRY(ctx, cudaMemsetAsync(P->deg.ptr(), 0, (8 * V + 8) * sizeof(u32), s));
+    } else {
+        CUDA_TRY(ctx, cudaMemsetAsync(P->lcount.ptr(), 0, (4 * V + 4) * sizeof(u32), s));
+        CUDA_TRY(ctx, cudaMemsetAsync(P->ecount.ptr(), 0, (4 * V + 4) * sizeof(u32), s));
+    }
+    return EULER_OK;
+}
+
+// EULER_RUN_EXPAND_EDGES: the per-edge arrays of the graph just built (two-word keys give their first bases in tf)
+static int expand_edges(euler_ctx *ctx, Pipeline *P, u32 &launches)
+{
+    if (!(P->flags & EULER_RUN_EXPAND_EDGES)) return EULER_OK;
+    const u64 E = P->E;
+    launches += 1;
+    EULER_TRY(P->ee.reserve(ctx, E)); EULER_TRY(P->lev.reserve(ctx, E)); EULER_TRY(P->ent.reserve(ctx, E));
+    EULER_TRY(graph_setup_edges(ctx, P->wide ? nullptr : P->lkeys.ptr(), P->lvals.ptr(), P->loffs.ptr(), P->U_l, P->l, P->ev1.ptr(),
+                                P->ev2.ptr(), P->lstart.ptr(), P->estart.ptr(), (u32)E, P->ee.ptr(), P->lev.ptr(), P->ent.ptr(),
+                                P->wide ? P->tf.ptr() : nullptr));
+    P->expanded = true;
+    return EULER_OK;
+}
+
+// Tail of every build: wait for the graph and make it the current one, add its sizes, retries, launches and phase times
+// to P->st (the driver has set its own fields) and copy that out.  ms_graph runs from ev[graph_from] to ev[graph_to].
+// A build that counted (graph_from = 1) times the count ev[0] -> ev[1], the count kernel ev[4] -> ev[1] and ms_total
+// over both; otherwise ms_total is the graph alone.  The per-bucket builds (path 1) time bkt_build ev[5] -> ev[2].
+static int finish_run(euler_ctx *ctx, Pipeline *P, u64 lt_cap, u64 vt_cap, u32 retries, u32 launches, int graph_from, int graph_to,
+                      euler_stats *stats)
+{
+    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+    P->have_graph = true;
+    euler_stats &st = P->st;
+    st.distinct_lmers = P->U_l; st.distinct_kmers = P->V; st.edge_count = P->E;
+    st.lmer_table_capacity = lt_cap; st.kmer_table_capacity = vt_cap; st.retries = retries; st.kernel_launches = launches;
+    cudaEventElapsedTime(&st.ms_graph, ctx->ev[graph_from], ctx->ev[graph_to]);
+    if (graph_from == 1) {
+        cudaEventElapsedTime(&st.ms_count, ctx->ev[0], ctx->ev[1]);
+        cudaEventElapsedTime(&st.ms_total, ctx->ev[0], ctx->ev[graph_to]);
+        cudaEventElapsedTime(&st.ms_count_kernel, ctx->ev[4], ctx->ev[1]);
+    } else {
+        st.ms_total = st.ms_graph;
+    }
+    if (st.path == 1) cudaEventElapsedTime(&st.ms_build_kernel, ctx->ev[5], ctx->ev[2]);
+    if (stats) *stats = st;
+    return EULER_OK;
+}
+
 // l in 33..64: the same stages over two-word keys (wide.cu).  Correctness-first: one thread per read,
 // explicit both-strand l-mer arrays, ids in slot order or ascending (hi, lo) order.
 static int pipeline_run_wide(euler_ctx *ctx, Pipeline *P, u32 l, u32 flags, u64 distinct_hint, euler_stats *stats)
 {
-    P->l = l; P->flags = flags; P->have_graph = false; P->expanded = false; P->text_valid = false; P->wide = true;
     const u32 k = l - 1;
     const u64 B = P->n_bases;
     cudaStream_t s = ctx->stream;
-    memset(&P->st, 0, sizeof(P->st));
-    P->st.n_reads = P->nreads; P->st.n_bases = B;
+    begin_run(P, l, flags, true, P->nreads, B);
     EULER_TRY(P->stats.reserve(ctx, 16));
     u64 est_l, est_v;
-    if (distinct_hint) { est_l = distinct_hint; est_v = distinct_hint + distinct_hint / 16; }
-    else if (P->learned_bases == B && P->learned_lc) { est_l = P->learned_lc + P->learned_lc / 32; est_v = P->learned_vc + P->learned_vc / 32; }
-    else { est_l = B ? B : 1; est_v = est_l; }
+    estimate_from_reads(P, B, distinct_hint, est_l, est_v);
     u64 lt_cap = cap_for(est_l), vt_cap = cap_for(est_v);
     u64 h[8] = {0};
     u32 retries = 0, launches = 0;
@@ -263,15 +347,8 @@ static int pipeline_run_wide(euler_ctx *ctx, Pipeline *P, u32 l, u32 flags, u64 
     P->U_l = U_l; P->V = V; P->E = E;
     if (V >= 0x3fffffffull || N_l >= 0x7fffffffull)
         return euler_fail(ctx, EULER_ERR_RANGE, "graph exceeds u32 ids (U_l=%llu V=%llu E=%llu)", U_l, V, E);
-    EULER_TRY(P->lkeys.reserve(ctx, U_l)); EULER_TRY(P->lkeys_hi.reserve(ctx, U_l)); EULER_TRY(P->lvals.reserve(ctx, U_l));
-    EULER_TRY(P->loffs.reserve(ctx, U_l)); EULER_TRY(P->ev1.reserve(ctx, U_l)); EULER_TRY(P->ev2.reserve(ctx, U_l));
-    EULER_TRY(P->tf.reserve(ctx, U_l + 16));
-    EULER_TRY(P->vkeys.reserve(ctx, V)); EULER_TRY(P->vkeys_hi.reserve(ctx, V));
-    EULER_TRY(P->lcount.reserve(ctx, 4 * V + 4)); EULER_TRY(P->ecount.reserve(ctx, 4 * V + 4));
-    EULER_TRY(P->lstart.reserve(ctx, 4 * V + 4)); EULER_TRY(P->estart.reserve(ctx, 4 * V + 4));
-    EULER_TRY(P->ev.reserve(ctx, V));
-    CUDA_TRY(ctx, cudaMemsetAsync(P->lcount.ptr(), 0, (4 * V + 4) * sizeof(u32), s));
-    CUDA_TRY(ctx, cudaMemsetAsync(P->ecount.ptr(), 0, (4 * V + 4) * sizeof(u32), s));
+    EULER_TRY(reserve_graph(ctx, P, U_l, V, true));
+    EULER_TRY(clear_degrees(ctx, P, V, false));
     EULER_TRY(wide_compact_vertices(ctx, P->wvt_keys.ptr(), P->vt_id0.ptr(), vt_cap, k, P->vkeys.ptr(), P->vkeys_hi.ptr()));
     EULER_TRY(wide_compact_lmers(ctx, P->wlt_keys.ptr(), P->wlt_cnt.ptr(), P->lt_base.ptr(), lt_cap, l, P->lkeys.ptr(),
                                  P->lkeys_hi.ptr(), P->lvals.ptr()));
@@ -292,28 +369,11 @@ static int pipeline_run_wide(euler_ctx *ctx, Pipeline *P, u32 l, u32 flags, u64 
                                    P->ev.ptr()));
     launches += 5;
     CUDA_TRY(ctx, cudaEventRecord(ctx->ev[2], s));
-    if (flags & EULER_RUN_EXPAND_EDGES) {
-        launches += 1;
-        EULER_TRY(P->ee.reserve(ctx, E)); EULER_TRY(P->lev.reserve(ctx, E)); EULER_TRY(P->ent.reserve(ctx, E));
-        EULER_TRY(graph_setup_edges(ctx, nullptr, P->lvals.ptr(), P->loffs.ptr(), U_l, l, P->ev1.ptr(), P->ev2.ptr(), P->lstart.ptr(),
-                                    P->estart.ptr(), (u32)E, P->ee.ptr(), P->lev.ptr(), P->ent.ptr(), P->tf.ptr()));
-        P->expanded = true;
-    }
-    CUDA_TRY(ctx, cudaEventRecord(ctx->ev[3], s));
-    CUDA_TRY(ctx, cudaStreamSynchronize(s));
-    P->have_graph = true;
+    EULER_TRY(expand_edges(ctx, P, launches));
     P->learned_bases = B;
     P->learned_lc = (U_l + 1) / 2 + 16; P->learned_vc = (V + 1) / 2 + 16;
-    euler_stats &st = P->st;
-    st.n_kmer_windows = N_k; st.n_lmer_windows = N_l; st.distinct_lmers = U_l; st.distinct_kmers = V; st.edge_count = E;
-    st.lmer_table_capacity = lt_cap; st.kmer_table_capacity = vt_cap; st.retries = retries;
-    cudaEventElapsedTime(&st.ms_count, ctx->ev[0], ctx->ev[1]);
-    cudaEventElapsedTime(&st.ms_graph, ctx->ev[1], ctx->ev[2]);
-    cudaEventElapsedTime(&st.ms_total, ctx->ev[0], ctx->ev[2]);
-    cudaEventElapsedTime(&st.ms_count_kernel, ctx->ev[4], ctx->ev[1]);
-    st.kernel_launches = launches;
-    if (stats) *stats = st;
-    return EULER_OK;
+    P->st.n_kmer_windows = N_k; P->st.n_lmer_windows = N_l;
+    return finish_run(ctx, P, lt_cap, vt_cap, retries, launches, 1, 2, stats);
 }
 
 
@@ -338,6 +398,36 @@ static u64 pow2_at_least(u64 x)
 }
 #define EULER_FALLBACK 1   // internal: take the global-table path instead
 #define BKT_MAX_DISTINCT 50000000ull   // distinct canonical l-mers up to which the bucketed path is taken by default
+
+// One round of the per-bucket build over nb regions of rcap records, shared-memory tables of cap slots, ucap / vcap
+// artefact entries and a boundary table of bcap: reserve all of it, let fill_regions() put the records in place (or
+// only reset the stats words when they already are), build, and read the 8 stats words back into h.  The repair after
+// a round is the driver's own.
+template <typename Fill>
+static int bkt_round(euler_ctx *ctx, Pipeline *P, u32 l, u32 nb, u32 rcap, u32 cap, u64 ucap, u64 vcap, u64 bcap, u32 &launches,
+                     u64 *h, Fill fill_regions)
+{
+    EULER_TRY(dev_reserve(ctx, P->bk_records, (size_t)nb * rcap * 16 + 16));
+    EULER_TRY(P->bk_cursors.reserve(ctx, nb));
+    EULER_TRY(dev_reserve(ctx, P->bk_state, bkt_state_bytes(nb)));
+    EULER_TRY(P->bk_bkeys.reserve(ctx, bcap)); EULER_TRY(P->bk_bvals.reserve(ctx, 2 * bcap));
+    EULER_TRY(reserve_graph(ctx, P, ucap, vcap, false));
+    EULER_TRY(fill_regions());
+    BktBuild bb;
+    bb.records = P->bk_records.p; bb.counts = P->bk_cursors.ptr(); bb.nb = nb; bb.nranks = 1; bb.rcap = rcap; bb.l = l; bb.cap = cap;
+    bb.lkeys = P->lkeys.ptr(); bb.lvals = P->lvals.ptr(); bb.loffs = P->loffs.ptr(); bb.ev1 = P->ev1.ptr(); bb.ev2 = P->ev2.ptr(); bb.ucap = ucap;
+    bb.vkeys = P->vkeys.ptr(); bb.lcount = P->lcount.ptr(); bb.ecount = P->ecount.ptr(); bb.lstart = P->lstart.ptr();
+    bb.estart = P->estart.ptr(); bb.ev = P->ev.ptr(); bb.vcap = vcap;
+    bb.state = P->bk_state.p; bb.bkeys = P->bk_bkeys.ptr(); bb.bvals = P->bk_bvals.ptr(); bb.bcap = bcap; bb.stats = P->stats.ptr();
+    CUDA_TRY(ctx, cudaEventRecord(ctx->ev[5], ctx->stream));
+    EULER_TRY(bkt_build(ctx, bb));
+    CUDA_TRY(ctx, cudaEventRecord(ctx->ev[2], ctx->stream));
+    launches += 4;   // build, second pass, boundary publish, fix-up
+    EULER_TRY(read_u64s(ctx, P->stats.ptr(), h, 8));   // the only host round trip of a steady-state step
+    if (h[2] & BKT_FLAG_INTERNAL)
+        return euler_fail(ctx, EULER_ERR_STATE, "internal: bucketed build consistency check failed (flags %llx)", h[2]);
+    return EULER_OK;
+}
 
 static int pipeline_run_bucketed(euler_ctx *ctx, Pipeline *P, u32 l, u32 flags, u64 distinct_hint, euler_stats *stats)
 {
@@ -385,23 +475,17 @@ static int pipeline_run_bucketed(euler_ctx *ctx, Pipeline *P, u32 l, u32 flags, 
     u64 h[8] = {0};
     u32 retries = 0, launches = 0;
     bool need_part = true;
+    EULER_TRY(P->bk_dst.reserve(ctx, 16));
     CUDA_TRY(ctx, cudaEventRecord(ctx->ev[0], s));
     EULER_TRY(enc_mark_starts(ctx, P->d_off, P->nreads, B, P->start_bits.ptr()));
     launches++;
     while (true) {
         if ((u64)nb * rcap * 16 > (48ull << 30)) return EULER_FALLBACK;
-        EULER_TRY(dev_reserve(ctx, P->bk_records, (size_t)nb * rcap * 16 + 16));
-        EULER_TRY(P->bk_cursors.reserve(ctx, nb));
-        EULER_TRY(dev_reserve(ctx, P->bk_state, bkt_state_bytes(nb)));
-        EULER_TRY(P->bk_bkeys.reserve(ctx, bcap)); EULER_TRY(P->bk_bvals.reserve(ctx, 2 * bcap));
-        EULER_TRY(P->bk_dst.reserve(ctx, 16));
-        EULER_TRY(P->lkeys.reserve(ctx, ucap)); EULER_TRY(P->lvals.reserve(ctx, ucap)); EULER_TRY(P->loffs.reserve(ctx, ucap));
-        EULER_TRY(P->ev1.reserve(ctx, ucap)); EULER_TRY(P->ev2.reserve(ctx, ucap));
-        EULER_TRY(P->vkeys.reserve(ctx, vcap));
-        EULER_TRY(P->lcount.reserve(ctx, 4 * vcap + 4)); EULER_TRY(P->ecount.reserve(ctx, 4 * vcap + 4));
-        EULER_TRY(P->lstart.reserve(ctx, 4 * vcap + 4)); EULER_TRY(P->estart.reserve(ctx, 4 * vcap + 4));
-        EULER_TRY(P->ev.reserve(ctx, vcap));
-        if (need_part) {
+        EULER_TRY(bkt_round(ctx, P, l, nb, rcap, cap, ucap, vcap, bcap, launches, h, [&]() -> int {
+            if (!need_part) {
+                CUDA_TRY(ctx, cudaMemsetAsync(P->stats.ptr() + 2, 0, 6 * sizeof(u64), s));   // flags, totals, max region
+                return EULER_OK;
+            }
             uint4 *self = (uint4 *)P->bk_records.p;
             CUDA_TRY(ctx, cudaMemcpyAsync(P->bk_dst.ptr(), &self, sizeof(self), cudaMemcpyHostToDevice, s));
             CUDA_TRY(ctx, cudaMemsetAsync(P->stats.ptr(), 0, 32 * sizeof(u64), s));
@@ -412,21 +496,8 @@ static int pipeline_run_bucketed(euler_ctx *ctx, Pipeline *P, u32 l, u32 flags, 
             CUDA_TRY(ctx, cudaEventRecord(ctx->ev[1], s));
             launches++;
             need_part = false;
-        } else {
-            CUDA_TRY(ctx, cudaMemsetAsync(P->stats.ptr() + 2, 0, 6 * sizeof(u64), s));   // flags, totals, max region
-        }
-        BktBuild bb;
-        bb.records = P->bk_records.p; bb.counts = P->bk_cursors.ptr(); bb.nb = nb; bb.nranks = 1; bb.rcap = rcap; bb.l = l;
-        bb.cap = cap;
-        bb.lkeys = P->lkeys.ptr(); bb.lvals = P->lvals.ptr(); bb.loffs = P->loffs.ptr(); bb.ev1 = P->ev1.ptr(); bb.ev2 = P->ev2.ptr(); bb.ucap = ucap;
-        bb.vkeys = P->vkeys.ptr(); bb.lcount = P->lcount.ptr(); bb.ecount = P->ecount.ptr(); bb.lstart = P->lstart.ptr();
-        bb.estart = P->estart.ptr(); bb.ev = P->ev.ptr(); bb.vcap = vcap;
-        bb.state = P->bk_state.p; bb.bkeys = P->bk_bkeys.ptr(); bb.bvals = P->bk_bvals.ptr(); bb.bcap = bcap; bb.stats = P->stats.ptr();
-        CUDA_TRY(ctx, cudaEventRecord(ctx->ev[5], s));
-        EULER_TRY(bkt_build(ctx, bb));
-        CUDA_TRY(ctx, cudaEventRecord(ctx->ev[2], s));
-        launches += 4;   // build, second pass, boundary publish, fix-up
-        EULER_TRY(read_u64s(ctx, P->stats.ptr(), h, 8));   // the only host round trip of a steady-state step
+            return EULER_OK;
+        }));
         if (getenv("EULER_B200_BKT_TIMING")) {   // library built with -DBKT_TIMING: clock cycles per build phase, summed over the blocks
             u64 t[8];
             EULER_TRY(read_u64s(ctx, P->stats.ptr() + 16, t, 8));
@@ -434,7 +505,6 @@ static int pipeline_run_bucketed(euler_ctx *ctx, Pipeline *P, u32 l, u32 flags, 
                     nb, t[0] / 1e6, t[1] / 1e6, t[2] / 1e6, t[3] / 1e6, t[4] / 1e6, t[5] / 1e6, t[6] / 1e6);
         }
         const u64 fl = h[2];
-        if (fl & BKT_FLAG_INTERNAL) return euler_fail(ctx, EULER_ERR_STATE, "internal: bucketed build consistency check failed (flags %llx)", fl);
         if (!(fl & (BKT_FLAG_REGION | BKT_FLAG_TABLE | BKT_FLAG_OUTPUT | BKT_FLAG_BOUNDARY))) break;
         if (++retries > 8) return EULER_FALLBACK;
         if (fl & BKT_FLAG_REGION) {   // stats[6] = the largest region
@@ -490,16 +560,7 @@ static int pipeline_run_bucketed(euler_ctx *ctx, Pipeline *P, u32 l, u32 flags, 
         launches += 3 * ((2 * l + 7) / 8) + 3 * ((2 * k + 7) / 8) + 8;
     }
     CUDA_TRY(ctx, cudaEventRecord(ctx->ev[6], s));
-    if (flags & EULER_RUN_EXPAND_EDGES) {
-        launches += 1;
-        EULER_TRY(P->ee.reserve(ctx, E)); EULER_TRY(P->lev.reserve(ctx, E)); EULER_TRY(P->ent.reserve(ctx, E));
-        EULER_TRY(graph_setup_edges(ctx, P->lkeys.ptr(), P->lvals.ptr(), P->loffs.ptr(), U_l, l, P->ev1.ptr(), P->ev2.ptr(),
-                                    P->lstart.ptr(), P->estart.ptr(), (u32)E, P->ee.ptr(), P->lev.ptr(), P->ent.ptr()));
-        P->expanded = true;
-    }
-    CUDA_TRY(ctx, cudaEventRecord(ctx->ev[3], s));
-    CUDA_TRY(ctx, cudaStreamSynchronize(s));
-    P->have_graph = true;
+    EULER_TRY(expand_edges(ctx, P, launches));
     P->learned_bases = B;
     P->learned_lc = (U_l + 1) / 2 + 16; P->learned_vc = (V + 1) / 2 + 16;
     P->bk_learned_bases = B; P->bk_learned_l = l; P->bk_learned_nb = nb; P->bk_learned_u = U_l; P->bk_learned_v = V;
@@ -510,47 +571,30 @@ static int pipeline_run_bucketed(euler_ctx *ctx, Pipeline *P, u32 l, u32 flags, 
         if (!env_u32("EULER_B200_BKT_NB", 0) && (want * 2 < nb || want > (u64)nb * 2)) { P->bk_learned_nb = (u32)want; P->bk_learned_rcap = 0; }
     }
     euler_stats &st = P->st;
-    st.n_kmer_windows = N_k; st.n_lmer_windows = N_l; st.distinct_lmers = U_l; st.distinct_kmers = V; st.edge_count = E;
-    st.lmer_table_capacity = (u64)nb * cap; st.kmer_table_capacity = (u64)nb * cap; st.retries = retries;
-    cudaEventElapsedTime(&st.ms_count, ctx->ev[0], ctx->ev[1]);
-    cudaEventElapsedTime(&st.ms_graph, ctx->ev[1], ctx->ev[6]);
-    cudaEventElapsedTime(&st.ms_total, ctx->ev[0], ctx->ev[6]);
-    cudaEventElapsedTime(&st.ms_count_kernel, ctx->ev[4], ctx->ev[1]);
-    cudaEventElapsedTime(&st.ms_build_kernel, ctx->ev[5], ctx->ev[2]);
-    st.kernel_launches = launches;
+    st.n_kmer_windows = N_k; st.n_lmer_windows = N_l;
     st.path = 1; st.n_buckets = nb; st.bucket_records = h[6]; st.redo_buckets = (u32)h[7];
-    if (stats) *stats = st;
-    return EULER_OK;
+    return finish_run(ctx, P, (u64)nb * cap, (u64)nb * cap, retries, launches, 1, 6, stats);
 }
 
 static int pipeline_run(euler_ctx *ctx, Pipeline *P, u32 l, u32 flags, u64 distinct_hint, euler_stats *stats)
 {
     if (l < 2 || l > 64) return euler_fail(ctx, EULER_ERR_ARG, "l-mer length %u out of range [2,64]", l);
     if (l > 32) return pipeline_run_wide(ctx, P, l, flags, distinct_hint, stats);
-    P->wide = false;
-    P->l = l; P->flags = flags; P->have_graph = false; P->expanded = false; P->text_valid = false;
-    memset(&P->st, 0, sizeof(P->st));
-    P->st.n_reads = P->nreads; P->st.n_bases = P->n_bases;
-    if (!P->from_table && use_bucketed()) {
-        const int rc = pipeline_run_bucketed(ctx, P, l, flags, distinct_hint, stats);
-        if (rc != EULER_FALLBACK) return rc;
-        P->have_graph = false; P->expanded = false;
-    }
     const u32 k = l - 1;
     const u64 B = P->n_bases;
     cudaStream_t s = ctx->stream;
-    memset(&P->st, 0, sizeof(P->st));
-    P->st.n_reads = P->nreads; P->st.n_bases = B;
+    begin_run(P, l, flags, false, P->nreads, B);
+    if (!P->from_table && use_bucketed()) {   // it changes nothing of P->st or the graph state before it falls back
+        const int rc = pipeline_run_bucketed(ctx, P, l, flags, distinct_hint, stats);
+        if (rc != EULER_FALLBACK) return rc;
+    }
 
     EULER_TRY(P->stats.reserve(ctx, 16));
     EULER_TRY(P->start_bits.reserve(ctx, B / 32 + 2));
     P->dist_bits_bases = ~0ull;   // the bitmap no longer belongs to an euler_dist_count call
 
-    // expected distinct canonical l-mers / k-mers
     u64 est_l, est_v;
-    if (distinct_hint) { est_l = distinct_hint; est_v = distinct_hint + distinct_hint / 16; }
-    else if (P->learned_bases == B && P->learned_lc) { est_l = P->learned_lc + P->learned_lc / 32; est_v = P->learned_vc + P->learned_vc / 32; }
-    else { est_l = B ? B : 1; est_v = est_l; }
+    estimate_from_reads(P, B, distinct_hint, est_l, est_v);
     const bool from_table = P->from_table;
     if (from_table && !distinct_hint) { est_l = P->tbl_n ? P->tbl_n : 1; est_v = 2 * est_l; }
     u64 lt_cap = cap_for(est_l), vt_cap = cap_for(est_v);
@@ -646,21 +690,9 @@ static int pipeline_run(euler_ctx *ctx, Pipeline *P, u32 l, u32 flags, u64 disti
         return euler_fail(ctx, EULER_ERR_RANGE, "graph exceeds u32 ids (U_l=%llu V=%llu E=%llu)", U_l, V, E);
     if ((h[3] >> 32) != E) return euler_fail(ctx, EULER_ERR_STATE, "internal: edge total %llu != 2 N_l %llu", h[3] >> 32, E);
 
-    EULER_TRY(P->lkeys.reserve(ctx, U_l)); EULER_TRY(P->lvals.reserve(ctx, U_l)); EULER_TRY(P->loffs.reserve(ctx, U_l));
-    EULER_TRY(P->ev1.reserve(ctx, U_l)); EULER_TRY(P->ev2.reserve(ctx, U_l));
-    EULER_TRY(P->vkeys.reserve(ctx, V));
-    EULER_TRY(P->lcount.reserve(ctx, 4 * V + 4)); EULER_TRY(P->ecount.reserve(ctx, 4 * V + 4));
-    EULER_TRY(P->lstart.reserve(ctx, 4 * V + 4)); EULER_TRY(P->estart.reserve(ctx, 4 * V + 4));
-    EULER_TRY(P->ev.reserve(ctx, V));
-
+    EULER_TRY(reserve_graph(ctx, P, U_l, V, false));
     const bool paired = !(flags & EULER_RUN_CANONICAL_IDS);   // slot-order ids: the strands of a vertex have adjacent ids
-    if (paired) {
-        EULER_TRY(P->deg.reserve(ctx, 8 * V + 8));
-        CUDA_TRY(ctx, cudaMemsetAsync(P->deg.ptr(), 0, (8 * V + 8) * sizeof(u32), s));
-    } else {
-        CUDA_TRY(ctx, cudaMemsetAsync(P->lcount.ptr(), 0, (4 * V + 4) * sizeof(u32), s));
-        CUDA_TRY(ctx, cudaMemsetAsync(P->ecount.ptr(), 0, (4 * V + 4) * sizeof(u32), s));
-    }
+    EULER_TRY(clear_degrees(ctx, P, V, paired));
     EULER_TRY(graph_compact_vertices(ctx, P->vt_keys.ptr(), P->vt_id0.ptr(), vt_cap, k, P->vkeys.ptr()));
     VertexTable vt = {P->vt_keys.ptr(), P->vt_id0.ptr(), nullptr, vt_cap, k, vth};
     if (flags & EULER_RUN_CANONICAL_IDS) {
@@ -701,30 +733,12 @@ static int pipeline_run(euler_ctx *ctx, Pipeline *P, u32 l, u32 flags, u64 disti
                                        P->ev.ptr()));
     launches += 1;
     CUDA_TRY(ctx, cudaEventRecord(ctx->ev[2], s));
-    if (flags & EULER_RUN_EXPAND_EDGES) {
-        launches += 1;
-        EULER_TRY(P->ee.reserve(ctx, E)); EULER_TRY(P->lev.reserve(ctx, E)); EULER_TRY(P->ent.reserve(ctx, E));
-        EULER_TRY(graph_setup_edges(ctx, P->lkeys.ptr(), P->lvals.ptr(), P->loffs.ptr(), U_l, l, P->ev1.ptr(), P->ev2.ptr(),
-                                    P->lstart.ptr(), P->estart.ptr(), (u32)E, P->ee.ptr(), P->lev.ptr(), P->ent.ptr()));
-        P->expanded = true;
-    }
-    CUDA_TRY(ctx, cudaEventRecord(ctx->ev[3], s));
-    CUDA_TRY(ctx, cudaStreamSynchronize(s));
-    P->have_graph = true;
+    EULER_TRY(expand_edges(ctx, P, launches));
     P->learned_bases = B;
     // canonical distinct counts: palindromes are rare, U/2 rounded up is a safe learned size
     P->learned_lc = (U_l + 1) / 2 + 16; P->learned_vc = (V + 1) / 2 + 16;
-
-    euler_stats &st = P->st;
-    st.n_kmer_windows = N_k; st.n_lmer_windows = N_l; st.distinct_lmers = U_l; st.distinct_kmers = V; st.edge_count = E;
-    st.lmer_table_capacity = lt_cap; st.kmer_table_capacity = vt_cap; st.retries = retries;
-    cudaEventElapsedTime(&st.ms_count, ctx->ev[0], ctx->ev[1]);
-    cudaEventElapsedTime(&st.ms_graph, ctx->ev[1], ctx->ev[2]);
-    cudaEventElapsedTime(&st.ms_total, ctx->ev[0], ctx->ev[2]);
-    cudaEventElapsedTime(&st.ms_count_kernel, ctx->ev[4], ctx->ev[1]);
-    st.kernel_launches = launches;
-    if (stats) *stats = st;
-    return EULER_OK;
+    P->st.n_kmer_windows = N_k; P->st.n_lmer_windows = N_l;
+    return finish_run(ctx, P, lt_cap, vt_cap, retries, launches, 1, 2, stats);
 }
 
 // per-rank build of the partitioned path over 16-byte keys (wide_dist.cu); same contract as dist_build_impl
@@ -735,12 +749,10 @@ static int wide_dist_build_impl(euler_ctx *ctx, Pipeline *P, const void *d_keys,
     if (nranks > 8) return euler_fail(ctx, EULER_ERR_ARG, "128-bit keys: at most 8 ranks");
     cudaStream_t s = ctx->stream;
     const u32 k = l - 1;
-    P->l = l; P->flags = 0; P->have_graph = false; P->expanded = false; P->text_valid = false; P->wide = true;
-    memset(&P->st, 0, sizeof(P->st));
+    begin_run(P, l, 0, true, 0, 0);
     EULER_TRY(P->stats.reserve(ctx, 64));
-    const bool learned = !distinct_hint && P->learned_bases == nkeys && P->learned_lc;
-    const u64 est = distinct_hint ? distinct_hint : (learned ? P->learned_lc : (nkeys ? nkeys : 1));
-    u64 lt_cap = cap_for(est), vt_cap = cap_for(learned ? P->learned_vc : est);
+    u64 lt_cap, vt_cap;
+    caps_from_keys(P, nkeys, distinct_hint, lt_cap, vt_cap);
     u64 h[8] = {0};
     u32 retries = 0, launches = 0;
     CUDA_TRY(ctx, cudaEventRecord(ctx->ev[0], s));
@@ -772,15 +784,8 @@ static int wide_dist_build_impl(euler_ctx *ctx, Pipeline *P, const void *d_keys,
     const u64 U_l = h[3], V = h[4];
     P->U_l = U_l; P->V = V;
     if (V >= 0x3fffffffull || U_l >= 0xffffffffull) return euler_fail(ctx, EULER_ERR_RANGE, "graph exceeds u32 ids");
-    EULER_TRY(P->lkeys.reserve(ctx, U_l)); EULER_TRY(P->lkeys_hi.reserve(ctx, U_l)); EULER_TRY(P->lvals.reserve(ctx, U_l));
-    EULER_TRY(P->loffs.reserve(ctx, U_l)); EULER_TRY(P->ev1.reserve(ctx, U_l)); EULER_TRY(P->ev2.reserve(ctx, U_l));
-    EULER_TRY(P->tf.reserve(ctx, U_l + 16));
-    EULER_TRY(P->vkeys.reserve(ctx, V)); EULER_TRY(P->vkeys_hi.reserve(ctx, V));
-    EULER_TRY(P->lcount.reserve(ctx, 4 * V + 4)); EULER_TRY(P->ecount.reserve(ctx, 4 * V + 4));
-    EULER_TRY(P->lstart.reserve(ctx, 4 * V + 4)); EULER_TRY(P->estart.reserve(ctx, 4 * V + 4));
-    EULER_TRY(P->ev.reserve(ctx, V));
-    CUDA_TRY(ctx, cudaMemsetAsync(P->lcount.ptr(), 0, (4 * V + 4) * sizeof(u32), s));
-    CUDA_TRY(ctx, cudaMemsetAsync(P->ecount.ptr(), 0, (4 * V + 4) * sizeof(u32), s));
+    EULER_TRY(reserve_graph(ctx, P, U_l, V, true));
+    EULER_TRY(clear_degrees(ctx, P, V, false));
     EULER_TRY(wide_compact_vertices(ctx, P->wvt_keys.ptr(), P->vt_id0.ptr(), vt_cap, k, P->vkeys.ptr(), P->vkeys_hi.ptr()));
     EULER_TRY(wide_compact_homed(ctx, P->wlt_keys.ptr(), P->wlt_cnt.ptr(), P->lt_own.ptr(), P->lt_base.ptr(), lt_cap, l,
                                  P->lkeys.ptr(), P->lkeys_hi.ptr(), P->lvals.ptr()));
@@ -800,20 +805,11 @@ static int wide_dist_build_impl(euler_ctx *ctx, Pipeline *P, const void *d_keys,
     EULER_TRY(read_u64(ctx, P->stats.ptr() + 6, &E));
     launches += 10;
     P->E = E;
-    P->have_graph = true;
     P->learned_bases = nkeys;
     P->learned_lc = h[5] + h[5] / 32 + 16;
     P->learned_vc = (V + 1) / 2 + V / 32 + 16;
-    euler_stats &st = P->st;
-    st.n_lmer_windows = nkeys; st.distinct_lmers = U_l; st.distinct_kmers = V; st.edge_count = E;
-    st.lmer_table_capacity = lt_cap; st.kmer_table_capacity = vt_cap; st.retries = retries;
-    cudaEventElapsedTime(&st.ms_count, ctx->ev[0], ctx->ev[1]);
-    cudaEventElapsedTime(&st.ms_graph, ctx->ev[1], ctx->ev[2]);
-    cudaEventElapsedTime(&st.ms_total, ctx->ev[0], ctx->ev[2]);
-    cudaEventElapsedTime(&st.ms_count_kernel, ctx->ev[4], ctx->ev[1]);
-    st.kernel_launches = launches;
-    if (stats) *stats = st;
-    return EULER_OK;
+    P->st.n_lmer_windows = nkeys;
+    return finish_run(ctx, P, lt_cap, vt_cap, retries, launches, 1, 2, stats);
 }
 
 static Pipeline *get_pipe(euler_ctx *ctx)
@@ -1247,13 +1243,10 @@ static int dist_build_impl(euler_ctx *ctx, const void *d_keys, uint64_t nkeys, u
     if (l > 32) return wide_dist_build_impl(ctx, P, d_keys, nkeys, nregions, region_stride, region_counts, l, rank, nranks, distinct_hint, stats);
     cudaStream_t s = ctx->stream;
     const u32 k = l - 1;
-    P->wide = false;
-    P->l = l; P->flags = 0; P->have_graph = false; P->expanded = false;
-    memset(&P->st, 0, sizeof(P->st));
+    begin_run(P, l, 0, false, 0, 0);
     EULER_TRY(P->stats.reserve(ctx, 64));
-    const bool learned = !distinct_hint && P->learned_bases == nkeys && P->learned_lc;
-    const u64 est = distinct_hint ? distinct_hint : (learned ? P->learned_lc : (nkeys ? nkeys : 1));
-    u64 lt_cap = cap_for(est), vt_cap = cap_for(learned ? P->learned_vc : est);
+    u64 lt_cap, vt_cap;
+    caps_from_keys(P, nkeys, distinct_hint, lt_cap, vt_cap);
     u64 h[8] = {0};
     u32 retries = 0, launches = 0;
     CUDA_TRY(ctx, cudaEventRecord(ctx->ev[0], s));
@@ -1323,18 +1316,8 @@ static int dist_build_impl(euler_ctx *ctx, const void *d_keys, uint64_t nkeys, u
     const bool big = 2 * nkeys >= 0xffffffffull || (force_big && atoi(force_big) == 1);
     P->U_l = U_l; P->V = V;
     if (V >= 0x3fffffffull) return euler_fail(ctx, EULER_ERR_RANGE, "vertex count exceeds u32 ids");
-    EULER_TRY(P->lkeys.reserve(ctx, U_l)); EULER_TRY(P->lvals.reserve(ctx, U_l)); EULER_TRY(P->loffs.reserve(ctx, U_l));
-    EULER_TRY(P->ev1.reserve(ctx, U_l)); EULER_TRY(P->ev2.reserve(ctx, U_l)); EULER_TRY(P->vkeys.reserve(ctx, V));
-    EULER_TRY(P->lcount.reserve(ctx, 4 * V + 4)); EULER_TRY(P->ecount.reserve(ctx, 4 * V + 4));
-    EULER_TRY(P->lstart.reserve(ctx, 4 * V + 4)); EULER_TRY(P->estart.reserve(ctx, 4 * V + 4));
-    EULER_TRY(P->ev.reserve(ctx, V));
-    if (!big) {   // paired degree regions: two sectors per l-mer instead of four (common.cuh, DegOut)
-        EULER_TRY(P->deg.reserve(ctx, 8 * V + 8));
-        CUDA_TRY(ctx, cudaMemsetAsync(P->deg.ptr(), 0, (8 * V + 8) * sizeof(u32), s));
-    } else {
-        CUDA_TRY(ctx, cudaMemsetAsync(P->lcount.ptr(), 0, (4 * V + 4) * sizeof(u32), s));
-        CUDA_TRY(ctx, cudaMemsetAsync(P->ecount.ptr(), 0, (4 * V + 4) * sizeof(u32), s));
-    }
+    EULER_TRY(reserve_graph(ctx, P, U_l, V, false));
+    EULER_TRY(clear_degrees(ctx, P, V, !big));   // paired degree regions: two sectors per l-mer instead of four
     EULER_TRY(graph_compact_vertices(ctx, P->vt_keys.ptr(), P->vt_id0.ptr(), vt_cap, k, P->vkeys.ptr()));
     VertexTable vt = {P->vt_keys.ptr(), P->vt_id0.ptr(), nullptr, vt_cap, k, TableHash{0, 0}};
     EULER_TRY(P->vt_bbase.reserve(ctx, vt_cap / EULER_BUCKET + 1));
@@ -1359,23 +1342,13 @@ static int dist_build_impl(euler_ctx *ctx, const void *d_keys, uint64_t nkeys, u
     }
     P->E = E;
     CUDA_TRY(ctx, cudaEventRecord(ctx->ev[2], s));
-    CUDA_TRY(ctx, cudaStreamSynchronize(s));
-    P->have_graph = true;
     P->learned_bases = nkeys;
     // sizes for the next run of the same input: distinct canonical l-mers held by this rank (homed or
     // not; counted by the insert kernel) and canonical owned vertices (palindromes are rare)
     P->learned_lc = h[5] + h[5] / 32 + 16;
     P->learned_vc = (V + 1) / 2 + V / 32 + 16;
-    euler_stats &st = P->st;
-    st.n_bases = 0; st.n_reads = 0; st.n_lmer_windows = nkeys; st.distinct_lmers = U_l; st.distinct_kmers = V; st.edge_count = E;
-    st.lmer_table_capacity = lt_cap; st.kmer_table_capacity = vt_cap; st.retries = retries;
-    cudaEventElapsedTime(&st.ms_count, ctx->ev[0], ctx->ev[1]);
-    cudaEventElapsedTime(&st.ms_graph, ctx->ev[1], ctx->ev[2]);
-    cudaEventElapsedTime(&st.ms_total, ctx->ev[0], ctx->ev[2]);
-    cudaEventElapsedTime(&st.ms_count_kernel, ctx->ev[4], ctx->ev[1]);
-    st.kernel_launches = launches;
-    if (stats) *stats = st;
-    return EULER_OK;
+    P->st.n_lmer_windows = nkeys;
+    return finish_run(ctx, P, lt_cap, vt_cap, retries, launches, 1, 2, stats);
 }
 
 // ---- multi-GPU form of the bucketed path -----------------------------------------------------------------------
@@ -1476,8 +1449,7 @@ int euler_bkt_build(euler_ctx *ctx, const void *d_area, uint32_t l, uint32_t my_
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     Pipeline *P = get_pipe(ctx);
     cudaStream_t s = ctx->stream;
-    P->wide = false; P->l = l; P->flags = 0; P->have_graph = false; P->expanded = false; P->text_valid = false;
-    memset(&P->st, 0, sizeof(P->st));
+    begin_run(P, l, 0, false, 0, 0);
     EULER_TRY(P->stats.reserve(ctx, 64));
     const u32 nb = nb_per_rank;
     const u64 key = ((u64)nb << 32) ^ ((u64)nranks << 8) ^ l;   // what the learned capacities belong to
@@ -1500,36 +1472,17 @@ int euler_bkt_build(euler_ctx *ctx, const void *d_area, uint32_t l, uint32_t my_
     CUDA_TRY(ctx, cudaEventRecord(ctx->ev[7], s));
     while (true) {
         if ((u64)nb * rcap * 16 > (64ull << 30)) return euler_fail(ctx, EULER_ERR_NOMEM, "bucket regions of %u x %u records do not fit", nb, rcap);
-        EULER_TRY(dev_reserve(ctx, P->bk_records, (size_t)nb * rcap * 16 + 16));
-        EULER_TRY(P->bk_cursors.reserve(ctx, nb));
-        EULER_TRY(dev_reserve(ctx, P->bk_state, bkt_state_bytes(nb)));
-        EULER_TRY(P->bk_bkeys.reserve(ctx, bcap)); EULER_TRY(P->bk_bvals.reserve(ctx, 2 * bcap));
-        EULER_TRY(P->lkeys.reserve(ctx, ucap)); EULER_TRY(P->lvals.reserve(ctx, ucap)); EULER_TRY(P->loffs.reserve(ctx, ucap));
-        EULER_TRY(P->ev1.reserve(ctx, ucap)); EULER_TRY(P->ev2.reserve(ctx, ucap));
-        EULER_TRY(P->vkeys.reserve(ctx, vcap));
-        EULER_TRY(P->lcount.reserve(ctx, 4 * vcap + 4)); EULER_TRY(P->ecount.reserve(ctx, 4 * vcap + 4));
-        EULER_TRY(P->lstart.reserve(ctx, 4 * vcap + 4)); EULER_TRY(P->estart.reserve(ctx, 4 * vcap + 4));
-        EULER_TRY(P->ev.reserve(ctx, vcap));
-        CUDA_TRY(ctx, cudaMemsetAsync(P->stats.ptr(), 0, 8 * sizeof(u64), s));
-        if (need_regroup) {
-            CUDA_TRY(ctx, cudaMemsetAsync(P->bk_cursors.ptr(), 0, (size_t)nb * sizeof(u32), s));
-            EULER_TRY(bkt_regroup(ctx, d_area, d_counts, nranks, scap, nb, rcap, P->bk_records.p, P->bk_cursors.ptr(), P->stats.ptr()));
-            launches++;
-            need_regroup = false;
-        }
-        BktBuild bb;
-        bb.records = P->bk_records.p; bb.counts = P->bk_cursors.ptr(); bb.nb = nb; bb.nranks = 1; bb.rcap = rcap; bb.l = l; bb.cap = cap;
-        bb.lkeys = P->lkeys.ptr(); bb.lvals = P->lvals.ptr(); bb.loffs = P->loffs.ptr(); bb.ev1 = P->ev1.ptr(); bb.ev2 = P->ev2.ptr(); bb.ucap = ucap;
-        bb.vkeys = P->vkeys.ptr(); bb.lcount = P->lcount.ptr(); bb.ecount = P->ecount.ptr(); bb.lstart = P->lstart.ptr();
-        bb.estart = P->estart.ptr(); bb.ev = P->ev.ptr(); bb.vcap = vcap;
-        bb.state = P->bk_state.p; bb.bkeys = P->bk_bkeys.ptr(); bb.bvals = P->bk_bvals.ptr(); bb.bcap = bcap; bb.stats = P->stats.ptr();
-        CUDA_TRY(ctx, cudaEventRecord(ctx->ev[5], s));
-        EULER_TRY(bkt_build(ctx, bb));
-        CUDA_TRY(ctx, cudaEventRecord(ctx->ev[2], s));
-        launches += 4;   // build, second pass, boundary publish, fix-up
-        EULER_TRY(read_u64s(ctx, P->stats.ptr(), h, 8));
+        EULER_TRY(bkt_round(ctx, P, l, nb, rcap, cap, ucap, vcap, bcap, launches, h, [&]() -> int {
+            CUDA_TRY(ctx, cudaMemsetAsync(P->stats.ptr(), 0, 8 * sizeof(u64), s));
+            if (need_regroup) {
+                CUDA_TRY(ctx, cudaMemsetAsync(P->bk_cursors.ptr(), 0, (size_t)nb * sizeof(u32), s));
+                EULER_TRY(bkt_regroup(ctx, d_area, d_counts, nranks, scap, nb, rcap, P->bk_records.p, P->bk_cursors.ptr(), P->stats.ptr()));
+                launches++;
+                need_regroup = false;
+            }
+            return EULER_OK;
+        }));
         const u64 fl = h[2];
-        if (fl & BKT_FLAG_INTERNAL) return euler_fail(ctx, EULER_ERR_STATE, "internal: bucketed build consistency check failed (flags %llx)", fl);
         if ((fl & BKT_FLAG_TABLE) && cap * 2 > BKT_MAX_CAP)
             return euler_fail(ctx, EULER_ERR_OVERFLOW, "a bucket does not fit its shared-memory table: partition again with more buckets per rank");
         if (!(fl & (BKT_FLAG_REGION | BKT_FLAG_TABLE | BKT_FLAG_OUTPUT | BKT_FLAG_BOUNDARY))) break;
@@ -1543,20 +1496,12 @@ int euler_bkt_build(euler_ctx *ctx, const void *d_area, uint32_t l, uint32_t my_
     const u64 U_l = h[3], V = h[4], E = h[5];
     if (V >= 0x3fffffffull || U_l >= 0xffffffffull) return euler_fail(ctx, EULER_ERR_RANGE, "graph exceeds u32 ids (U_l=%llu V=%llu)", U_l, V);
     P->U_l = U_l; P->V = V; P->E = E;
-    CUDA_TRY(ctx, cudaStreamSynchronize(s));
-    P->have_graph = true;
     P->bk_dist_key = key; P->bk_learned_u = U_l; P->bk_learned_v = V; P->bk_dist_rcap = (u32)(h[6] + h[6] / 8 + 16);
     P->bk_dist_cap = cap;
     euler_stats &st = P->st;
-    st.distinct_lmers = U_l; st.distinct_kmers = V; st.edge_count = E;
-    st.lmer_table_capacity = (u64)nb * cap; st.kmer_table_capacity = (u64)nb * cap; st.retries = retries;
-    st.ms_count = P->bk_scatter_ms;
-    cudaEventElapsedTime(&st.ms_graph, ctx->ev[7], ctx->ev[2]);
-    st.ms_total = st.ms_graph;
-    cudaEventElapsedTime(&st.ms_build_kernel, ctx->ev[5], ctx->ev[2]);
-    st.kernel_launches = launches; st.path = 1; st.n_buckets = nb; st.bucket_records = h[6]; st.redo_buckets = (u32)h[7];
-    if (stats) *stats = st;
-    return EULER_OK;
+    st.ms_count = P->bk_scatter_ms;   // the scatter pass of euler_bkt_scatter
+    st.path = 1; st.n_buckets = nb; st.bucket_records = h[6]; st.redo_buckets = (u32)h[7];
+    return finish_run(ctx, P, (u64)nb * cap, (u64)nb * cap, retries, launches, 7, 2, stats);
 }
 
 int euler_synth_reads_dev(euler_ctx *ctx, uint64_t genome_len, uint32_t read_len, uint32_t err_ppm, uint64_t first_read,

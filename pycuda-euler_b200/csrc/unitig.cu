@@ -450,6 +450,5 @@ int unitigs_multik(euler_ctx *ctx, const void *d_buf, const u64 *d_off, u64 nrea
         if (steps) steps[i] = euler_multik_step{K, n, nb - n, added, st};
         if (last) { *d_out = text; *out_bytes = nb; *ncontigs = n; }
     }
-    kept.free();
     return rc;
 }
