@@ -180,11 +180,14 @@ def arr_contigs(g, alive):
     return [(s, cyc, sm) for s, sm, cyc in out]
 
 
-def arrays(buf, off, ks, limit=1, clean=True, last=None, **kw):
+def arrays(buf, off, ks, limit=1, clean=True, last=None, trace=None, **kw):
     """the rule on unitig_np's graph (reads as oracle.pack_reads gives them); last (a dict) receives the last step's
-    graph (key "g") and its surviving nodes (key "alive")"""
+    graph (key "g") and its surviving nodes (key "alive").  trace (a list) receives one dict per step: K, contigs (its
+    [(contig, is_cycle, sum)]), weights (the w_C it hands on, one per contig) and odd_pal (the palindromic K-mers whose
+    count is the previous contigs' odd weight rounded up to even, above their read count)"""
     prev, Kp, steps, sums = [], None, [], []
     for K in ks:
+        odd_pal = 0
         rlo, rhi, rcnt = oracle.count_mers(buf, off, K)
         rcnt = rcnt.astype(np.int64)
         lo, hi, cnt = rlo, rhi, rcnt
@@ -202,9 +205,16 @@ def arrays(buf, off, ks, limit=1, clean=True, last=None, **kw):
             w = np.repeat(np.asarray(ws, np.int64), nw)
             tlo, thi = _revcomp(K, wlo, whi)
             pal = (wlo == tlo) & (whi == thi)
+            odd = pal & (w & 1 == 1)
             w = np.where(pal, w + (w & 1), w)
+            if trace is not None and odd.any():
+                rid = _find(K, rlo, rhi, wlo[odd], whi[odd])
+                below = np.where(rid >= 0, rcnt[np.maximum(rid, 0)], 0) < w[odd]
+                plo, phi, pw = _merge_max(K, wlo[odd][below], whi[odd][below], w[odd][below])
             wlo, whi, w = np.concatenate([wlo, tlo]), np.concatenate([whi, thi]), np.concatenate([w, w])
             lo, hi, cnt = _merge_max(K, np.concatenate([rlo, wlo]), np.concatenate([rhi, whi]), np.concatenate([rcnt, w]))
+            if trace is not None and odd.any():
+                odd_pal = int((cnt[_find(K, lo, hi, plo, phi)] == pw).sum())
         keep = cnt > limit
         g = unitig_np.Graph(K, lo[keep], hi[keep], cnt[keep])
         # nodes whose read count is <= limit (absent: 0), counted once per strand pair
@@ -224,6 +234,8 @@ def arrays(buf, off, ks, limit=1, clean=True, last=None, **kw):
         steps.append({"K": K, "contigs": len(out), "bases": sum(len(c) for c, _, _ in out), "nodes_added": added,
                       "clean": st})
         prev = [(c, weight(s, len(c) - K + 1, limit), cyc) for c, cyc, s in out]
+        if trace is not None:
+            trace.append({"K": K, "contigs": out, "weights": [w for _, w, _ in prev], "odd_pal": odd_pal})
         Kp = K
     return [c for c, _, _ in prev], sums, steps
 

@@ -34,6 +34,24 @@ def test_restatements_agree_on_shapes(name):
         assert added > 0   # the contigs do bring K-mers in
 
 
+def test_trace_changes_nothing():
+    """arrays(trace=...) returns what it returns without, which is what strings returns; the trace is its steps"""
+    reads = unitig_shapes.tandem() + unitig_shapes.inverted() + unitig_shapes.repeats()
+    buf, off = oracle.pack_reads(reads)
+    for ks in ([20, 32, 48], [21, 31, 33]):
+        trace = []
+        a = arrays(buf, off, ks, 1, trace=trace)
+        assert a == arrays(buf, off, ks, 1)
+        s = strings([r.upper() for r in reads], ks, 1)
+        assert canon_pairs(a[0], a[1], ks[-1]) == canon_pairs(s[0], s[1], ks[-1]) and a[2] == s[2]
+        assert [t["K"] for t in trace] == ks and trace[0]["odd_pal"] == 0
+        for t, st in zip(trace, a[2]):
+            assert len(t["contigs"]) == len(t["weights"]) == st["contigs"]
+            assert sum(len(c) for c, _, _ in t["contigs"]) == st["bases"]
+        assert [(c, s) for c, _, s in trace[-1]["contigs"]] == list(zip(a[0], a[1]))
+        assert any(cyc for t in trace for _, cyc, _ in t["contigs"])   # the bare tandem arrays are cycles
+
+
 # ---- hand-built cases ---------------------------------------------------------------------------------------------
 def _joint_reads():
     """two reads of a 175 bp genome that overlap by 25 bases, twice each: the 21-mers join them, the 31-mers do not"""

@@ -45,10 +45,13 @@ def inverted():
     return reads
 
 
-def repeat_genome(seed, genome_len, n_families, elem_len, copies, tandem_unit=7, tandem_copies=40):
+def repeat_genome(seed, genome_len, n_families, elem_len, copies, tandem_unit=7, tandem_copies=40, tandems=(),
+                  inverted=0, inverted_len=(20, 60)):
     """a random genome carrying repeat families: per family an element of elem_len = (lo, hi) bases, inserted
     copies = (lo, hi) times, a third of the copies reverse-complemented and a third with 1..3 substitutions; plus one
-    tandem array"""
+    tandem array.  Optional extras, drawn after all of that so that callers without them keep their genome: tandems,
+    one array per (unit length, (lo, hi) copies); and `inverted` inverted repeats x + twin(x), |x| in inverted_len
+    (palindromic K-mers at even K, hairpins at odd K)"""
     rng = random.Random(seed)
     g = list(_rand(rng, genome_len))
     for _ in range(n_families):
@@ -66,6 +69,14 @@ def repeat_genome(seed, genome_len, n_families, elem_len, copies, tandem_unit=7,
     unit = _rand(rng, tandem_unit)
     p = rng.randrange(0, genome_len - tandem_unit * tandem_copies)
     g[p:p + tandem_unit * tandem_copies] = unit * tandem_copies
+    for n, cp in tandems:
+        arr = _rand(rng, n) * rng.randint(*cp)
+        p = rng.randrange(0, genome_len - len(arr))
+        g[p:p + len(arr)] = arr
+    for _ in range(inverted):
+        x = _rand(rng, rng.randint(*inverted_len))
+        p = rng.randrange(0, genome_len - 2 * len(x))
+        g[p:p + 2 * len(x)] = x + twin(x)
     return "".join(g)
 
 
